@@ -50,6 +50,21 @@ def env_int(k, d):
     return int(os.environ.get(k, d))
 
 
+def dump_arrays(outdir, arrays):
+    """--dump-outputs: every array as DIR/<name>.npy in float64 (integer results and float32 values convert exactly), so
+    that two builds run with the same arguments (hence on the same seeded inputs) can be compared output for output."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), np.asarray(a, np.float64))
+
+
+def result_arrays(leg, raw_results):
+    """The lfd_result structs a caller of lfd_wait receives for the frames of one step, one array per field, frames first."""
+    from lfd_b200 import _lib
+    rec = np.frombuffer(b"".join(raw_results), dtype=np.dtype(_lib.Result))
+    return {"%s_%s" % (leg, f.rstrip("_")): rec[f] for f in rec.dtype.names}
+
+
 def make_pool(n, rank):
     """n distinct frames of the config-3 mix (seeded by run/camcol/filter/field), with their blot rects."""
     import lfd_b200
@@ -555,6 +570,8 @@ def run_ours(args):
                               "warmup": args.warmup, "ms_per_step": 1e3 * elapsed / args.steps, "profile_only": True,
                               "config": {"workload": WORKLOAD, "frames_per_step_per_gpu": B},
                               "stages": [{"stage": n, "ms_per_step": ms / n_serial} for n, ms in stage_ms]}))
+            if args.dump_outputs:
+                dump_arrays(args.dump_outputs, result_arrays("resident", res_resident))
         sampler.stop()
         return 0
 
@@ -597,6 +614,8 @@ def run_ours(args):
 
     launches_total = int(reduce_sum(launches + launches_e2e))
     os.sched_setaffinity(0, orig_affinity)     # the CPU baseline and the drop-in leg use every host core
+    if args.dump_outputs and rank == 0:
+        dump_arrays(args.dump_outputs, {**result_arrays("resident", res_resident), **result_arrays("e2e", res_e2e)})
 
     # ---- verify: the results of the LAST TIMED step of both legs against the oracle, outside the timed regions ----
     verified = mismatches = None
@@ -872,7 +891,7 @@ def run_ours_config5(args):
     sampler = ClockSampler(local)
     sampler.start()
     cases = c5_cases(quick=args.quick)
-    reps = max(args.steps // 10, 3)
+    reps = args.steps
     rows, verified, launches0 = [], 0, h.kernel_launches()
     tot_votes = tot_ms = 0.0
     try:
@@ -942,6 +961,8 @@ def run_ours_config5(args):
             "gvotes_per_s_rho1_mean": float(np.mean([r["gvotes_per_s"] for r in fine])) if fine else None,
             "cases": rows}
     print(json.dumps(line))
+    if args.dump_outputs:     # per case, what the last timed lfd_hough_lines call counted
+        dump_arrays(args.dump_outputs, {"config5_" + k: [r[k] for r in rows] for k in ("nnz", "votes", "lines")})
     h.close()
     return 0
 
@@ -1050,7 +1071,13 @@ def main():
     ap.add_argument("--no-dropin", action="store_true", help="skip the DetectTrails-on-FITS-files leg")
     ap.add_argument("--no-verify", action="store_true", help="skip the oracle check of the timed steps' results")
     ap.add_argument("--verify", action="store_true", help="(default) check the timed steps' results against the oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the results of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of this project's timed path (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     # stdout carries exactly ONE line, the JSON: libraries that print to fd 1 while we run (NCCL's version banner,

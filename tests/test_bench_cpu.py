@@ -54,6 +54,24 @@ def test_reference_arm_prints_one_json_line():
     assert d["config"]["workload"] == "config3-camcol-mix"
 
 
+def test_dump_outputs_writes_every_result_field(tmp_path):
+    """--dump-outputs: one float64 .npy per lfd_result field of the step's frames, frames first, values exact."""
+    bench = _bench()
+    from lfd_b200 import _lib
+    rs = [_lib.Result(), _lib.Result()]
+    rs[0].detected, rs[0].pass_, rs[0].theta = 1, 1, np.float32(0.1)
+    rs[1].rect_detection[1] = 7
+    rs[1].top_box[1][15][0] = np.float32(-2.5)
+    bench.dump_arrays(str(tmp_path / "out"), bench.result_arrays("resident", [bytes(r) for r in rs]))
+    names = sorted(p.name for p in (tmp_path / "out").iterdir())
+    assert names == sorted("resident_%s.npy" % f.rstrip("_") for f, _t in _lib.Result._fields_)
+    load = lambda n: np.load(tmp_path / "out" / ("resident_%s.npy" % n))   # noqa: E731
+    assert all(np.load(tmp_path / "out" / n).dtype == np.float64 for n in names)
+    assert load("detected").tolist() == [1, 0] and load("pass").tolist() == [1, 0]
+    assert load("theta")[0] == np.float32(0.1) and load("rect_detection").tolist() == [[0, 0], [0, 7]]
+    assert load("top_box").shape == (2, 2, 16, 2) and load("top_box")[1, 1, 15, 0] == -2.5
+
+
 def test_roofline_names_the_time_dominant_kernel():
     """build_roofline: the kernel with the most bracketed time per step (all launches of the function together) is the one
     named, whatever stage it belongs to; the streaming-stage kernel is kept beside it."""
