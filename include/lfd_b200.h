@@ -73,8 +73,7 @@ enum lfd_stage {
     LFD_STAGE_GRAY = 1,      /* convertScaleAbs output          processfield.py:346,456 */
     LFD_STAGE_EQU = 2,       /* equalizeHist output             processfield.py:347,457 */
     LFD_STAGE_ERODED = 3,    /* erode output (dim only)         processfield.py:464     */
-    LFD_STAGE_MORPH = 4,     /* dilate output = Canny/Hough input  processfield.py:354,471 (with LFD_FUSED=1 the plane only
-                                exists after a run with LFD_KEEP_TAPS: the fused kernel never writes it otherwise) */
+    LFD_STAGE_MORPH = 4,     /* dilate output = Canny/Hough input  processfield.py:354,471 */
     LFD_STAGE_CANNY = 5,     /* Canny(.,0,255)                  processfield.py:236     */
     LFD_STAGE_BOX = 6,       /* box_img                         processfield.py:235,261 */
     LFD_STAGE_HIST = 7,      /* uint32[256] histogram of GRAY */

@@ -171,7 +171,7 @@ struct Fd { int fd; explicit Fd(const char* p) : fd(open(p, O_RDONLY | O_CLOEXEC
 // way: 12.2 MB per frame on every loader thread at once, i.e. the host's memory bus.  read() copies with ordinary stores,
 // so every destination line is first read for ownership: 3 bytes over the bus per payload byte.  Mapping the file and
 // copying with non-temporal stores moves 2 (profiles/lab/ingest_lab.cpp: +50-60 % frames/s at 8 threads); the H2D DMA
-// reads the slot from DRAM either way.  LFD_INGEST_COPY=pread restores the plain read.
+// reads the slot from DRAM either way.  Payloads under 1 MiB, and files that cannot be mapped, take the plain pread().
 #if defined(__x86_64__)
 __attribute__((target("avx2"))) static void stream_copy_avx2(char* dst, const char* src, size_t n)
 {
@@ -212,18 +212,12 @@ static void stream_copy(char* dst, const char* src, size_t n)
 #endif
 }
 
-static bool ingest_use_mmap()
-{
-    static const bool on = []() { const char* e = getenv("LFD_INGEST_COPY"); return !(e && strcmp(e, "pread") == 0); }();
-    return on;
-}
-
 // nbytes of the file at `off` into dest.  false: short file or I/O error.
 static bool read_payload(int fd, long off, long nbytes, char* dest)
 {
     struct stat st;
     if (fstat(fd, &st) != 0 || (long)st.st_size < off + nbytes) return false;    // (a mapping past the end would fault)
-    if (ingest_use_mmap() && nbytes >= (1 << 20)) {
+    if (nbytes >= (1 << 20)) {
         const long pg = sysconf(_SC_PAGESIZE), a0 = off & ~(pg - 1);
         void* m = mmap(nullptr, (size_t)(off - a0 + nbytes), PROT_READ, MAP_SHARED | MAP_POPULATE, fd, a0);
         if (m != MAP_FAILED) {

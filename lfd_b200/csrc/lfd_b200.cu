@@ -24,7 +24,6 @@
 #include "k_ccl.cuh"
 #include "k_hough.cuh"
 #include "k_morph.cuh"
-#include "k_mnms.cuh"
 #include "k_prep.cuh"
 #include "k_rects.cuh"
 #include "host_ingest.cuh"
@@ -33,17 +32,20 @@ static std::string g_create_error;
 
 // dynamic shared-memory opt-in (cudaFuncSetAttribute) is per function AND per device: high-water marks per device
 #define LFD_MAX_DEVICES 64
-#define LFD_MAX_SPLIT 4
 struct DevLimits { size_t band_max = 48 * 1024, rects_max = 48 * 1024, anyk_max = 48 * 1024; };
 static DevLimits g_dev_limits[LFD_MAX_DEVICES];
+
+// with the two passes overlapped, a batch of >= 16 frames is cut in this many parts (1 / 2 / 3 / 4 parts measured
+// 1.85 / 1.72 / 1.73 / 1.70 ms a step: DESIGN.md §3)
+#define LFD_BATCH_PARTS 2
 
 enum { T_PREP = 0, T_MORPH, T_CANNY, T_CCL_FG, T_CCL_BG, T_RECTS, T_HOUGH, T_CHECK, T_PER_PASS };
 static const char* k_timing_names[] = {
     "setup(memset+star_mask)",
     "prep(blot+flip+clip+u8+hist)",
-    "bright:lut+morph(+sobel+nms when fused)", "bright:sobel+nms", "bright:ccl_fg(hysteresis)", "bright:ccl_bg(holes)",
+    "bright:lut+morph", "bright:sobel+nms", "bright:ccl_fg(hysteresis)", "bright:ccl_bg(holes)",
     "bright:rects+boxfill", "bright:hough", "bright:check_theta",
-    "dim:lut+morph(+sobel+nms when fused)", "dim:sobel+nms", "dim:ccl_fg(hysteresis)", "dim:ccl_bg(holes)",
+    "dim:lut+morph", "dim:sobel+nms", "dim:ccl_fg(hysteresis)", "dim:ccl_bg(holes)",
     "dim:rects+boxfill", "dim:hough", "dim:check_theta",
     "results_d2h"};
 #define N_TIMINGS 17
@@ -76,10 +78,9 @@ struct lfd_handle {
     cudaStream_t stream = nullptr;        // uploads, prep, bright pass, results
     // the batch is cut in `nsplit` parts; part k runs its bright pass on xs[k][0] and its dim pass on xs[k][1]
     // (xs[0][0] is `stream` itself); every extra stream joins `stream` through its own event
-    cudaStream_t xs[LFD_MAX_SPLIT][2];
-    cudaEvent_t xjoin[LFD_MAX_SPLIT][2];
+    cudaStream_t xs[LFD_BATCH_PARTS][2];
+    cudaEvent_t xjoin[LFD_BATCH_PARTS][2];
     cudaEvent_t ev_fork = nullptr;
-    int nsplit_cfg = 2;                   // env LFD_NSPLIT (1..LFD_MAX_SPLIT)
     // host->device copy gate (lfd_set_h2d_gate): an advisory file lock shared with the other ranks of the same host bridge
     // slot, held from the moment the batch copy is enqueued until it has completed (released by a stream host callback)
     int gate_fd = -1;
@@ -132,8 +133,8 @@ struct lfd_handle {
     cudaEvent_t ev[N_TIMINGS + 1];
     bool ev_valid[N_TIMINGS + 1];
     float timings[N_TIMINGS];
-    cudaEvent_t kb[LFD_MAX_SPLIT][2][KB_COUNT][2];    // [part][pass][kernel][begin / end], created on first use
-    bool kb_used[LFD_MAX_SPLIT][2][KB_COUNT];         // recorded by the last run
+    cudaEvent_t kb[LFD_BATCH_PARTS][2][KB_COUNT][2];  // [part][pass][kernel][begin / end], created on first use
+    bool kb_used[LFD_BATCH_PARTS][2][KB_COUNT];       // recorded by the last run
     float kb_ms[2][KB_COUNT];                         // last run: per pass, summed over the parts
     int kb_launches[2][KB_COUNT];
     int cur_part = 0;                                 // part index of the run_pass_kernels call in progress
@@ -149,10 +150,6 @@ struct lfd_handle {
     AnyKernel anyk_h[2][2];
     bool anyk_on[2] = {false, false};
     int prep_grid[3] = {0, 0, 0};     // resident CTAs of k_prep<mode> on this device (one full wave)
-    // fused morphology + Sobel + NMS (k_mnms.cuh): 3-D tensor maps over gray[pass][frame][y][x], box 256 x FZ_RB x 1
-    CUtensorMap tm_gray[2];
-    bool fused_ok = false;            // frame shape allows the tensor maps (W % 16 == 0, W >= 256) and LFD_NO_FUSED is unset
-    int fused_case[2] = {-1, -1};     // per pass: index into the instantiated kernel shapes, -1 = unfused kernels
     cudaEvent_t mark[4];              // caller-placed timestamps on the handle's stream (lfd_timer_mark)
     bool mark_valid[4];
     // developer aid (env LFD_KTIMING=1): one event after every launch, reported by source line
@@ -358,7 +355,7 @@ extern "C" int lfd_destroy(lfd_handle* h)
     if (!h) return LFD_E_ARG;
     cudaSetDevice(h->device);
     if (h->stream) cudaStreamSynchronize(h->stream);
-    for (int k = 0; k < LFD_MAX_SPLIT; k++)
+    for (int k = 0; k < LFD_BATCH_PARTS; k++)
         for (int p = 0; p < 2; p++)
             if (h->xs[k][p] && h->xs[k][p] != h->stream) cudaStreamSynchronize(h->xs[k][p]);
     if (h->gate_fd >= 0) { flock(h->gate_fd, LOCK_UN); close(h->gate_fd); h->gate_fd = -1; }
@@ -376,7 +373,7 @@ extern "C" int lfd_destroy(lfd_handle* h)
     if (h->ctl_h) cudaFreeHost(h->ctl_h);
     if (h->counters_h) cudaFreeHost(h->counters_h);
     for (int i = 0; i <= N_TIMINGS; i++) if (h->ev_valid[i]) cudaEventDestroy(h->ev[i]);
-    for (int k = 0; k < LFD_MAX_SPLIT; k++)
+    for (int k = 0; k < LFD_BATCH_PARTS; k++)
         for (int p = 0; p < 2; p++)
             for (int b = 0; b < KB_COUNT; b++)
                 for (int e = 0; e < 2; e++)
@@ -384,7 +381,7 @@ extern "C" int lfd_destroy(lfd_handle* h)
     for (int i = 0; i < 4; i++) if (h->mark_valid[i]) cudaEventDestroy(h->mark[i]);
     if (h->graph_exec) cudaGraphExecDestroy(h->graph_exec);
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-    for (int k = 0; k < LFD_MAX_SPLIT; k++)
+    for (int k = 0; k < LFD_BATCH_PARTS; k++)
         for (int p = 0; p < 2; p++) {
             if (h->xjoin[k][p]) cudaEventDestroy(h->xjoin[k][p]);
             if (h->xs[k][p] && h->xs[k][p] != h->stream) cudaStreamDestroy(h->xs[k][p]);
@@ -417,14 +414,13 @@ static int create_impl(lfd_handle* h, int device, int max_batch, int H, int W, c
     long long worst = (long long)H * ((W + 1) / 2);
     if (h->cfg.max_runs > worst) h->cfg.max_runs = (int)worst;
     CK(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
-    for (int k = 0; k < LFD_MAX_SPLIT; k++)
+    for (int k = 0; k < LFD_BATCH_PARTS; k++)
         for (int p = 0; p < 2; p++) {
             if (k == 0 && p == 0) { h->xs[0][0] = h->stream; continue; }
             CK(cudaStreamCreateWithFlags(&h->xs[k][p], cudaStreamNonBlocking));
             CK(cudaEventCreateWithFlags(&h->xjoin[k][p], cudaEventDisableTiming));
         }
     CK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-    { const char* ns = getenv("LFD_NSPLIT"); if (ns && ns[0] >= '1' && ns[0] <= '0' + LFD_MAX_SPLIT) h->nsplit_cfg = ns[0] - '0'; }
     {
         cudaDeviceProp prop;
         CK(cudaGetDeviceProperties(&prop, device));
@@ -454,7 +450,7 @@ static int create_impl(lfd_handle* h, int device, int max_batch, int H, int W, c
     }
     for (int i = 0; i <= N_TIMINGS; i++) { CK(cudaEventCreate(&h->ev[i])); h->ev_valid[i] = true; }
     for (int i = 0; i < 4; i++) { CK(cudaEventCreate(&h->mark[i])); h->mark_valid[i] = true; }
-    for (int k = 0; k < LFD_MAX_SPLIT; k++)
+    for (int k = 0; k < LFD_BATCH_PARTS; k++)
         for (int p = 0; p < 2; p++)
             for (int b = 0; b < KB_COUNT; b++)
                 for (int e = 0; e < 2; e++) CK(cudaEventCreate(&h->kb[k][p][b][e]));
@@ -477,14 +473,6 @@ static int create_impl(lfd_handle* h, int device, int max_batch, int H, int W, c
         DA(h->strong[p], (size_t)B * NW);
         DA(h->edges[p], (size_t)B * NW);
         DA(h->box[p], (size_t)B * NW);
-    }
-    {
-        // Fused morphology + Sobel + NMS (k_mnms.cuh) is opt-in (LFD_FUSED=1): measured on B200 it executes as many
-        // instructions as the k_morph_march + k_nms_march pair and runs longer (profiles/r02c_*), so the pair stays the
-        // production path.  It needs 16-byte row strides for the tensor map and a frame at least one box wide.
-        const char* nf = getenv("LFD_FUSED");
-        h->fused_ok = (nf && nf[0] == '1') && (W % 16) == 0 && W >= FZ_BOXW;
-        h->fused_case[0] = h->fused_case[1] = -1;
     }
     DA(h->tap_u8, N);
     DA(h->ctl, (size_t)2 * B);
@@ -543,15 +531,7 @@ static int create_impl(lfd_handle* h, int device, int max_batch, int H, int W, c
         CK(cudaMemcpy(h->rbuf_d[p], h->rbuf_h[p].data(), B * sizeof(RectBuf), cudaMemcpyHostToDevice));
     }
 #undef DA
-    // Pinned staging of the frames.  LFD_STAGING=wc asks for write-combined pages: the loaders' stores then bypass the
-    // caches (no read-for-ownership of lines that are only ever written by the CPU and read by the DMA engine); CPU READS of
-    // such memory are very slow, so it is only for drivers that never read the staging back (profiles/lab/h2d_lab: the
-    // copy itself runs at the same 55.5 GB/s from either kind).
-    {
-        const char* sk = getenv("LFD_STAGING");
-        if (sk && sk[0] == 'w') CK(cudaHostAlloc((void**)&h->frames_h, (size_t)B * N * sizeof(float), cudaHostAllocWriteCombined));
-        else CK(cudaMallocHost((void**)&h->frames_h, (size_t)B * N * sizeof(float)));
-    }
+    CK(cudaMallocHost((void**)&h->frames_h, (size_t)B * N * sizeof(float)));
     CK(cudaMallocHost((void**)&h->res_h, (size_t)B * sizeof(lfd_result)));
     CK(cudaMallocHost((void**)&h->rects_h, (size_t)B * h->cfg.max_star_rects * sizeof(int4)));
     CK(cudaMallocHost((void**)&h->rect_off_h, ((size_t)B + 1) * sizeof(int)));
@@ -613,61 +593,6 @@ static int check_pass_params(lfd_handle* h, const lfd_pass_params& p, bool dim)
     return LFD_OK;
 }
 
-// Kernel shapes the fused kernel is instantiated for: {erode h, erode w, dilate h, dilate w}
-static const int k_fused_shapes[][4] = {{0, 0, 4, 4},       // params_bright default (detecttrails.py:204)
-                                         {3, 3, 9, 9},       // params_dim default (detecttrails.py:220-221)
-                                         {3, 3, 15, 15},     // high-sensitivity dim (BASELINE.json config 4)
-                                         {0, 0, 9, 9},
-                                         {0, 0, 3, 3}};
-#define FUSED_NCASES 5
-#define FUSED_DISPATCH(CASE, MACRO)                                                                \
-    switch (CASE) {                                                                                 \
-    case 0: MACRO(0, 0, 4, 4) break;                                                                \
-    case 1: MACRO(3, 3, 9, 9) break;                                                                \
-    case 2: MACRO(3, 3, 15, 15) break;                                                              \
-    case 3: MACRO(0, 0, 9, 9) break;                                                                \
-    case 4: MACRO(0, 0, 3, 3) break;                                                                \
-    default: break;                                                                                 \
-    }
-
-// Tensor map of gray[pass] ([B][H][W] uint8, box = 256 x U x 1) and the dynamic shared-memory opt-in of the kernel
-// instantiation that matches this pass's structuring elements; fused_case[pass] = -1 when there is none.
-static int fused_setup(lfd_handle* h, int pass, int eh, int ew, int dh, int dw)
-{
-    h->fused_case[pass] = -1;
-    if (!h->fused_ok) return LFD_OK;
-    int cs = -1;
-    for (int i = 0; i < FUSED_NCASES; i++)
-        if (k_fused_shapes[i][0] == eh && k_fused_shapes[i][1] == ew && k_fused_shapes[i][2] == dh && k_fused_shapes[i][3] == dw) cs = i;
-    if (cs < 0) return LFD_OK;
-    int U = 0, smem = 0;
-    cudaError_t ae = cudaSuccess;
-#define FZ_ATTR(EH_, EW_, DH_, DW_)                                                                                         \
-    U = FzGeom<EH_, DH_>::U; smem = FzGeom<EH_, DH_>::SMEM_B;                                                                \
-    ae = cudaFuncSetAttribute(k_morph_nms<EH_, EW_, DH_, DW_, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);   \
-    if (ae == cudaSuccess) ae = cudaFuncSetAttribute(k_morph_nms<EH_, EW_, DH_, DW_, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    FUSED_DISPATCH(cs, FZ_ATTR)
-#undef FZ_ATTR
-    if (ae != cudaSuccess) { h->err = std::string("cudaFuncSetAttribute(k_morph_nms): ") + cudaGetErrorString(ae); return LFD_E_CUDA; }
-    if (h->d.H < U) return LFD_OK;
-    typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                 const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                 CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess ||
-        qres != cudaDriverEntryPointSuccess || !fn) { cudaGetLastError(); return LFD_OK; }
-    const cuuint64_t gdim[3] = {(cuuint64_t)h->d.W, (cuuint64_t)h->d.H, (cuuint64_t)h->B};
-    const cuuint64_t gstr[2] = {(cuuint64_t)h->d.W, (cuuint64_t)h->d.W * (cuuint64_t)h->d.H};      // bytes, dimensions 1 and 2
-    const cuuint32_t box[3] = {FZ_BOXW, (cuuint32_t)U, 1};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    CUresult cr = ((EncodeFn)fn)(&h->tm_gray[pass], CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, h->gray[pass], gdim, gstr, box, estr,
-                                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr == CUDA_SUCCESS) h->fused_case[pass] = cs;
-    return LFD_OK;
-}
-
 extern "C" int lfd_set_params(lfd_handle* h, const lfd_params* p)
 {
     if (!h || !p) return LFD_E_ARG;
@@ -680,8 +605,6 @@ extern "C" int lfd_set_params(lfd_handle* h, const lfd_params* p)
         const lfd_pass_params& pp = pass ? p->dim : p->bright;
         // theta = np.pi/180 and threshold = 1 are literals in the reference (processfield.py:370, :488)
         rc = hough_setup(h, &h->hb[pass], h->d.H, h->d.W, pp.houghMethod, M_PI / 180, 1, h->B, false, h->cfg.max_lines);
-        if (rc != LFD_OK) return rc;
-        rc = fused_setup(h, pass, pass ? pp.erode_h : 0, pass ? pp.erode_w : 0, pp.dilate_h, pp.dilate_w);
         if (rc != LFD_OK) return rc;
     }
     h->params = *p;
@@ -776,7 +699,6 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
         if (!h->nms_tap[pass]) { int rc = dev_alloc(h, &h->nms_tap[pass], (size_t)h->B * d.N); if (rc) return rc; }
         ntap = h->nms_tap[pass] + fN;
     }
-    bool fused = false;        // morphology + Sobel + NMS done by one k_morph_nms launch
     if (part == 0) {
     // LUT + morphology
     k_lut<<<dim3(n, 1), 256, 0, s>>>(h->hist + (size_t)f0 * 256, h->lut + (size_t)f0 * 256, C, h->B, d.N, pass); LAUNCH_CHECK();
@@ -802,20 +724,6 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
             k_morph_any<<<ag, 256, anyk_smem(re, rd), s>>>(v_gray, lutp, v_morph, v_nz, etap, C, pass, d, ekd, dkd);
             done = true;
         }
-        // the all-ones rectangles of configs 1-4: one fused launch, gray rows staged by TMA (k_mnms.cuh); the morph plane is
-        // written only as a stage tap
-        if (!done && h->fused_case[pass] >= 0) {
-            const int fchunks = (d.H + FZ_R - 1) / FZ_R, funits = nstrips * fchunks;
-            dim3 fg((funits + FZ_WARPS - 1) / FZ_WARPS, n);
-#define FUSED_LAUNCH(EH_, EW_, DH_, DW_)                                                                              \
-            if (taps) k_morph_nms<EH_, EW_, DH_, DW_, true><<<fg, FZ_WARPS * 32, FzGeom<EH_, DH_>::SMEM_B, s>>>(h->tm_gray[pass], f0, \
-                                          lutp, v_morph, v_nz, etap, v_cand, v_strong, ntap, C, pass, d, nstrips, funits, 0, 255); \
-            else k_morph_nms<EH_, EW_, DH_, DW_, false><<<fg, FZ_WARPS * 32, FzGeom<EH_, DH_>::SMEM_B, s>>>(h->tm_gray[pass], f0, \
-                                          lutp, nullptr, v_nz, nullptr, v_cand, v_strong, nullptr, C, pass, d, nstrips, funits, 0, 255);
-            FUSED_DISPATCH(h->fused_case[pass], FUSED_LAUNCH)
-#undef FUSED_LAUNCH
-            done = true; fused = true;
-        }
 #define MORPH_CASE(EH_, EW_, DH_, DW_)                                                                              \
         if (!done && (d.W % 8) == 0 && mc.eh == EH_ && mc.ew == EW_ && mc.dh == DH_ && mc.dw == DW_) {                \
             k_morph_march<EH_, EW_, DH_, DW_><<<gg, MARCH_WPC * 32, 0, s>>>(v_gray, lutp, v_morph, v_nz, etap, \
@@ -837,8 +745,7 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
     KB_MARK(KB_MORPH, 1);
     STAGE_EVENT(tbase + 1);
     }
-    // Sobel + NMS (done by the fused kernel when that is selected)
-    if (!fused) {
+    // Sobel + NMS
     if ((d.W % 8) == 0) {        // k_nms_march stores only non-zero mask words
         CK(cudaMemsetAsync(v_cand, 0, (size_t)n * d.NW * sizeof(u32), s));
         CK(cudaMemsetAsync(v_strong, 0, (size_t)n * d.NW * sizeof(u32), s));
@@ -856,7 +763,6 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
     }
     LAUNCH_CHECK();
     KB_MARK(KB_NMS, 1);
-    }
     STAGE_EVENT(tbase + 2);
     // foreground runs: hysteresis + outer contours
     k_ccl_rowcount<<<rows, CCL_WARPS * 32, 0, s>>>(v_cand, v_ccl0, C, pass, d, 0); LAUNCH_CHECK();
@@ -981,10 +887,9 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
     const bool graph = overlap && h->use_graphs && !(flags & (LFD_KEEP_TAPS | LFD_FULL_LINES));
     h->stage_timings_valid = !graph;
     // everything from the fork to the result copies; captured into a CUDA graph when `graph`
-    // with overlap and a batch of >= 16 frames the batch is also cut in nsplit parts (default two halves): 2 x nsplit
+    // with overlap and a batch of >= 16 frames the batch is also cut in LFD_BATCH_PARTS parts (two halves): 2 x nsplit
     // independent chains (bright / dim x part) keep the SMs busy through the latency-bound CCL / geometry phases
-    int nsplit = (overlap && n >= 16) ? h->nsplit_cfg : 1;
-    if (nsplit > 1 && n / nsplit < 8) nsplit = n / 8 > 0 ? n / 8 : 1;
+    const int nsplit = (overlap && n >= 16) ? LFD_BATCH_PARTS : 1;
     auto passes = [&](bool stage_events) -> int {
         int rc2;
         if (overlap) {
@@ -1141,7 +1046,7 @@ extern "C" int lfd_wait(lfd_handle* h, lfd_result* out)
     }
     memset(h->kb_ms, 0, sizeof(h->kb_ms));
     memset(h->kb_launches, 0, sizeof(h->kb_launches));
-    for (int k = 0; k < LFD_MAX_SPLIT; k++)
+    for (int k = 0; k < LFD_BATCH_PARTS; k++)
         for (int p = 0; p < 2; p++)
             for (int b = 0; b < KB_COUNT; b++) {
                 if (!h->kb_used[k][p][b]) continue;
@@ -1252,11 +1157,7 @@ extern "C" int lfd_get_stage(lfd_handle* h, int frame, int pass, int stage, void
     case LFD_STAGE_ERODED:
         if (!h->eroded_tap || pass != 1) { h->err = "eroded tap not recorded (dim pass with LFD_KEEP_TAPS)"; return LFD_E_STATE; }
         src = h->eroded_tap + (size_t)frame * N; break;
-    case LFD_STAGE_MORPH:
-        // the fused production kernel never writes the morphology plane; it exists when the taps were kept (or on the
-        // unfused fallback path)
-        if (h->fused_case[pass] >= 0 && !(h->last_flags & LFD_KEEP_TAPS) && !h->anyk_on[pass]) { h->err = "morph plane not recorded (LFD_KEEP_TAPS)"; return LFD_E_STATE; }
-        src = h->morph[pass] + (size_t)frame * N; break;
+    case LFD_STAGE_MORPH: src = h->morph[pass] + (size_t)frame * N; break;
     case LFD_STAGE_CANNY:
         k_expand_mask<<<dim3(256, 1), 256, 0, s>>>(h->edges[pass] + (size_t)frame * d.NW, h->tap_u8, d1); LAUNCH_CHECK();
         src = h->tap_u8; break;

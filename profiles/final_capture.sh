@@ -5,7 +5,6 @@ set -u
 TAG=${1:-r02z}
 OUT=gpurun_out
 (timeout 1200 python -m pytest tests -m gpu -x -q --timeout 400 2>&1 | tail -4) > $OUT/${TAG}_tests.log; cat $OUT/${TAG}_tests.log
-(LFD_FUSED=1 timeout 600 python -m pytest tests/test_gpu_stages.py tests/test_gpu_batchpath.py -m gpu -x -q --timeout 400 2>&1 | tail -2) > $OUT/${TAG}_tests_fused.log; cat $OUT/${TAG}_tests_fused.log
 timeout 600 python bench.py --steps 40 --warmup 3 > $OUT/${TAG}_bench.json 2> $OUT/${TAG}_bench.err; echo "bench rc=$?"
 timeout 400 python bench.py --steps 40 --warmup 3 --serial-steps --no-dropin > $OUT/${TAG}_bench_serial_steps.json 2> /dev/null
 timeout 400 python bench.py --workload config4 --steps 20 --warmup 3 > $OUT/${TAG}_bench_c4.json 2> $OUT/${TAG}_bench_c4.err; echo "config4 rc=$?"

@@ -1,6 +1,6 @@
 #!/bin/bash
 # Per-kernel executed warp instructions, issue utilisation and duration of one warm resident step (cheap metrics only).
-# usage: bash profiles/inst_list.sh <tag>   (env such as LFD_NO_FUSED=1 is passed through)
+# usage: bash profiles/inst_list.sh <tag>   (the environment is passed through, e.g. LFD_B200_LIB=<path> to measure another build)
 set -u
 TAG=$1
 OUT=gpurun_out

@@ -93,7 +93,7 @@ def test_production_batches_match_oracle(cv2mod):
         res3 = h.wait()
         for j in range(n):
             assert device_verdict(res3[j], frames[0].shape) == tuple(ref[100 + j]), (j, kinds[100 + j])
-        # edge maps and box images the untapped (fused, graph) path left behind == the oracle's, pixel for pixel
+        # edge maps and box images the untapped (graph, batch parts) path left behind == the oracle's, pixel for pixel
         picked = [j for j in range(n) if ref[100 + j][0] is True][:3] + [j for j in range(n) if ref[100 + j][0] is False][:2]
         for j in picked:
             taps = {}

@@ -315,13 +315,10 @@ def test_scaled_frames_take_the_decoded_path(tmp_path):
     assert _lib.fits_load_frame(big, guard[:H]) is None and not guard[H:].any()
 
 
-def test_native_payload_copy_modes(tmp_path):
-    """The frame payload copy of the native reader (mapped file + non-temporal stores by default, plain pread with
-    LFD_INGEST_COPY=pread - read once per process, hence the child): same bytes either way, also into a slot that is not
-    32-byte aligned; a file shorter than its header claims is declined instead of faulting on the mapping."""
-    import hashlib
-    import subprocess
-    import sys
+def test_native_mapped_payload_copy(tmp_path):
+    """The native reader copies a full-size frame payload from the mapped file with non-temporal stores: the same bytes
+    as the Python reader, also into a slot that is not 32-byte aligned; a file shorter than its header claims is
+    declined instead of faulting on the mapping."""
     tree = synth.write_sdss_tree(str(tmp_path), 2888, 1, [100], filters=("r",))
     lfd_b200.setup(tree["bosspath"], tree["photoobjpath"], tree["photoreduxpath"], str(tmp_path))
     H, W = synth.FRAME_H, synth.FRAME_W
@@ -332,13 +329,6 @@ def test_native_payload_copy_modes(tmp_path):
     assert _lib.fits_load_frame(fpath, slot) is not None and np.array_equal(slot, ref)
     odd = np.zeros(H * W + 8, np.uint32)[3:3 + H * W].reshape(H, W)             # 12 bytes past the allocation's alignment
     assert _lib.fits_load_frame(fpath, odd) is not None and np.array_equal(odd, ref)
-    code = ("import sys, hashlib, numpy as np; sys.path.insert(0, %r); from lfd_b200 import _lib\n"
-            "s = np.zeros((%d, %d), np.uint32); assert _lib.fits_load_frame(%r, s) is not None\n"
-            "print('SHA', hashlib.sha1(s.tobytes()).hexdigest())" % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))), H, W, fpath))
-    env = dict(os.environ, LFD_INGEST_COPY="pread")
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=120)
-    assert out.returncode == 0, out.stderr
-    assert "SHA " + hashlib.sha1(ref.tobytes()).hexdigest() in out.stdout
     short = str(tmp_path / "short.fits")
     data = open(fpath, "rb").read()
     open(short, "wb").write(data[:len(data) - 2880 * 3])
