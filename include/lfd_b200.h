@@ -272,7 +272,8 @@ int lfd_ingest_batch(void* staging, int height, int width, int n, const char* co
                      char* values, int32_t* rects, int max_rects, int32_t* n_rects, int32_t* status_frame,
                      int32_t* status_cat, int nthreads);
 /* Work counters of the last run, summed over the batch: [0] nonzero px voted equ, [1] box, [2] votes,
- * [3] runs fg, [4] runs bg, [5] contours, [6] passing rects, [7] frames that ran dim, [8] frames that ran Hough. */
+ * [3] runs fg, [4] runs bg, [5] contours, [6] passing rects, [7] frames that ran dim, [8] frames that ran Hough,
+ * [14] labelling bands whose run-id look-back gave up waiting (frame reported LFD_FRAME_OVERFLOW; expected 0). */
 int lfd_get_counters(lfd_handle* h, int64_t* out, int n);
 
 #ifdef __cplusplus

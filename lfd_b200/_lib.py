@@ -487,7 +487,7 @@ class Handle:
         self._ck(self._L.lfd_get_counters(self.h, c, 16))
         names = ["nnz_equ", "nnz_box", "votes", "runs_fg", "runs_bg", "contours", "passing_rects", "frames_dim",
                  "frames_hough", "frames_bright_run", "frames_dim_run", "rects_warp_path", "rects_thread_overflow",
-                 "hough_smem_atomics"]
+                 "hough_smem_atomics", "ccl_lookback_stalls"]
         return {k: int(c[i]) for i, k in enumerate(names)}
 
     def timer_mark(self, slot):

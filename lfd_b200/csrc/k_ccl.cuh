@@ -23,17 +23,8 @@ struct CclBuf {
     int* ymax;        // [maxruns]  valid at roots
     int* compidx;     // [maxruns]  valid at roots: contour index or -1
     int* rowbase;     // [H+1]
-    u16* wpre;        // [H*WW]  run starts in the words before word w of the row
-    int* rowcnt;      // [H]
+    unsigned* look;   // [1 + bands]  k_ccl_band's ticket, then one look-back word per band (zeroed by k_ctl_init)
 };
-
-// mask word w of row y for kind 0 (as is) / kind 1 (complement, tail bits cleared)
-__device__ __forceinline__ u32 ccl_word(const u32* __restrict__ m, int y, int w, Dims d, int kind)
-{
-    if (w < 0 || w >= d.WW) return 0u;
-    u32 v = m[(size_t)y * d.WW + w];
-    return kind ? (~v & tail_mask(w, d.W)) : v;
-}
 
 // find with path halving (racy but safe: every store points a node at one of its ancestors)
 __device__ __forceinline__ int uf_find(int* parent, int i)
@@ -74,110 +65,18 @@ __device__ __forceinline__ void uf_union(int* parent, int a, int b)
 
 #define CCL_WARPS 8
 
-// 1. per row: number of runs + per-word exclusive prefix of run starts.  A warp takes CCL_RC_ROWS consecutive rows
-// and issues their mask loads together (the kernel is pure load latency: 12 MB per half batch); the word to the left
-// comes from the neighbouring lane instead of a second load.
-#define CCL_RC_ROWS 4
-__global__ void __launch_bounds__(CCL_WARPS * 32)
-k_ccl_rowcount(const u32* __restrict__ mask, CclBuf* __restrict__ bufs, const FrameCtl* __restrict__ ctl,
-               int pass, Dims d, int kind)
-{
-    int f = blockIdx.y;
-    if (!ctl[f].active[pass]) return;
-    const int y0 = (blockIdx.x * CCL_WARPS + (threadIdx.x >> 5)) * CCL_RC_ROWS;
-    if (y0 >= d.H) return;
-    const u32* m = mask + (size_t)f * d.NW;
-    CclBuf b = bufs[f];
-    const int lane = lane_id();
-    int base[CCL_RC_ROWS];
-    u32 left[CCL_RC_ROWS];                                   // last word of the previous 32-word chunk of the row
-#pragma unroll
-    for (int r = 0; r < CCL_RC_ROWS; r++) { base[r] = 0; left[r] = 0u; }
-    for (int w0 = 0; w0 < d.WW; w0 += 32) {
-        const int w = w0 + lane;
-        u32 cur[CCL_RC_ROWS];
-#pragma unroll
-        for (int r = 0; r < CCL_RC_ROWS; r++) cur[r] = (y0 + r < d.H) ? ccl_word(m, y0 + r, w, d, kind) : 0u;
-#pragma unroll
-        for (int r = 0; r < CCL_RC_ROWS; r++) {
-            u32 prev = __shfl_up_sync(FULLMASK, cur[r], 1);
-            if (lane == 0) prev = left[r];
-            left[r] = __shfl_sync(FULLMASK, cur[r], 31);
-            const u32 starts = cur[r] & ~((cur[r] << 1) | (prev >> 31));
-            const int c = __popc(starts);
-            int inc = c;
-            if (__any_sync(FULLMASK, c != 0)) {              // (no run starts in these 32 words: the prefix stays at base)
-                for (int o = 1; o < 32; o <<= 1) {
-                    int v = __shfl_up_sync(FULLMASK, inc, o);
-                    if (lane >= o) inc += v;
-                }
-            }
-            if (w < d.WW && y0 + r < d.H) b.wpre[(size_t)(y0 + r) * d.WW + w] = (u16)(base[r] + inc - c);
-            base[r] += __shfl_sync(FULLMASK, inc, 31);
-        }
-    }
-#pragma unroll
-    for (int r = 0; r < CCL_RC_ROWS; r++)
-        if (lane == 0 && y0 + r < d.H) b.rowcnt[y0 + r] = base[r];
-}
-
-// 2. exclusive scan of the row counts (one block per frame) -> rowbase[H+1], nruns
-__global__ void __launch_bounds__(1024)
-k_ccl_rowscan(CclBuf* __restrict__ bufs, FrameCtl* __restrict__ ctl, int pass, Dims d, int kind, int maxruns)
-{
-    int f = blockIdx.x;
-    if (!ctl[f].active[pass]) return;
-    CclBuf b = bufs[f];
-    __shared__ int wsum[32];
-    __shared__ int carry;
-    int t = threadIdx.x, lane = t & 31, wid = t >> 5;
-    if (t == 0) carry = 0;
-    __syncthreads();
-    for (int y0 = 0; y0 < d.H; y0 += 1024) {
-        int y = y0 + t;
-        int c = (y < d.H) ? b.rowcnt[y] : 0;
-        int inc = c;
-        for (int o = 1; o < 32; o <<= 1) {
-            int v = __shfl_up_sync(FULLMASK, inc, o);
-            if (lane >= o) inc += v;
-        }
-        if (lane == 31) wsum[wid] = inc;
-        __syncthreads();
-        if (wid == 0) {
-            int s = wsum[lane], si = s;
-            for (int o = 1; o < 32; o <<= 1) {
-                int v = __shfl_up_sync(FULLMASK, si, o);
-                if (lane >= o) si += v;
-            }
-            wsum[lane] = si - s;
-        }
-        __syncthreads();
-        int excl = carry + wsum[wid] + inc - c;
-        if (y < d.H) b.rowbase[y] = excl;
-        __syncthreads();
-        if (t == 1023) carry = excl + c;
-        __syncthreads();
-    }
-    if (t == 0) {
-        int total = carry;
-        b.rowbase[d.H] = total;
-        if (total > maxruns) {
-            atomicOr(&ctl[f].status, LFD_FRAME_OVERFLOW);
-            ctl[f].active[0] = ctl[f].active[1] = 0;     // drop the frame: later kernels skip it
-            total = 0;
-        }
-        ctl[f].nruns[kind] = total;
-    }
-}
+// The runs of a row are sorted by xs and pairwise disjoint, so rows are searched by bisection over
+// runs[rowbase[y] .. rowbase[y+1]) and the mask is never read again once the runs exist.
 
 // index of the run of row y that contains pixel p (which must be set)
-__device__ __forceinline__ int run_at(const u32* __restrict__ m, const CclBuf& b, int y, int p, Dims d, int kind)
+__device__ __forceinline__ int run_at(const CclBuf& b, int y, int p)
 {
-    int w = p >> 5, bit = p & 31;
-    u32 cur = ccl_word(m, y, w, d, kind), prev = ccl_word(m, y, w - 1, d, kind);
-    u32 starts = cur & ~((cur << 1) | (prev >> 31));
-    u32 upto = (bit == 31) ? 0xffffffffu : ((2u << bit) - 1u);
-    return b.rowbase[y] + b.wpre[(size_t)y * d.WW + w] + __popc(starts & upto) - 1;
+    int a = b.rowbase[y], e = b.rowbase[y + 1] - 1;          // last run with xs <= p
+    while (a < e) {
+        int mid = (a + e + 1) >> 1;
+        if ((int)b.runs[mid].xs <= p) a = mid; else e = mid - 1;
+    }
+    return a;
 }
 
 // Linking two adjacent rows.  The overlap graph between the sorted run lists of rows y-1 and y is a
@@ -185,30 +84,29 @@ __device__ __forceinline__ int run_at(const u32* __restrict__ m, const CclBuf& b
 // "r is the first run below that u touches".  So each run does exactly two lookups - first neighbour in
 // the row above, first neighbour in the row below - instead of walking all of its neighbours; a
 // frame-wide background run then costs the same as a one-pixel run.
-__device__ __forceinline__ int first_touching(const u32* __restrict__ m, const CclBuf& b, int yy, Run r, Dims d, int kind)
+__device__ __forceinline__ int first_touching(const CclBuf& b, int yy, Run r, int kind)
 {
     const int c = kind ? 0 : 1;
-    int lo = max((int)r.xs - c, 0), hi = min((int)r.xe + c, d.W - 1);
-    for (int w = lo >> 5; w <= (hi >> 5); w++) {
-        u32 v = ccl_word(m, yy, w, d, kind);
-        int blo = max(lo - (w << 5), 0), bhi = min(hi - (w << 5), 31);
-        u32 bits = v & bit_range(blo, bhi);
-        if (bits) return run_at(m, b, yy, (w << 5) + __ffs(bits) - 1, d, kind);
+    const int lo = (int)r.xs - c, hi = (int)r.xe + c;
+    const int e1 = b.rowbase[yy + 1];
+    int a = b.rowbase[yy], e = e1;                             // first run of row yy that ends at or after lo
+    while (a < e) {
+        int mid = (a + e) >> 1;
+        if ((int)b.runs[mid].xe < lo) a = mid + 1; else e = mid;
     }
-    return -1;
+    return (a < e1 && (int)b.runs[a].xs <= hi) ? a : -1;
 }
 
 // link rows y-1 and y: work items [0, n_below) are runs of row y (look up), [n_below, n_below+n_above)
 // are runs of row y-1 (look down)
-__device__ __forceinline__ void link_rows(const u32* __restrict__ m, const CclBuf& b, int y, Dims d, int kind,
-                                          int first, int stride)
+__device__ __forceinline__ void link_rows(const CclBuf& b, int y, int kind, int first, int stride)
 {
     int a0 = b.rowbase[y - 1], a1 = b.rowbase[y], b1 = b.rowbase[y + 1];
     int nb = b1 - a1, na = a1 - a0;
     for (int i = first; i < nb + na; i += stride) {
         bool below = i < nb;
         int id = below ? a1 + i : a0 + (i - nb);
-        int j = first_touching(m, b, below ? y - 1 : y, b.runs[id], d, kind);
+        int j = first_touching(b, below ? y - 1 : y, b.runs[id], kind);
         if (j >= 0) uf_union(b.parent, id, j);
     }
 }
@@ -249,176 +147,291 @@ __device__ __forceinline__ void suf_union(int* p, int a, int b)
 #define CCL_BAND_CAP 1536          // runs of one band kept in shared memory (12 B each = 18 KB)
 
 // dynamic shared memory of k_ccl_band: CCL_BAND rows of mask words, then the band's parents and runs
-// (+ the band's per-word run-rank prefixes, u16, and its CCL_BAND + 1 row bases)
+// (+ its CCL_BAND + 1 band-local row bases and the run rank, within its row, of the first run start of every mask word, u16)
 __host__ __device__ inline size_t ccl_band_smem(int WW)
 {
     return (size_t)CCL_BAND * WW * 4 + (size_t)CCL_BAND_CAP * 12 + (size_t)(CCL_BAND + 2) * 4 + (size_t)CCL_BAND * WW * 2;
 }
 
-// 3+4a fused: materialise the runs of a CCL_BAND-row band, link all of its row pairs at once with a
-// union-find that lives in shared memory, and publish band-local roots.  Run ids are raster-ordered, so
-// a band's runs are the contiguous range [rowbase[y0], rowbase[y1]) and local index = id - rowbase[y0].
-// The band's mask rows are staged in shared memory first (complemented for kind 1), so run ends and
-// neighbour lookups never go back to global memory.  Bands with more runs than CCL_BAND_CAP use the
-// global parent array with the same code path.
-__global__ void __launch_bounds__(256)
-k_ccl_band(const u32* __restrict__ mask, CclBuf* __restrict__ bufs, const FrameCtl* __restrict__ ctl,
-           int pass, Dims d, int kind)
+// Look-back words of k_ccl_band, CclBuf::look[1 + band]: 0 = nothing published yet, else a state in the top two bits
+// over a run count: the band's own count (aggregate) or the count of bands 0 .. band (inclusive prefix).
+#define CCL_LB_AGG (1u << 30)
+#define CCL_LB_INC (2u << 30)
+#define CCL_LB_VAL ((1u << 30) - 1u)
+#define CCL_LB_SPIN (1 << 20)      // polls of one predecessor before the frame is given up (never reached when every claimed band publishes)
+
+// exclusive prefix of `band` from its predecessors' look-back words (one thread); *stalled is set when a predecessor
+// published nothing within CCL_LB_SPIN polls
+__device__ __forceinline__ int ccl_lookback(const unsigned* look, int band, bool* stalled)
 {
-    int f = blockIdx.y;
+    int excl = 0;
+    for (int j = band - 1; j >= 0; j--) {
+        unsigned v;
+        int spins = 0;
+        while (((v = ((const volatile unsigned*)look)[1 + j]) >> 30) == 0u) {
+            if (++spins > CCL_LB_SPIN) { *stalled = true; return excl; }
+            __nanosleep(64);
+        }
+        excl += (int)(v & CCL_LB_VAL);
+        if ((v & ~CCL_LB_VAL) == CCL_LB_INC) break;
+    }
+    return excl;
+}
+
+// The run-based labelling of one mask, one CCL_BAND-row band at a time: count the band's runs, materialise them, link
+// all of its row pairs at once with a union-find that lives in shared memory, and publish band-local roots.
+//   * The band's mask rows are staged in shared memory (complemented for kind 1), so counting, run ends and neighbour
+//     lookups never go back to global memory.
+//   * Run ids are raster-ordered: a band's runs are [base, base + nb), where base = runs of the bands above.  Everything
+//     up to the publish works on band-local indices; base comes from a decoupled look-back over the bands' counts.
+//   * Forward progress: bands are claimed in order from the frame's ticket (look[0]), so every band a CTA waits on is
+//     held by a resident CTA, and every claimed band publishes its count before it waits on anything.  A CTA that
+//     sees the frame inactive returns before its first claim; once it has claimed, it publishes whatever ctl says.
+//   * The band that completes the frame writes rowbase[H] and nruns; a frame with more than maxruns runs is dropped
+//     (LFD_FRAME_OVERFLOW, both passes' active flags cleared) and no band stores a run past maxruns.
+//   * Bands with more runs than CCL_BAND_CAP use the global parent array with global ids, so they take their base
+//     before the fill.
+__global__ void __launch_bounds__(256)
+k_ccl_band(const u32* __restrict__ mask, CclBuf* __restrict__ bufs, FrameCtl* __restrict__ ctl,
+           int pass, Dims d, int kind, int maxruns, unsigned long long* __restrict__ counters)
+{
+    const int f = blockIdx.y;
     if (!ctl[f].active[pass]) return;
-    if (ctl[f].nruns[kind] == 0) return;
     const u32* m = mask + (size_t)f * d.NW;
     CclBuf b = bufs[f];
     extern __shared__ u32 band_sm[];
-    // A CTA takes the bands blockIdx.x, blockIdx.x + gridDim.x, ...: one band per CTA when a few frames are in the launch
-    // (shortest latency), CCL_BAND_CTAS bands-looping CTAs per frame in big batches, where the per-CTA prologue (11 % of the
-    // kernel's instructions with one band per CTA) is what counts: +1.4 % frames/s on the pipelined 64-frame step, while the
-    // launch alone gets 1.2-1.5x longer (DESIGN.md section 7).
-    for (int band = blockIdx.x; band * CCL_BAND < d.H; band += gridDim.x) {
-    __syncthreads();
-    const int y0 = band * CCL_BAND, y1 = min(y0 + CCL_BAND, d.H);
-    const int base = b.rowbase[y0], nb = b.rowbase[y1] - base;
-    if (nb == 0) continue;
+    __shared__ int s_band, s_base;
+    __shared__ bool s_stalled;
+    const int WW = d.WW, nbands = (d.H + CCL_BAND - 1) / CCL_BAND;
+    const int warp = threadIdx.x >> 5, lane = lane_id();
     u32* sw = band_sm;                                        // [CCL_BAND][WW]
-    int* sp = (int*)(band_sm + CCL_BAND * d.WW);              // [CCL_BAND_CAP]
+    int* sp = (int*)(band_sm + CCL_BAND * WW);                // [CCL_BAND_CAP]
     Run* srun = (Run*)(sp + CCL_BAND_CAP);                    // [CCL_BAND_CAP]
-    int* srb = (int*)(srun + CCL_BAND_CAP);                   // [CCL_BAND + 2] row bases of rows y0 .. y1
-    u16* swp = (u16*)(srb + CCL_BAND + 2);                    // [CCL_BAND][WW] run-rank prefix of every mask word
-    const bool insm = nb <= CCL_BAND_CAP;
-    const int WW = d.WW;
-    {
-        // stage the band: its mask rows and prefix words are contiguous in global memory; four independent loads per
-        // thread and iteration (this loop used to be one dependent load -> store per iteration: 12 % of the samples)
-        const int tot = (y1 - y0) * WW;
-        const u32* src = m + (size_t)y0 * WW;
-        const u16* psrc = b.wpre + (size_t)y0 * WW;
-        for (int i0 = threadIdx.x; i0 < tot; i0 += 4 * blockDim.x) {
-            u32 v[4]; u16 pw[4];
-#pragma unroll
-            for (int k = 0; k < 4; k++) {
-                const int i = i0 + k * blockDim.x;
-                v[k] = i < tot ? src[i] : 0u;
-                pw[k] = i < tot ? psrc[i] : (u16)0;
-            }
-#pragma unroll
-            for (int k = 0; k < 4; k++) {
-                const int i = i0 + k * blockDim.x;
-                if (i < tot) { sw[i] = kind ? ~v[k] : v[k]; swp[i] = pw[k]; }
-            }
-        }
-        if (threadIdx.x <= y1 - y0) srb[threadIdx.x] = b.rowbase[y0 + threadIdx.x];
+    int* srb = (int*)(srun + CCL_BAND_CAP);                   // [CCL_BAND + 1] band-local row bases of rows y0 .. y1
+    u16* swp = (u16*)(srb + CCL_BAND + 2);                    // [CCL_BAND][WW] run rank in its row of the word's first start
+    // A CTA claims bands until the frame has none left: one band per CTA when a few frames are in the launch (shortest
+    // latency), CCL_BAND_CTAS bands-looping CTAs per frame in big batches, where the per-CTA prologue (11 % of the
+    // kernel's instructions with one band per CTA) is what counts (DESIGN.md section 7).
+    for (;;) {
+        __syncthreads();                                      // the previous band's shared state is consumed
+        if (threadIdx.x == 0) { s_band = (int)atomicAdd(&b.look[0], 1u); s_stalled = false; }
         __syncthreads();
-        if (kind && (d.W & 31))                               // complemented rows: clear the bits past the frame edge
-            for (int yy = threadIdx.x; yy < y1 - y0; yy += blockDim.x) sw[yy * WW + WW - 1] &= tail_mask(WW - 1, d.W);
-    }
-    __syncthreads();
-    // fill: one warp per row, rows strided over the 8 warps
-    for (int y = y0 + (threadIdx.x >> 5); y < y1; y += 8) {
-        int rb = srb[y - y0];
-        if (srb[y - y0 + 1] == rb) continue;                      // no run in this row (most rows of a sparse edge map)
-        const u32* row = sw + (y - y0) * WW;
-        // words that are not all-ones, one ballot per 32-word chunk (W <= 4096 -> at most 4 chunks): a run
-        // that leaves its word ends in the next such word, found with a bit scan instead of a serial walk
-        // (the background of a sparse frame is one frame-wide run per row)
-        u32 nf[4];
+        const int band = s_band;
+        if (band >= nbands) break;
+        const int y0 = band * CCL_BAND, y1 = min(y0 + CCL_BAND, d.H), nr = y1 - y0;
+        {
+            // stage the band's mask rows (contiguous in global memory): four independent loads per thread and iteration
+            const int tot = nr * WW;
+            const u32* src = m + (size_t)y0 * WW;
+            for (int i0 = threadIdx.x; i0 < tot; i0 += 4 * blockDim.x) {
+                u32 v[4];
 #pragma unroll
-        for (int c = 0; c < 4; c++) {
-            int w = c * 32 + lane_id();
-            nf[c] = __ballot_sync(FULLMASK, w >= WW || row[w] != 0xffffffffu);
-        }
-        for (int w = lane_id(); w < WW; w += 32) {
-            u32 cur = row[w], prev = w ? row[w - 1] : 0u;
-            u32 starts = cur & ~((cur << 1) | (prev >> 31));
-            if (!starts) continue;
-            int id = rb + swp[(y - y0) * WW + w];
-            while (starts) {
-                int s = __ffs(starts) - 1;
-                starts &= starts - 1;
-                u32 above = ~(cur >> s);
-                int t = above ? (__ffs(above) - 1) : 32;
-                int xe;
-                if (s + t < 32) {
-                    xe = (w << 5) + s + t - 1;
-                } else {
-                    int w2 = WW;                                   // first not-full word after w
-                    const int c0 = w >> 5, pos = w & 31;
-#pragma unroll
-                    for (int c = 0; c < 4; c++) {
-                        if (c < c0 || w2 < WW) continue;
-                        u32 mbits = nf[c];
-                        if (c == c0) mbits &= (pos == 31) ? 0u : (0xffffffffu << (pos + 1));
-                        if (mbits) w2 = c * 32 + __ffs(mbits) - 1;
-                    }
-                    if (w2 >= WW) xe = (WW << 5) - 1;
-                    else xe = (w2 << 5) + __ffs(~row[w2]) - 2;
+                for (int k = 0; k < 4; k++) {
+                    const int i = i0 + k * blockDim.x;
+                    v[k] = i < tot ? src[i] : 0u;
                 }
-                Run r; r.xs = (u16)((w << 5) + s); r.xe = (u16)xe; r.y = (u16)y; r.pad = 0;
-                b.runs[id] = r;
-                b.flag[id] = 0;
-                b.ymax[id] = y;
-                b.compidx[id] = -1;
-                if (insm) { srun[id - base] = r; sp[id - base] = id - base; }
-                else b.parent[id] = id;
-                id++;
+#pragma unroll
+                for (int k = 0; k < 4; k++) {
+                    const int i = i0 + k * blockDim.x;
+                    if (i < tot) sw[i] = kind ? ~v[k] : v[k];
+                }
+            }
+            __syncthreads();
+            if (kind && (d.W & 31))                           // complemented rows: clear the bits past the frame edge
+                for (int r = threadIdx.x; r < nr; r += blockDim.x) sw[r * WW + WW - 1] &= tail_mask(WW - 1, d.W);
+        }
+        __syncthreads();
+        // count: one warp per row, 32 words at a time: run starts per word, warp scan -> rank of the word's first start
+        for (int r = warp; r < nr; r += CCL_WARPS) {
+            const u32* row = sw + r * WW;
+            int base = 0;
+            for (int w0 = 0; w0 < WW; w0 += 32) {
+                const int w = w0 + lane;
+                const u32 cur = w < WW ? row[w] : 0u, prev = (w && w <= WW) ? row[w - 1] : 0u;
+                const u32 starts = cur & ~((cur << 1) | (prev >> 31));
+                const int c = __popc(starts);
+                int inc = c;
+                if (__any_sync(FULLMASK, c != 0)) {
+                    for (int o = 1; o < 32; o <<= 1) {
+                        int v = __shfl_up_sync(FULLMASK, inc, o);
+                        if (lane >= o) inc += v;
+                    }
+                }
+                if (w < WW) swp[r * WW + w] = (u16)(base + inc - c);
+                base += __shfl_sync(FULLMASK, inc, 31);
+            }
+            if (lane == 0) srb[r + 1] = base;
+        }
+        __syncthreads();
+        if (warp == 0) {                                      // row counts -> band-local row bases (nr <= 32)
+            const int c = lane < nr ? srb[lane + 1] : 0;
+            int inc = c;
+            for (int o = 1; o < 32; o <<= 1) {
+                int v = __shfl_up_sync(FULLMASK, inc, o);
+                if (lane >= o) inc += v;
+            }
+            if (lane < nr) srb[lane + 1] = inc;
+            if (lane == 0) srb[0] = 0;
+        }
+        __syncthreads();
+        const int nb = srb[nr];
+        const bool insm = nb <= CCL_BAND_CAP;
+        if (threadIdx.x == 0) {
+            // publish the count before waiting on anything; band 0's count is already its inclusive prefix
+            atomicExch(&b.look[1 + band], (band == 0 ? CCL_LB_INC : CCL_LB_AGG) | (unsigned)nb);
+            if (!insm || band == 0) {
+                bool st = false;
+                const int ex = band ? ccl_lookback(b.look, band, &st) : 0;
+                if (band) atomicExch(&b.look[1 + band], CCL_LB_INC | (unsigned)(ex + nb));
+                s_base = ex; s_stalled = st;
             }
         }
-    }
-    __syncthreads();
-    // link every run with the first run it touches in the row above and in the row below (staircase argument)
-    const int c = kind ? 0 : 1;
-    for (int i = threadIdx.x; i < nb; i += blockDim.x) {
-        Run r = insm ? srun[i] : b.runs[base + i];
-        int lo = max((int)r.xs - c, 0), hi = min((int)r.xe + c, d.W - 1);
+        __syncthreads();
+        // a dense band needs its global ids up front; a frame over maxruns stores no run past maxruns
+        const bool fits_early = !insm && s_base + nb <= maxruns;
+        // fill: one warp per row, rows strided over the 8 warps; ids are band-local
+        if (insm || fits_early) {
+            const int gb = insm ? 0 : s_base;
+            for (int r = warp; r < nr; r += CCL_WARPS) {
+                const int rb = srb[r];
+                if (srb[r + 1] == rb) continue;                   // no run in this row (most rows of a sparse edge map)
+                const u32* row = sw + r * WW;
+                const int y = y0 + r;
+                // words that are not all-ones, one ballot per 32-word chunk (W <= 4096 -> at most 4 chunks): a run
+                // that leaves its word ends in the next such word, found with a bit scan instead of a serial walk
+                // (the background of a sparse frame is one frame-wide run per row)
+                u32 nf[4];
 #pragma unroll
-        for (int dy = -1; dy <= 1; dy += 2) {
-            int yy = (int)r.y + dy;
-            if (yy < y0 || yy >= y1) continue;
-            const u32* row = sw + (yy - y0) * WW;
-            int j = -1;
-            for (int w = lo >> 5; w <= (hi >> 5); w++) {
-                int blo = max(lo - (w << 5), 0), bhi = min(hi - (w << 5), 31);
-                u32 bits = row[w] & bit_range(blo, bhi);
-                if (bits) {
-                    // run of row yy that contains pixel p
-                    int bit = __ffs(bits) - 1;
+                for (int c = 0; c < 4; c++) {
+                    int w = c * 32 + lane;
+                    nf[c] = __ballot_sync(FULLMASK, w >= WW || row[w] != 0xffffffffu);
+                }
+                for (int w = lane; w < WW; w += 32) {
                     u32 cur = row[w], prev = w ? row[w - 1] : 0u;
                     u32 starts = cur & ~((cur << 1) | (prev >> 31));
-                    u32 upto = (bit == 31) ? 0xffffffffu : ((2u << bit) - 1u);
-                    j = srb[yy - y0] + swp[(yy - y0) * WW + w] + __popc(starts & upto) - 1;
-                    break;
+                    if (!starts) continue;
+                    int id = rb + swp[r * WW + w];
+                    while (starts) {
+                        int s = __ffs(starts) - 1;
+                        starts &= starts - 1;
+                        u32 above = ~(cur >> s);
+                        int t = above ? (__ffs(above) - 1) : 32;
+                        int xe;
+                        if (s + t < 32) {
+                            xe = (w << 5) + s + t - 1;
+                        } else {
+                            int w2 = WW;                                   // first not-full word after w
+                            const int c0 = w >> 5, pos = w & 31;
+#pragma unroll
+                            for (int c = 0; c < 4; c++) {
+                                if (c < c0 || w2 < WW) continue;
+                                u32 mbits = nf[c];
+                                if (c == c0) mbits &= (pos == 31) ? 0u : (0xffffffffu << (pos + 1));
+                                if (mbits) w2 = c * 32 + __ffs(mbits) - 1;
+                            }
+                            if (w2 >= WW) xe = (WW << 5) - 1;
+                            else xe = (w2 << 5) + __ffs(~row[w2]) - 2;
+                        }
+                        Run run; run.xs = (u16)((w << 5) + s); run.xe = (u16)xe; run.y = (u16)y; run.pad = 0;
+                        if (insm) { srun[id] = run; sp[id] = id; }
+                        else {
+                            b.runs[gb + id] = run;
+                            b.flag[gb + id] = 0;
+                            b.ymax[gb + id] = y;
+                            b.compidx[gb + id] = -1;
+                            b.parent[gb + id] = gb + id;
+                        }
+                        id++;
+                    }
                 }
             }
-            if (j >= 0) { if (insm) suf_union(sp, i, j - base); else uf_union(b.parent, base + i, j); }
+            __syncthreads();
+            // link every run with the first run it touches in the row above and in the row below (staircase argument)
+            const int c = kind ? 0 : 1;
+            for (int i = threadIdx.x; i < nb; i += blockDim.x) {
+                Run r = insm ? srun[i] : b.runs[gb + i];
+                int lo = max((int)r.xs - c, 0), hi = min((int)r.xe + c, d.W - 1);
+#pragma unroll
+                for (int dy = -1; dy <= 1; dy += 2) {
+                    int yy = (int)r.y + dy;
+                    if (yy < y0 || yy >= y1) continue;
+                    const u32* row = sw + (yy - y0) * WW;
+                    int j = -1;
+                    for (int w = lo >> 5; w <= (hi >> 5); w++) {
+                        int blo = max(lo - (w << 5), 0), bhi = min(hi - (w << 5), 31);
+                        u32 bits = row[w] & bit_range(blo, bhi);
+                        if (bits) {
+                            // band-local index of the run of row yy that contains pixel p
+                            int bit = __ffs(bits) - 1;
+                            u32 cur = row[w], prev = w ? row[w - 1] : 0u;
+                            u32 starts = cur & ~((cur << 1) | (prev >> 31));
+                            u32 upto = (bit == 31) ? 0xffffffffu : ((2u << bit) - 1u);
+                            j = srb[yy - y0] + swp[(yy - y0) * WW + w] + __popc(starts & upto) - 1;
+                            break;
+                        }
+                    }
+                    if (j >= 0) { if (insm) suf_union(sp, i, j); else uf_union(b.parent, gb + i, gb + j); }
+                }
+            }
+        }
+        if (insm && band) {
+            // the band's own work is done: now take the base (the predecessors have had all that time to publish)
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                bool st = false;
+                const int ex = ccl_lookback(b.look, band, &st);
+                atomicExch(&b.look[1 + band], CCL_LB_INC | (unsigned)(ex + nb));
+                s_base = ex; s_stalled = st;
+            }
+        }
+        __syncthreads();
+        const int base = s_base;
+        const bool fits = base + nb <= maxruns;
+        if (insm && fits) {
+            volatile int* vp = sp;
+            for (int i = threadIdx.x; i < nb; i += blockDim.x) {
+                int r = i, pr;
+                while ((pr = vp[r]) != r) r = pr;
+                const Run run = srun[i];
+                b.runs[base + i] = run;
+                b.flag[base + i] = 0;
+                b.ymax[base + i] = run.y;
+                b.compidx[base + i] = -1;
+                b.parent[base + i] = base + r;
+            }
+        } else if (fits) {
+            for (int i = threadIdx.x; i < nb; i += blockDim.x) b.parent[base + i] = uf_find_ro(b.parent, base + i);
+        }
+        if (threadIdx.x < nr) b.rowbase[y0 + threadIdx.x] = base + srb[threadIdx.x];
+        if (threadIdx.x == 0) {
+            const bool stalled = s_stalled;
+            if (stalled) atomicAdd(&counters[14], 1ull);
+            if (band == nbands - 1 || stalled) {
+                int total = base + nb;
+                if (band == nbands - 1) b.rowbase[d.H] = total;
+                if (total > maxruns || stalled) {
+                    // drop the frame (a stalled look-back leaves its run ids unknown): later kernels skip it
+                    atomicOr(&ctl[f].status, LFD_FRAME_OVERFLOW);
+                    ctl[f].active[0] = ctl[f].active[1] = 0;
+                    total = 0;
+                }
+                if (band == nbands - 1) ctl[f].nruns[kind] = total;
+            }
         }
     }
-    __syncthreads();
-    if (insm) {
-        volatile int* vp = sp;
-        for (int i = threadIdx.x; i < nb; i += blockDim.x) {
-            int r = i, pr;
-            while ((pr = vp[r]) != r) r = pr;
-            b.parent[base + i] = base + r;
-        }
-    } else {
-        for (int i = threadIdx.x; i < nb; i += blockDim.x) b.parent[base + i] = uf_find_ro(b.parent, base + i);
-    }
-    }   // band
 }
 
 // 4b. stitch the bands: rows y = k * CCL_BAND against row y-1; one warp per seam
 __global__ void __launch_bounds__(CCL_WARPS * 32)
-k_ccl_merge(const u32* __restrict__ mask, CclBuf* __restrict__ bufs, const FrameCtl* __restrict__ ctl,
-            int pass, Dims d, int kind)
+k_ccl_merge(CclBuf* __restrict__ bufs, const FrameCtl* __restrict__ ctl, int pass, Dims d, int kind)
 {
     int f = blockIdx.y;
     if (!ctl[f].active[pass]) return;
     int y = (blockIdx.x * CCL_WARPS + (threadIdx.x >> 5) + 1) * CCL_BAND;
     if (y >= d.H) return;
-    const u32* m = mask + (size_t)f * d.NW;
     CclBuf b = bufs[f];
     if (ctl[f].nruns[kind] == 0) return;
-    link_rows(m, b, y, d, kind, lane_id(), 32);
+    link_rows(b, y, kind, lane_id(), 32);
 }
 
 // Contour bookkeeping, one entry per selected component.

@@ -325,8 +325,7 @@ __device__ __forceinline__ void rect_warp_path(const int* __restrict__ rmin, con
 __global__ void __launch_bounds__(RECT_WARPS * 32)
 k_rects_warp(CompBuf* __restrict__ comps, RectBuf* __restrict__ rbufs, const CclBuf* __restrict__ ccl0,
              const CclBuf* __restrict__ ccl1, FrameCtl* __restrict__ ctl, int pass, int nframes,
-             Dims d, double minLen, double lwTresh, unsigned long long* __restrict__ counters,
-             const u32* __restrict__ edges, int external_only)
+             Dims d, double minLen, double lwTresh, unsigned long long* __restrict__ counters, int external_only)
 {
     extern __shared__ u32 rsm[];
     const int warp = threadIdx.x >> 5, lane = lane_id();
@@ -378,7 +377,7 @@ k_rects_warp(CompBuf* __restrict__ comps, RectBuf* __restrict__ rbufs, const Ccl
                 Run rr = fg.runs[comps[f].root[e]];
                 if (rr.xs == 0) keep = true;
                 else {
-                    int bid = run_at(edges + (size_t)f * d.NW, bg, rr.y, (int)rr.xs - 1, d, 1);
+                    int bid = run_at(bg, rr.y, (int)rr.xs - 1);
                     keep = (bg.flag[bg.parent[bid]] & 1) != 0;
                 }
             }

@@ -110,6 +110,8 @@ struct lfd_handle {
     float* clipped = nullptr;         // [N] lazily (run_pass writeback)
     int* labels_tap = nullptr;        // [N] lazily
     FrameCtl* ctl = nullptr;          // [2][B]: one bookkeeping block per pass (the passes run concurrently)
+    unsigned* look = nullptr;         // [2][2][B][look_stride]: k_ccl_band's ticket + look-back words per pass, kind, frame
+    int look_stride = 0;
     lfd_result* res_d = nullptr;      // [B]
     int64_t* counters_d = nullptr;    // [16]
     uint2* segs[2] = {nullptr, nullptr};     // per pass: [B][2][NW]
@@ -205,10 +207,14 @@ static int next_pow2(int v) { int p = 1; while (p < v) p <<= 1; return p; }
 // small bookkeeping kernels
 // ------------------------------------------------------------------------------------------------
 // ctl: [2][B] (one block per pass); block p only ever looks at active[p] / hough[p]
-__global__ void k_ctl_init(FrameCtl* ctl, int B, lfd_result* res, int n, int act0, int act1)
+// look: k_ccl_band's tickets and look-back words, [2 pass][2 kind][B][lstride] (nullptr where no labelling follows)
+__global__ void k_ctl_init(FrameCtl* ctl, int B, lfd_result* res, int n, int act0, int act1, unsigned* look, int lstride)
 {
     int f = blockIdx.x * blockDim.x + threadIdx.x;
     if (f >= n) return;
+    if (look)
+        for (int pk = 0; pk < 4; pk++)
+            for (int i = 0; i < lstride; i++) look[((size_t)pk * B + f) * lstride + i] = 0u;
     FrameCtl c;
     memset(&c, 0, sizeof(c));
     c.active[0] = act0; c.active[1] = act1;
@@ -483,19 +489,22 @@ static int create_impl(lfd_handle* h, int device, int max_batch, int H, int W, c
     DA(h->segs[0], (size_t)B * 2 * NW);
     DA(h->segs[1], (size_t)B * 2 * NW);
     const int MR = h->cfg.max_runs, MC = h->cfg.max_components;
+    h->look_stride = 1 + (H + CCL_BAND - 1) / CCL_BAND;
+    DA(h->look, (size_t)4 * B * h->look_stride);
     const int slotcap = 2 * MR + 4 * MC, hullcap = 2 * slotcap + 4 * MC;
     // one slab per field, sliced per frame; everything the two passes touch exists once per pass
     for (int p = 0; p < 2; p++)
     for (int k = 0; k < 2; k++) {
         h->ccl_h[p][k].resize(B);
-        Run* runs; int *parent, *flag, *ymax, *compidx, *rowbase, *rowcnt; u16* wpre;
+        Run* runs; int *parent, *flag, *ymax, *compidx, *rowbase;
         DA(runs, (size_t)B * MR); DA(parent, (size_t)B * MR); DA(flag, (size_t)B * MR); DA(ymax, (size_t)B * MR);
-        DA(compidx, (size_t)B * MR); DA(rowbase, (size_t)B * (H + 1)); DA(wpre, (size_t)B * NW); DA(rowcnt, (size_t)B * H);
+        DA(compidx, (size_t)B * MR); DA(rowbase, (size_t)B * (H + 1));
         for (int f = 0; f < B; f++) {
             CclBuf& c = h->ccl_h[p][k][f];
             c.runs = runs + (size_t)f * MR; c.parent = parent + (size_t)f * MR; c.flag = flag + (size_t)f * MR;
             c.ymax = ymax + (size_t)f * MR; c.compidx = compidx + (size_t)f * MR;
-            c.rowbase = rowbase + (size_t)f * (H + 1); c.wpre = wpre + (size_t)f * NW; c.rowcnt = rowcnt + (size_t)f * H;
+            c.rowbase = rowbase + (size_t)f * (H + 1);
+            c.look = h->look + ((size_t)(p * 2 + k) * B + f) * h->look_stride;
         }
         DA(h->ccl_d[p][k], (size_t)B);
         CK(cudaMemcpy(h->ccl_d[p][k], h->ccl_h[p][k].data(), B * sizeof(CclBuf), cudaMemcpyHostToDevice));
@@ -689,7 +698,6 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
     const bool taps = flags & LFD_KEEP_TAPS;
     const int tbase = 2 + pass * (T_PER_PASS - 1);   // event index preceding this pass's first stage
     HoughBufs& hb = h->hb[pass];
-    dim3 rows((d.H + CCL_WARPS * CCL_RC_ROWS - 1) / (CCL_WARPS * CCL_RC_ROWS), n);
     const int nbands = (d.H + CCL_BAND - 1) / CCL_BAND;
     dim3 bands((n >= 16 && nbands > CCL_BAND_CTAS) ? CCL_BAND_CTAS : nbands, n), seams((nbands + CCL_WARPS - 1) / CCL_WARPS, n);
 
@@ -765,12 +773,11 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
     KB_MARK(KB_NMS, 1);
     STAGE_EVENT(tbase + 2);
     // foreground runs: hysteresis + outer contours
-    k_ccl_rowcount<<<rows, CCL_WARPS * 32, 0, s>>>(v_cand, v_ccl0, C, pass, d, 0); LAUNCH_CHECK();
-    k_ccl_rowscan<<<n, 1024, 0, s>>>(v_ccl0, C, pass, d, 0, h->cfg.max_runs); LAUNCH_CHECK();
+    unsigned long long* const cnt = (unsigned long long*)h->counters_d;
     KB_MARK(KB_CCL_BAND_FG, 0);
-    k_ccl_band<<<bands, 256, ccl_band_smem(d.WW), s>>>(v_cand, v_ccl0, C, pass, d, 0); LAUNCH_CHECK();
+    k_ccl_band<<<bands, 256, ccl_band_smem(d.WW), s>>>(v_cand, v_ccl0, C, pass, d, 0, h->cfg.max_runs, cnt); LAUNCH_CHECK();
     KB_MARK(KB_CCL_BAND_FG, 1);
-    k_ccl_merge<<<seams, CCL_WARPS * 32, 0, s>>>(v_cand, v_ccl0, C, pass, d, 0); LAUNCH_CHECK();
+    k_ccl_merge<<<seams, CCL_WARPS * 32, 0, s>>>(v_ccl0, C, pass, d, 0); LAUNCH_CHECK();
     const dim3 flat(CCL_FLAT_CTAS, n);
     CK(cudaMemsetAsync(v_edges, 0, (size_t)n * d.NW * sizeof(u32), s));
     k_ccl_stats_flat<<<flat, 256, 0, s>>>(v_strong, v_ccl0, C, pass, d, 0); LAUNCH_CHECK();
@@ -778,19 +785,17 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
     k_ccl_extremes_flat<<<flat, 256, 0, s>>>(v_edges, v_ccl0, v_comp, C, pass, d, 0); LAUNCH_CHECK();
     STAGE_EVENT(tbase + 3);
     // background runs: hole contours
-    k_ccl_rowcount<<<rows, CCL_WARPS * 32, 0, s>>>(v_edges, v_ccl1, C, pass, d, 1); LAUNCH_CHECK();
-    k_ccl_rowscan<<<n, 1024, 0, s>>>(v_ccl1, C, pass, d, 1, h->cfg.max_runs); LAUNCH_CHECK();
     KB_MARK(KB_CCL_BAND_BG, 0);
-    k_ccl_band<<<bands, 256, ccl_band_smem(d.WW), s>>>(v_edges, v_ccl1, C, pass, d, 1); LAUNCH_CHECK();
+    k_ccl_band<<<bands, 256, ccl_band_smem(d.WW), s>>>(v_edges, v_ccl1, C, pass, d, 1, h->cfg.max_runs, cnt); LAUNCH_CHECK();
     KB_MARK(KB_CCL_BAND_BG, 1);
-    k_ccl_merge<<<seams, CCL_WARPS * 32, 0, s>>>(v_edges, v_ccl1, C, pass, d, 1); LAUNCH_CHECK();
+    k_ccl_merge<<<seams, CCL_WARPS * 32, 0, s>>>(v_ccl1, C, pass, d, 1); LAUNCH_CHECK();
     k_ccl_stats_flat<<<flat, 256, 0, s>>>(nullptr, v_ccl1, C, pass, d, 1); LAUNCH_CHECK();
     k_ccl_alloc_flat<<<flat, 256, 0, s>>>(v_ccl1, nullptr, v_comp, C, pass, d, 1); LAUNCH_CHECK();
     k_ccl_extremes_flat<<<flat, 256, 0, s>>>(v_edges, v_ccl1, v_comp, C, pass, d, 1); LAUNCH_CHECK();
     STAGE_EVENT(tbase + 4);
     // rectangles + box image
     KB_MARK(KB_RECTS, 0);
-    k_rects_warp<<<h->sm_count * 16, RECT_WARPS * 32, rects_smem(n), s>>>(v_comp, v_rbuf, v_ccl0, v_ccl1, C, pass, n, d, pp.minAreaRectMinLen, pp.lwTresh, (unsigned long long*)h->counters_d, v_edges, pp.contoursMode == 0 ? 1 : 0); LAUNCH_CHECK();
+    k_rects_warp<<<h->sm_count * 16, RECT_WARPS * 32, rects_smem(n), s>>>(v_comp, v_rbuf, v_ccl0, v_ccl1, C, pass, n, d, pp.minAreaRectMinLen, pp.lwTresh, (unsigned long long*)h->counters_d, pp.contoursMode == 0 ? 1 : 0); LAUNCH_CHECK();
     KB_MARK(KB_RECTS, 1);
     CK(cudaMemsetAsync(v_box, 0, (size_t)n * d.NW * sizeof(u32), s));
     k_fill_boxes<<<dim3(16, n), 128, 0, s>>>(v_rbuf, v_box, C, pass, d); LAUNCH_CHECK();
@@ -840,7 +845,7 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
                         !(flags & (LFD_SERIAL_PASSES | LFD_KEEP_TAPS | LFD_FULL_LINES)) && !h->ktiming;
     if (!replay) memset(h->kb_used, 0, sizeof(h->kb_used));       // a replayed graph records the brackets of its capture again
     if (h->ktiming) { h->kn = 0; ktime_mark(h, 0); }
-    k_ctl_init<<<(n + 127) / 128, 128, 0, s>>>(h->ctl, h->B, h->res_d, n, mode != 2, mode != 1); LAUNCH_CHECK();
+    k_ctl_init<<<(n + 127) / 128, 128, 0, s>>>(h->ctl, h->B, h->res_d, n, mode != 2, mode != 1, h->look, h->look_stride); LAUNCH_CHECK();
     CK(cudaMemsetAsync(h->hist, 0, (size_t)2 * h->B * 256 * sizeof(u32), s));
     if (mode == 0) {
         CK(cudaMemsetAsync(h->starmask, 0, (size_t)n * d.NW * sizeof(u32), s));
@@ -1255,7 +1260,7 @@ extern "C" int lfd_hough_lines(lfd_handle* h, const uint8_t* img, int height, in
     HoughBufs& hb = hs.hb;
     CK(cudaMemcpyAsync(hs.img, img, (size_t)d.N, cudaMemcpyHostToDevice, s));
     CK(cudaMemsetAsync(h->counters_d, 0, 16 * sizeof(int64_t), s));
-    k_ctl_init<<<1, 32, 0, s>>>(hs.ctl, 1, hs.res, 1, 1, 0); LAUNCH_CHECK();
+    k_ctl_init<<<1, 32, 0, s>>>(hs.ctl, 1, hs.res, 1, 1, 0, nullptr, 0); LAUNCH_CHECK();
     // mark Hough as enabled for pass 0
     FrameCtl c; memset(&c, 0, sizeof(c)); c.active[0] = 1; c.hough[0] = 1;
     CK(cudaMemcpyAsync(hs.ctl, &c, sizeof(c), cudaMemcpyHostToDevice, s));
@@ -1312,7 +1317,7 @@ extern "C" int lfd_canny(lfd_handle* h, const uint8_t* img, int low, int high, u
     const int pass = 0, n = 1;
     FrameCtl* const C = h->ctl;
     CK(cudaMemcpyAsync(h->morph[pass], img, (size_t)d.N, cudaMemcpyHostToDevice, s));
-    k_ctl_init<<<1, 32, 0, s>>>(h->ctl, h->B, h->res_d, 1, 1, 0); LAUNCH_CHECK();
+    k_ctl_init<<<1, 32, 0, s>>>(h->ctl, h->B, h->res_d, 1, 1, 0, h->look, h->look_stride); LAUNCH_CHECK();
     // device times -> lfd_get_timings entries 0..1 (Sobel + NMS incl. the input mask, hysteresis by run CCL)
     CK(cudaEventRecord(h->ev[0], s));
     k_pack_mask<<<592, 256, 0, s>>>(h->morph[pass], h->nz[pass], d); LAUNCH_CHECK();
@@ -1329,13 +1334,11 @@ extern "C" int lfd_canny(lfd_handle* h, const uint8_t* img, int low, int high, u
     }
     LAUNCH_CHECK();
     CK(cudaEventRecord(h->ev[1], s));
-    dim3 rows((d.H + CCL_WARPS * CCL_RC_ROWS - 1) / (CCL_WARPS * CCL_RC_ROWS), n);
     const int nbands = (d.H + CCL_BAND - 1) / CCL_BAND;
     dim3 bands(nbands, n), seams((nbands + CCL_WARPS - 1) / CCL_WARPS, n);
-    k_ccl_rowcount<<<rows, CCL_WARPS * 32, 0, s>>>(h->cand[pass], h->ccl_d[pass][0], C, pass, d, 0); LAUNCH_CHECK();
-    k_ccl_rowscan<<<n, 1024, 0, s>>>(h->ccl_d[pass][0], C, pass, d, 0, h->cfg.max_runs); LAUNCH_CHECK();
-    k_ccl_band<<<bands, 256, ccl_band_smem(d.WW), s>>>(h->cand[pass], h->ccl_d[pass][0], C, pass, d, 0); LAUNCH_CHECK();
-    k_ccl_merge<<<seams, CCL_WARPS * 32, 0, s>>>(h->cand[pass], h->ccl_d[pass][0], C, pass, d, 0); LAUNCH_CHECK();
+    k_ccl_band<<<bands, 256, ccl_band_smem(d.WW), s>>>(h->cand[pass], h->ccl_d[pass][0], C, pass, d, 0, h->cfg.max_runs,
+                                                      (unsigned long long*)h->counters_d); LAUNCH_CHECK();
+    k_ccl_merge<<<seams, CCL_WARPS * 32, 0, s>>>(h->ccl_d[pass][0], C, pass, d, 0); LAUNCH_CHECK();
     CK(cudaMemsetAsync(h->edges[pass], 0, (size_t)d.NW * sizeof(u32), s));
     k_ccl_stats_flat<<<dim3(CCL_FLAT_CTAS, n), 256, 0, s>>>(h->strong[pass], h->ccl_d[pass][0], C, pass, d, 0); LAUNCH_CHECK();
     k_ccl_alloc_flat<<<dim3(CCL_FLAT_CTAS, n), 256, 0, s>>>(h->ccl_d[pass][0], h->edges[pass], h->comp_d[pass], C, pass, d, 0); LAUNCH_CHECK();
@@ -1373,7 +1376,7 @@ extern "C" int lfd_fit_min_area_rect(lfd_handle* h, const uint8_t* img, int cont
     do {
         cudaError_t ce;
         if ((ce = cudaMemcpyAsync(h->morph[0], img, (size_t)d.N, cudaMemcpyHostToDevice, s)) != cudaSuccess) { h->err = cudaGetErrorString(ce); rc = LFD_E_CUDA; break; }
-        k_ctl_init<<<1, 32, 0, s>>>(h->ctl, h->B, h->res_d, 1, 1, 0);
+        k_ctl_init<<<1, 32, 0, s>>>(h->ctl, h->B, h->res_d, 1, 1, 0, h->look, h->look_stride);
         k_pack_mask<<<592, 256, 0, s>>>(h->morph[0], h->nz[0], d);
         h->launches += 2;
         h->cur_part = 0;

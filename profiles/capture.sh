@@ -14,7 +14,7 @@ ncu --set full --clock-control none --import-source on \
 echo "full capture rc=$?"
 # the small kernels of the CCL / geometry / Hough tail (source-level data for the next round of tuning)
 ncu --set full --clock-control none --import-source on \
-    -k regex:"k_ccl_merge|k_ccl_alloc|k_ccl_extremes|k_ccl_rowcount|k_ccl_rowscan|k_fill_boxes|k_hough_compact|k_hough_peaks|k_hough_topk|k_star_mask" -s 100 -c 40 \
+    -k regex:"k_ccl_merge|k_ccl_alloc|k_ccl_extremes|k_fill_boxes|k_hough_compact|k_hough_peaks|k_hough_topk|k_star_mask" -s 100 -c 40 \
     -o $OUT/prof_${TAG}_small -f $CMD > $OUT/ncu_s_$TAG.log 2>&1
 echo "small-kernel capture rc=$?"
 ncu -i $OUT/prof_$TAG.ncu-rep --page raw --csv > $OUT/prof_${TAG}_raw.csv 2>/dev/null
