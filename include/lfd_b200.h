@@ -86,7 +86,10 @@ enum lfd_stage {
     LFD_STAGE_ACCUM_BOX = 14,/* same for BOX */
     LFD_STAGE_LINES_EQU = 15,/* float32[n][2] (rho, theta) in cv2.HoughLines order; needs LFD_FULL_LINES */
     LFD_STAGE_LINES_BOX = 16,
-    LFD_STAGE_CLIPPED = 17   /* float32 H*W: the frame after the pass's in-place clip (processfield.py:342,453-454) */
+    LFD_STAGE_CLIPPED = 17,  /* float32 H*W: the frame after the pass's in-place clip (processfield.py:342,453-454) */
+    LFD_STAGE_INPUT = 18     /* float32 H*W: the un-flipped frame of a batch slot as the last whole-frame run read it, native
+                                byte order (swapped back after an LFD_INPUT_BIGENDIAN run); needs no LFD_KEEP_TAPS; `pass` is
+                                ignored.  LFD_E_STATE after lfd_run_pass / lfd_blot / a bare lfd_upload, which overwrite the slots */
 };
 
 /* one pass's parameters: the keys of params_bright / params_dim (detecttrails.py:202-230) */
@@ -147,6 +150,19 @@ typedef struct lfd_config {
     int32_t reserved[4];
 } lfd_config;
 
+/* one synthetic trail for lfd_submit_injected: the Gaussian line segment of lfd_b200/synth.py::_add_trail.  Pixel (x, y)
+ * gets peak * expf(-0.5f * (d / sigma)^2) added iff 0 <= t <= L and |d| <= ceil(5 * sigma) + 1, with, in float32,
+ * t = (x - x0) * ux + (y - y0) * uy, d = -(x - x0) * uy + (y - y0) * ux and ux, uy, L computed in double from the end
+ * points and rounded to float32 (oracle/inject_ref.py::render_trails).  A zero-length trail adds nothing; the frame
+ * edges clip the footprint. */
+typedef struct lfd_trail {
+    float x0, y0, x1, y1;   /* end points, UN-flipped FITS orientation, x = column, y = row, pixel centres at integers */
+    float sigma;            /* Gaussian cross-section sigma in px, finite and > 0 */
+    float peak;             /* added flux at the centre line, frame units, finite (may be negative) */
+} lfd_trail;
+
+#define LFD_MAX_INJECT_TRAILS 16   /* trails per batch slot */
+
 typedef struct lfd_handle lfd_handle;
 
 int lfd_abi_version(void);
@@ -188,7 +204,22 @@ int lfd_wait(lfd_handle* h, lfd_result* out /* n entries */);
 /* Device-resident variant used by the benchmark's `value` leg: runs the same pipeline on the frames
  * uploaded by the previous lfd_submit/lfd_upload without any host<->device copy of pixel data. */
 int lfd_upload(lfd_handle* h, const float* frames, int n, const int32_t* rects, const int32_t* rect_offsets, int flags);
+/* After lfd_submit_injected it re-runs the injected frames (they stay in the batch slots). */
 int lfd_run_resident(lfd_handle* h, int n, int flags);
+
+/* Injection and recovery (measuring what fraction of synthetic trails the detector finds).
+ * lfd_set_base uploads n_base native-order, un-flipped frames once into device memory the handle owns; their star
+ * rectangles follow lfd_submit's convention and max_star_rects check and are kept on the host.  A second call replaces
+ * the bases.  LFD_E_STATE while a batch is pending.
+ * lfd_submit_injected runs slot f on base_index[f] plus trails[trail_offsets[f] .. trail_offsets[f+1]) (trails and
+ * trail_offsets may both be NULL: no trails), with that base's rectangles: the trails are added on the device by
+ * k_inject just before the pipeline, so no pixel data crosses the host link.  It takes lfd_submit's flags except
+ * LFD_INPUT_BIGENDIAN; collect with lfd_wait.  LFD_E_ARG with nothing launched when n is outside 1..max_batch, a base
+ * index is out of range, a slot has more than LFD_MAX_INJECT_TRAILS trails, or a trail value is not finite or
+ * sigma <= 0; LFD_E_STATE when no base has been set.  k_inject's duration is lfd_get_kernel_times index 12. */
+int lfd_set_base(lfd_handle* h, const float* frames, int n_base, const int32_t* rects, const int32_t* rect_offsets);
+int lfd_submit_injected(lfd_handle* h, int n, const int32_t* base_index, const lfd_trail* trails,
+                        const int32_t* trail_offsets, int flags);
 
 /* One pass on one already flipped frame (process_field_bright / process_field_dim called directly).
  * If `writeback` != 0 the clipped float image is copied back into `img` (the reference mutates it). */
@@ -228,6 +259,7 @@ int lfd_get_timings(lfd_handle* h, float* ms, int max_entries, int* n_entries);
    of the last collected batch: CUDA events recorded on the launching stream on both sides of the launch - also inside
    the captured graph of the production path - so the durations are measured live, with the other streams running.
    index = 0 .. 11 (6 kernels x 2 passes); ms is summed over the batch parts, launches = number of parts.
+   index 12 = k_inject of the last collected lfd_submit_injected batch (always bracketed; launches 0 otherwise).
    Returns LFD_E_ARG past the last index. */
 int lfd_get_kernel_times(lfd_handle* h, int index, const char** name, int* pass, float* ms, int* launches);
 const char* lfd_timing_name(int i);

@@ -23,7 +23,9 @@ MAX_SET_LINES = 16
 
 STAGES = {"mask": 0, "gray": 1, "equ": 2, "eroded": 3, "morph": 4, "canny": 5, "box": 6, "hist": 7, "lut": 8,
           "nms": 9, "fg_labels": 10, "bg_labels": 11, "rects": 12, "accum_equ": 13, "accum_box": 14,
-          "lines_equ": 15, "lines_box": 16, "clipped": 17}
+          "lines_equ": 15, "lines_box": 16, "clipped": 17, "input": 18}
+MAX_INJECT_TRAILS = 16
+TRAIL_DTYPE = np.dtype([("x0", "<f4"), ("y0", "<f4"), ("x1", "<f4"), ("y1", "<f4"), ("sigma", "<f4"), ("peak", "<f4")])
 
 
 class PassParams(ctypes.Structure):
@@ -137,6 +139,12 @@ def lib():
                                        ctypes.c_double, ctypes.c_double, ctypes.c_longlong, ctypes.c_double,
                                        ctypes.POINTER(ctypes.c_char_p), ctypes.c_int, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_int,
                                        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]
+        for sym in ("lfd_set_base", "lfd_submit_injected"):     # added within ABI version 1: a stale build lacks them
+            if not hasattr(L, sym):
+                raise ImportError("liblfd_b200.so predates %s: rebuild it (`python -c 'import __graft_entry__ as g; g.build()'`)" % sym)
+        L.lfd_set_base.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]
+        L.lfd_submit_injected.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                          ctypes.c_int]
         if L.lfd_abi_version() != 1:
             raise ImportError("liblfd_b200.so ABI mismatch")
         _lib = L
@@ -375,6 +383,42 @@ class Handle:
         self._keep = None
         return np.frombuffer(self._results, dtype=np.dtype(Result), count=self._n).copy()
 
+    def set_base(self, frames, rects_per_frame=None):
+        """Upload (n_base, H, W) native-order, un-flipped float32 frames once as injection bases, with their star
+        rectangles (lfd_submit's convention); a second call replaces them (include/lfd_b200.h: lfd_set_base)."""
+        frames = np.ascontiguousarray(frames, dtype=np.float32)
+        if frames.ndim != 3 or frames.shape[1:] != (self.H, self.W):
+            raise ValueError("frames must have shape (n, %d, %d)" % (self.H, self.W))
+        _flat, _offs, rp, op = self._rects_arrays(rects_per_frame)
+        self._ck(self._L.lfd_set_base(self.h, frames.ctypes.data_as(ctypes.c_void_p), frames.shape[0], rp, op))
+
+    @staticmethod
+    def trails_array(trails):
+        """Trails as synth's dicts {p0: (x, y), p1: (x, y), sigma, peak} -> a TRAIL_DTYPE array (float32 fields)."""
+        out = np.zeros(len(trails), TRAIL_DTYPE)
+        for i, t in enumerate(trails):
+            out[i] = (t["p0"][0], t["p0"][1], t["p1"][0], t["p1"][1], t["sigma"], t["peak"])
+        return out
+
+    def submit_injected(self, base_index, trails_per_slot=None, flags=0):
+        """Run slot f on base base_index[f] plus the trails trails_per_slot[f] (synth's dicts), added on the device;
+        collect with wait() (include/lfd_b200.h: lfd_submit_injected)."""
+        bidx = np.ascontiguousarray(base_index, np.int32)
+        n = len(bidx)
+        tp, op = None, None
+        if trails_per_slot is not None:
+            if len(trails_per_slot) != n:
+                raise ValueError("trails_per_slot must have one entry per slot")
+            offs = np.zeros(n + 1, np.int32)
+            for i, ts in enumerate(trails_per_slot):
+                offs[i + 1] = offs[i] + len(ts)
+            arr = np.zeros(max(int(offs[-1]), 1), TRAIL_DTYPE)
+            if offs[-1]:
+                arr[:offs[-1]] = np.concatenate([self.trails_array(ts) for ts in trails_per_slot if len(ts)])
+            tp, op = arr.ctypes.data_as(ctypes.c_void_p), offs.ctypes.data_as(ctypes.c_void_p)
+        self._ck(self._L.lfd_submit_injected(self.h, n, bidx.ctypes.data_as(ctypes.c_void_p), tp, op, flags))
+        self._n = n
+
     def run_pass(self, pass_, img, flags=0, writeback=True):
         if img.dtype != np.float32 or not img.flags["C_CONTIGUOUS"] or img.shape != (self.H, self.W):
             raise ValueError("img must be a C-contiguous float32 array of shape (%d, %d)" % (self.H, self.W))
@@ -405,7 +449,7 @@ class Handle:
             out = np.empty(256, np.uint8)
         elif stage in ("fg_labels", "bg_labels"):
             out = np.empty((H, W), np.int32)
-        elif stage == "clipped":
+        elif stage in ("clipped", "input"):
             out = np.empty((H, W), np.float32)
         elif stage == "rects":
             out = np.zeros(self.stage_count(frame, pass_, stage), RECT_DTYPE)

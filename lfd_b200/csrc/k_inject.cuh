@@ -1,0 +1,115 @@
+// k_inject.cuh - on-device trail injection for completeness campaigns (lfd_set_base / lfd_submit_injected).
+//
+// in[f] = base[base_index[f]] + the Gaussian line segments of slot f, the trail of lfd_b200/synth.py::_add_trail with
+// the tails beyond |d| = ceil(5 sigma) + 1 dropped (oracle/inject_ref.py::render_trails is the checker).  Per pixel,
+// in float32 and in _add_trail's operation order:
+//   t = (x - x0) * ux + (y - y0) * uy,   d = -(x - x0) * uy + (y - y0) * ux
+//   pixel += peak * expf(-0.5f * (d / sigma)^2)   iff 0 <= t <= L and |d| <= pad
+// with ux, uy, L rounded to float32 from double on the host.  Every product and sum is an explicit round-to-nearest
+// intrinsic, so footprint membership is bit-identical to the NumPy reference and only expf may differ in the last bits.
+#pragma once
+#include "common.cuh"
+
+#define INJ_ROWS 8                  // frame rows per CTA
+#define INJ_THREADS 256
+
+// one trail as the kernel uses it (host-prepared from lfd_trail); L == 0 marks a zero-length trail (adds nothing)
+struct InjTrail {
+    float x0, y0, ux, uy, L, sigma, peak, pad;
+};
+
+// Conservative x-range [lo, hi] of the pixels of row y the float32 test can accept: the exact interval of the rotated
+// rectangle, widened by `slack` in t and d (far more than the float32 rounding of t and d) and by one pixel.
+__device__ __forceinline__ int2 inj_row_range(const InjTrail& T, int y, int W)
+{
+    const double slack = 1e-5 * (fabs((double)T.x0) + fabs((double)T.y0) + (double)W + (double)y) + 1e-3;
+    double lo = 0.0, hi = (double)(W - 1);
+    const double yy = (double)y - (double)T.y0;
+    // t(x) = ux * (x - x0) + yy * uy in [-slack, L + slack];  d(x) = -uy * (x - x0) + yy * ux in [-pad - slack, pad + slack]
+    const double c[2] = {(double)T.ux, -(double)T.uy};
+    const double o[2] = {yy * (double)T.uy, yy * (double)T.ux};
+    const double a[2] = {-slack, -(double)T.pad - slack};
+    const double b[2] = {(double)T.L + slack, (double)T.pad + slack};
+    for (int k = 0; k < 2; k++) {
+        if (c[k] == 0.0) {
+            if (o[k] < a[k] || o[k] > b[k]) return make_int2(1, 0);
+            continue;
+        }
+        double u = (a[k] - o[k]) / c[k] + (double)T.x0, v = (b[k] - o[k]) / c[k] + (double)T.x0;
+        if (u > v) { double s = u; u = v; v = s; }
+        lo = fmax(lo, u - 1.0);
+        hi = fmin(hi, v + 1.0);
+    }
+    if (!(lo <= hi)) return make_int2(1, 0);
+    return make_int2((int)floor(lo), (int)ceil(hi));
+}
+
+// grid (ceil(H / INJ_ROWS), n), INJ_THREADS threads; W % 4 == 0 (lfd_create)
+__global__ void __launch_bounds__(INJ_THREADS)
+k_inject(const float* __restrict__ base, const int* __restrict__ base_index, const InjTrail* __restrict__ trails,
+         const int* __restrict__ trail_off, float* __restrict__ out, Dims d)
+{
+    __shared__ InjTrail st[LFD_MAX_INJECT_TRAILS];
+    __shared__ int2 rng[INJ_ROWS][LFD_MAX_INJECT_TRAILS];
+    __shared__ int2 urng[INJ_ROWS];           // union of the row's ranges: outside it a float4 is copied as is
+    const int f = blockIdx.y, y0 = blockIdx.x * INJ_ROWS, tid = threadIdx.x;
+    const int t0 = trail_off[f], nt = trail_off[f + 1] - t0;
+    const int rows = min(INJ_ROWS, d.H - y0);
+    if (tid < nt) st[tid] = trails[t0 + tid];
+    __syncthreads();
+    for (int i = tid; i < rows * nt; i += INJ_THREADS) {
+        const int r = i / nt, k = i - r * nt;
+        rng[r][k] = st[k].L > 0.f ? inj_row_range(st[k], y0 + r, d.W) : make_int2(1, 0);
+    }
+    __syncthreads();
+    if (tid < rows) {
+        int lo = d.W, hi = -1;
+        for (int k = 0; k < nt; k++) { const int2 q = rng[tid][k]; if (q.x <= q.y) { lo = min(lo, q.x); hi = max(hi, q.y); } }
+        urng[tid] = make_int2(lo, hi);
+    }
+    __syncthreads();
+    const int W4 = d.W >> 2;
+    const float4* src = reinterpret_cast<const float4*>(base + (size_t)base_index[f] * d.N + (size_t)y0 * d.W);
+    float4* dst = reinterpret_cast<float4*>(out + (size_t)f * d.N + (size_t)y0 * d.W);
+    const int total = rows * W4;
+    // four independent 16-byte loads in flight per thread before any store
+    for (int i0 = tid; i0 < total; i0 += 4 * INJ_THREADS) {
+        float4 v[4];
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const int i = i0 + j * INJ_THREADS;
+            if (i < total) v[j] = __ldcs(src + i);
+        }
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const int i = i0 + j * INJ_THREADS;
+            if (i >= total) break;
+            const int r = i / W4, x4 = (i - r * W4) << 2;
+            const int2 u = urng[r];
+            if (x4 + 3 >= u.x && x4 <= u.y) {
+                const float yf = (float)(y0 + r);
+                float* e = &v[j].x;
+#pragma unroll
+                for (int c = 0; c < 4; c++) {
+                    const int x = x4 + c;
+                    const float xf = (float)x;
+                    float acc = e[c];
+                    for (int k = 0; k < nt; k++) {
+                        const int2 q = rng[r][k];
+                        if (x < q.x || x > q.y) continue;
+                        const InjTrail& T = st[k];
+                        const float ax = __fsub_rn(xf, T.x0), by = __fsub_rn(yf, T.y0);
+                        const float t = __fadd_rn(__fmul_rn(ax, T.ux), __fmul_rn(by, T.uy));
+                        const float dd = __fadd_rn(-__fmul_rn(ax, T.uy), __fmul_rn(by, T.ux));
+                        if (t >= 0.f && t <= T.L && fabsf(dd) <= T.pad) {
+                            const float q2 = __fdiv_rn(dd, T.sigma);
+                            acc = __fadd_rn(acc, __fmul_rn(T.peak, expf(__fmul_rn(-0.5f, __fmul_rn(q2, q2)))));
+                        }
+                    }
+                    e[c] = acc;
+                }
+            }
+            dst[i] = v[j];
+        }
+    }
+}

@@ -23,6 +23,7 @@
 #include "k_canny.cuh"
 #include "k_ccl.cuh"
 #include "k_hough.cuh"
+#include "k_inject.cuh"
 #include "k_morph.cuh"
 #include "k_prep.cuh"
 #include "k_rects.cuh"
@@ -89,6 +90,8 @@ struct lfd_handle {
     int64_t launches = 0;
     int last_n = 0, last_flags = 0;
     bool pending = false;
+    // what h->in holds: the un-flipped frames the last whole-frame run read (LFD_STAGE_INPUT), in FITS byte order if in_be
+    bool in_whole = false, in_be = false;
 
     // device
     float* in = nullptr;              // [B][N]
@@ -123,6 +126,20 @@ struct lfd_handle {
     std::vector<RectBuf> rbuf_h[2];
     std::vector<void*> allocs;
     HoughBufs hb[2];
+    // injection campaigns (lfd_set_base / lfd_submit_injected): resident base frames and per-slot trails
+    float* base_d = nullptr;          // [base_cap][N], replaced by lfd_set_base
+    int n_base = 0, base_cap = 0;
+    std::vector<int4> base_rects;     // star rectangles of the bases (host), base_rect_off[n_base + 1] indexes them
+    std::vector<int> base_rect_off;
+    InjTrail* inj_trails_d = nullptr; // [B * LFD_MAX_INJECT_TRAILS]
+    int* inj_off_d = nullptr;         // [B + 1]
+    int* inj_base_d = nullptr;        // [B]
+    InjTrail* inj_trails_h = nullptr; // pinned staging of the three above
+    int* inj_off_h = nullptr;
+    int* inj_base_h = nullptr;
+    cudaEvent_t ev_inj[2] = {nullptr, nullptr};   // around k_inject; inj_recorded: the last run was lfd_submit_injected
+    bool inj_recorded = false;
+    float inj_ms = 0.f;
 
     // host
     float* frames_h = nullptr;        // pinned [B][N]
@@ -377,6 +394,11 @@ extern "C" int lfd_destroy(lfd_handle* h)
     if (h->rects_h) cudaFreeHost(h->rects_h);
     if (h->rect_off_h) cudaFreeHost(h->rect_off_h);
     if (h->ctl_h) cudaFreeHost(h->ctl_h);
+    if (h->base_d) cudaFree(h->base_d);
+    if (h->inj_trails_h) cudaFreeHost(h->inj_trails_h);
+    if (h->inj_off_h) cudaFreeHost(h->inj_off_h);
+    if (h->inj_base_h) cudaFreeHost(h->inj_base_h);
+    for (int i = 0; i < 2; i++) if (h->ev_inj[i]) cudaEventDestroy(h->ev_inj[i]);
     if (h->counters_h) cudaFreeHost(h->counters_h);
     for (int i = 0; i <= N_TIMINGS; i++) if (h->ev_valid[i]) cudaEventDestroy(h->ev[i]);
     for (int k = 0; k < LFD_BATCH_PARTS; k++)
@@ -839,6 +861,7 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
     const Dims d = h->d;
     cudaStream_t s = h->stream;
     if (!h->have_params) { h->err = "lfd_set_params has not been called"; return LFD_E_STATE; }
+    h->inj_recorded = false;           // lfd_submit_injected sets it after this returns
     CK(cudaMemsetAsync(h->counters_d, 0, 16 * sizeof(int64_t), s));
     CK(cudaEventRecord(h->ev[0], s));
     const bool replay = h->graph_exec && h->use_graphs && h->graph_n == n && h->graph_flags == flags && mode == 0 &&
@@ -950,6 +973,7 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
     }
     CK(cudaEventRecord(h->ev[N_TIMINGS], s));
     h->last_n = n; h->last_flags = flags; h->pending = true;
+    h->in_whole = mode == 0; h->in_be = be != 0;
     return LFD_OK;
 }
 
@@ -1004,6 +1028,7 @@ extern "C" int lfd_upload(lfd_handle* h, const float* frames, int n, const int32
     }
     if (ce != cudaSuccess) { h->err = std::string("cudaMemcpyAsync(H2D): ") + cudaGetErrorString(ce); return LFD_E_CUDA; }
     h->last_flags = flags;
+    h->in_whole = false;
     return LFD_OK;
 }
 
@@ -1035,6 +1060,117 @@ extern "C" int lfd_run_resident(lfd_handle* h, int n, int flags)
     return run_pipeline(h, n, flags, 0, false);
 }
 
+// ------------------------------------------------------------------------------------------------
+// injection campaigns: resident bases + per-slot synthetic trails added on the device before k_prep
+// ------------------------------------------------------------------------------------------------
+extern "C" int lfd_set_base(lfd_handle* h, const float* frames, int n_base, const int32_t* rects, const int32_t* rect_offsets)
+{
+    if (!h) return LFD_E_ARG;
+    if (!frames || n_base < 1) { h->err = "lfd_set_base: frames must be non-NULL and n_base >= 1"; return LFD_E_ARG; }
+    cudaSetDevice(h->device);
+    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    if (rects && rect_offsets) {
+        if (rect_offsets[0] != 0) { h->err = "rect_offsets[0] must be 0"; return LFD_E_ARG; }
+        for (int f = 0; f < n_base; f++) {
+            int c = rect_offsets[f + 1] - rect_offsets[f];
+            if (c < 0 || c > h->cfg.max_star_rects) { h->err = "too many star rectangles for a frame (lfd_config.max_star_rects)"; return LFD_E_CAPACITY; }
+        }
+    }
+    const size_t N = h->d.N;
+    if (n_base > h->base_cap) {
+        if (h->base_d) { cudaFree(h->base_d); h->base_d = nullptr; }
+        h->base_cap = 0; h->n_base = 0;
+        CK(cudaMalloc((void**)&h->base_d, (size_t)n_base * N * sizeof(float)));
+        h->base_cap = n_base;
+    }
+    if (!h->inj_trails_d) {
+        int rc;
+        if ((rc = dev_alloc(h, &h->inj_trails_d, (size_t)h->B * LFD_MAX_INJECT_TRAILS)) != LFD_OK) return rc;
+        if ((rc = dev_alloc(h, &h->inj_off_d, (size_t)h->B + 1)) != LFD_OK) return rc;
+        if ((rc = dev_alloc(h, &h->inj_base_d, (size_t)h->B)) != LFD_OK) return rc;
+        CK(cudaMallocHost((void**)&h->inj_trails_h, (size_t)h->B * LFD_MAX_INJECT_TRAILS * sizeof(InjTrail)));
+        CK(cudaMallocHost((void**)&h->inj_off_h, ((size_t)h->B + 1) * sizeof(int)));
+        CK(cudaMallocHost((void**)&h->inj_base_h, (size_t)h->B * sizeof(int)));
+        for (int i = 0; i < 2; i++) CK(cudaEventCreate(&h->ev_inj[i]));
+    }
+    h->n_base = 0;
+    CK(cudaMemcpyAsync(h->base_d, frames, (size_t)n_base * N * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));          // the caller may free `frames` on return
+    h->base_rect_off.assign((size_t)n_base + 1, 0);
+    h->base_rects.clear();
+    if (rects && rect_offsets) {
+        for (int f = 0; f <= n_base; f++) h->base_rect_off[f] = rect_offsets[f];
+        h->base_rects.assign((const int4*)rects, (const int4*)rects + rect_offsets[n_base]);
+    }
+    h->n_base = n_base;
+    return LFD_OK;
+}
+
+extern "C" int lfd_submit_injected(lfd_handle* h, int n, const int32_t* base_index, const lfd_trail* trails,
+                                   const int32_t* trail_offsets, int flags)
+{
+    if (!h) return LFD_E_ARG;
+    cudaSetDevice(h->device);
+    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    if (h->n_base < 1) { h->err = "no base frames (call lfd_set_base)"; return LFD_E_STATE; }
+    if (n < 1 || n > h->B || !base_index) { h->err = "bad batch size or base_index"; return LFD_E_ARG; }
+    if (flags & LFD_INPUT_BIGENDIAN) { h->err = "injected frames are built in native byte order (LFD_INPUT_BIGENDIAN)"; return LFD_E_ARG; }
+    if (!trails != !trail_offsets || (trail_offsets && trail_offsets[0] != 0)) { h->err = "bad trails / trail_offsets"; return LFD_E_ARG; }
+    // validate everything before anything is staged or launched
+    for (int f = 0; f < n; f++) {
+        if (base_index[f] < 0 || base_index[f] >= h->n_base) { h->err = "base_index out of range"; return LFD_E_ARG; }
+        if (!trail_offsets) continue;
+        const int c = trail_offsets[f + 1] - trail_offsets[f];
+        if (c < 0 || c > LFD_MAX_INJECT_TRAILS) { h->err = "a slot has more than LFD_MAX_INJECT_TRAILS trails"; return LFD_E_ARG; }
+        for (int k = trail_offsets[f]; k < trail_offsets[f + 1]; k++) {
+            const lfd_trail& t = trails[k];
+            if (!isfinite(t.x0) || !isfinite(t.y0) || !isfinite(t.x1) || !isfinite(t.y1) || !isfinite(t.sigma) ||
+                !isfinite(t.peak) || !(t.sigma > 0.f)) { h->err = "trail values must be finite with sigma > 0"; return LFD_E_ARG; }
+        }
+    }
+    // per-slot star rectangles from the slot's base, into the lfd_submit staging
+    int total = 0;
+    for (int f = 0; f < n; f++) {
+        const int b = base_index[f], c = h->base_rect_off[b + 1] - h->base_rect_off[b];
+        h->rect_off_h[f] = total;
+        if (c) memcpy(h->rects_h + total, h->base_rects.data() + h->base_rect_off[b], (size_t)c * sizeof(int4));
+        total += c;
+    }
+    h->rect_off_h[n] = total;
+    if (total) CK(cudaMemcpyAsync(h->rects_d, h->rects_h, (size_t)total * sizeof(int4), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->rect_off_d, h->rect_off_h, ((size_t)n + 1) * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    // trails in the kernel's form: unit vector and length in double from the float32 end points, rounded to float32
+    int nt = 0;
+    for (int f = 0; f < n; f++) {
+        h->inj_base_h[f] = base_index[f];
+        h->inj_off_h[f] = nt;
+        if (!trail_offsets) continue;
+        for (int k = trail_offsets[f]; k < trail_offsets[f + 1]; k++) {
+            const lfd_trail& t = trails[k];
+            const double dx = (double)t.x1 - (double)t.x0, dy = (double)t.y1 - (double)t.y0, L = hypot(dx, dy);
+            InjTrail& q = h->inj_trails_h[nt++];
+            q.x0 = t.x0; q.y0 = t.y0; q.sigma = t.sigma; q.peak = t.peak;
+            q.L = (float)L;
+            q.ux = L > 0 ? (float)(dx / L) : 0.f;
+            q.uy = L > 0 ? (float)(dy / L) : 0.f;
+            q.pad = (float)(ceil(5.0 * (double)t.sigma) + 1.0);
+            if (L == 0) q.L = 0.f;
+        }
+    }
+    h->inj_off_h[n] = nt;
+    if (nt) CK(cudaMemcpyAsync(h->inj_trails_d, h->inj_trails_h, (size_t)nt * sizeof(InjTrail), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->inj_off_d, h->inj_off_h, ((size_t)n + 1) * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->inj_base_d, h->inj_base_h, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaEventRecord(h->ev_inj[0], h->stream));
+    k_inject<<<dim3((h->d.H + INJ_ROWS - 1) / INJ_ROWS, n), INJ_THREADS, 0, h->stream>>>(h->base_d, h->inj_base_d, h->inj_trails_d,
+                                                                                       h->inj_off_d, h->in, h->d); LAUNCH_CHECK();
+    CK(cudaEventRecord(h->ev_inj[1], h->stream));
+    int rc = run_pipeline(h, n, flags, 0, false);
+    if (rc != LFD_OK) return rc;
+    h->inj_recorded = true;
+    return LFD_OK;
+}
+
 extern "C" int lfd_wait(lfd_handle* h, lfd_result* out)
 {
     if (!h) return LFD_E_ARG;
@@ -1060,6 +1196,8 @@ extern "C" int lfd_wait(lfd_handle* h, lfd_result* out)
                 h->kb_ms[p][b] += ms;
                 h->kb_launches[p][b]++;
             }
+    h->inj_ms = 0.f;
+    if (h->inj_recorded && cudaEventElapsedTime(&h->inj_ms, h->ev_inj[0], h->ev_inj[1]) != cudaSuccess) { h->inj_ms = 0.f; cudaGetLastError(); }
     if (out) memcpy(out, h->res_h, (size_t)h->last_n * sizeof(lfd_result));
     return LFD_OK;
 }
@@ -1067,7 +1205,15 @@ extern "C" int lfd_wait(lfd_handle* h, lfd_result* out)
 // Bracketed kernels of the last collected batch: name, pass, summed duration over the batch parts and number of launches.
 extern "C" int lfd_get_kernel_times(lfd_handle* h, int index, const char** name, int* pass, float* ms, int* launches)
 {
-    if (!h || index < 0 || index >= 2 * KB_COUNT) return LFD_E_ARG;
+    if (!h || index < 0 || index > 2 * KB_COUNT) return LFD_E_ARG;
+    if (index == 2 * KB_COUNT) {       // k_inject, bracketed on every lfd_submit_injected (outside the graph)
+        const bool on = h->inj_recorded && !h->pending;
+        if (name) *name = "k_inject";
+        if (pass) *pass = 0;
+        if (ms) *ms = on ? h->inj_ms : 0.f;
+        if (launches) *launches = on ? 1 : 0;
+        return LFD_OK;
+    }
     const int p = index / KB_COUNT, b = index % KB_COUNT;
     if (name) *name = k_bracket_names[b];
     if (pass) *pass = p;
@@ -1110,6 +1256,7 @@ extern "C" int lfd_blot(lfd_handle* h, float* img, const int32_t* rects, int nre
     if (nrects == 0) return LFD_OK;
     memcpy(h->rects_h, rects, (size_t)nrects * sizeof(int4));
     CK(cudaMemcpyAsync(h->rects_d, h->rects_h, (size_t)nrects * sizeof(int4), cudaMemcpyHostToDevice, h->stream));
+    h->in_whole = false;
     CK(cudaMemcpyAsync(h->in, img, (size_t)h->d.N * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     k_blot<<<nrects, 128, 0, h->stream>>>(h->in, h->rects_d, nrects, h->d); LAUNCH_CHECK();
     CK(cudaMemcpyAsync(img, h->in, (size_t)h->d.N * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
@@ -1211,11 +1358,18 @@ extern "C" int lfd_get_stage(lfd_handle* h, int frame, int pass, int stage, void
     case LFD_STAGE_CLIPPED:
         if (!h->clipped) { h->err = "clipped image not recorded"; return LFD_E_STATE; }
         src = h->clipped; need = N * sizeof(float); break;
+    case LFD_STAGE_INPUT:
+        if (!h->in_whole) { h->err = "the batch slots do not hold the frames of a whole-frame run"; return LFD_E_STATE; }
+        src = h->in + (size_t)frame * N; need = N * sizeof(float); break;
     default: h->err = "unknown stage"; return LFD_E_ARG;
     }
     if (bytes < need) { h->err = "buffer too small"; return LFD_E_ARG; }
     CK(cudaMemcpyAsync(host_out, src, need, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
+    if (stage == LFD_STAGE_INPUT && h->in_be) {        // a raw FITS payload: back to native order
+        uint32_t* w = (uint32_t*)host_out;
+        for (size_t i = 0; i < N; i++) w[i] = __builtin_bswap32(w[i]);
+    }
     return LFD_OK;
 }
 
