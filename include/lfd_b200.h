@@ -249,7 +249,9 @@ int lfd_smem_atomic_peak(lfd_handle* h, double* gops);
 
 /* fit_minAreaRect(img, contoursMode, contoursMethod, minAreaRectMinLen, lwTresh) of processfield.py:201-263 on a host
  * uint8 image of the handle's frame size: Canny(0,255) -> findContours -> minAreaRect filter -> fillPoly.
- * box_out: uint8 height*width (0/255) = box_img; *detection = the function's first return value. */
+ * box_out: uint8 height*width (0/255) = box_img; *detection = the function's first return value.
+ * It runs as frame 0 of the bright pass: afterwards the CANNY, FG/BG_LABELS, RECTS and BOX taps of (0, LFD_PASS_BRIGHT)
+ * and lfd_get_counters describe this call (the taps need a whole-frame run or lfd_run_pass earlier on the handle). */
 int lfd_fit_min_area_rect(lfd_handle* h, const uint8_t* img, int contoursMode, int contoursMethod,
                           double minAreaRectMinLen, double lwTresh, uint8_t* box_out, int* detection);
 
@@ -305,6 +307,7 @@ int lfd_ingest_batch(void* staging, int height, int width, int n, const char* co
                      int32_t* status_cat, int nthreads);
 /* Work counters of the last run, summed over the batch: [0] nonzero px voted equ, [1] box, [2] votes,
  * [3] runs fg, [4] runs bg, [5] contours, [6] passing rects, [7] frames that ran dim, [8] frames that ran Hough,
+ * [11] contours whose rectangle a whole warp computed, [12] of those, short contours handed over because their thread's hull stack was full,
  * [14] labelling bands whose run-id look-back gave up waiting (frame reported LFD_FRAME_OVERFLOW; expected 0). */
 int lfd_get_counters(lfd_handle* h, int64_t* out, int n);
 

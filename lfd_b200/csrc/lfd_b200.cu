@@ -1529,7 +1529,8 @@ extern "C" int lfd_fit_min_area_rect(lfd_handle* h, const uint8_t* img, int cont
     int rc = LFD_OK;
     do {
         cudaError_t ce;
-        if ((ce = cudaMemcpyAsync(h->morph[0], img, (size_t)d.N, cudaMemcpyHostToDevice, s)) != cudaSuccess) { h->err = cudaGetErrorString(ce); rc = LFD_E_CUDA; break; }
+        if ((ce = cudaMemcpyAsync(h->morph[0], img, (size_t)d.N, cudaMemcpyHostToDevice, s)) != cudaSuccess ||
+            (ce = cudaMemsetAsync(h->counters_d, 0, 16 * sizeof(int64_t), s)) != cudaSuccess) { h->err = cudaGetErrorString(ce); rc = LFD_E_CUDA; break; }
         k_ctl_init<<<1, 32, 0, s>>>(h->ctl, h->B, h->res_d, 1, 1, 0, h->look, h->look_stride);
         k_pack_mask<<<592, 256, 0, s>>>(h->morph[0], h->nz[0], d);
         h->launches += 2;
@@ -1540,7 +1541,12 @@ extern "C" int lfd_fit_min_area_rect(lfd_handle* h, const uint8_t* img, int cont
         FrameCtl out;
         if ((ce = cudaMemcpyAsync(&out, h->ctl, sizeof(out), cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
             (ce = cudaMemcpyAsync(box_out, h->tap_u8, (size_t)d.N, cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
+            (ce = cudaMemcpyAsync(h->counters_h, h->counters_d, 16 * sizeof(int64_t), cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
             (ce = cudaStreamSynchronize(s)) != cudaSuccess) { h->err = cudaGetErrorString(ce); rc = LFD_E_CUDA; break; }
+        // the RECTS tap of (frame 0, bright pass) reads its counts from the host copy of the frame's control block; no
+        // k_check_theta runs here to save them, so save this call's own counts
+        h->ctl_h[0].ncomp_saved[0][0] = out.ncomp[0];
+        h->ctl_h[0].ncomp_saved[0][1] = out.ncomp[1];
         if (out.status & LFD_FRAME_OVERFLOW) { h->err = "per-frame work list overflow (lfd_config.max_runs / max_components)"; rc = LFD_E_CAPACITY; break; }
         *detection = out.hough[0] ? 1 : 0;
     } while (0);

@@ -158,6 +158,8 @@ def contour_point_sets(edges):
     bg = label_bg4(edges)
     out = []
     ys, xs = np.nonzero(fg >= 0)
+    if len(ys) == 0:
+        return out          # no edge pixel: no contour, and no hole either
     labs = fg[ys, xs]
     order = np.argsort(labs, kind="stable")
     ys, xs, labs = ys[order], xs[order], labs[order]
