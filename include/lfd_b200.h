@@ -84,7 +84,8 @@ enum lfd_stage {
     LFD_STAGE_RECTS = 12,    /* lfd_rect[n]; count via lfd_get_stage_count */
     LFD_STAGE_ACCUM_EQU = 13,/* int32 (numangle+2)*(numrho+2) Hough accumulator of MORPH */
     LFD_STAGE_ACCUM_BOX = 14,/* same for BOX */
-    LFD_STAGE_LINES_EQU = 15,/* float32[n][2] (rho, theta) in cv2.HoughLines order; needs LFD_FULL_LINES */
+    LFD_STAGE_LINES_EQU = 15,/* float32[n][2] (rho, theta) in cv2.HoughLines order; needs LFD_FULL_LINES; n via
+                                lfd_get_stage_count: n_lines, capped at the handle's max_lines */
     LFD_STAGE_LINES_BOX = 16,
     LFD_STAGE_CLIPPED = 17,  /* float32 H*W: the frame after the pass's in-place clip (processfield.py:342,453-454) */
     LFD_STAGE_INPUT = 18     /* float32 H*W: the un-flipped frame of a batch slot as the last whole-frame run read it, native

@@ -1278,8 +1278,9 @@ extern "C" int lfd_get_stage_count(lfd_handle* h, int frame, int pass, int stage
         *count = min(ch.ncomp_saved[pass][0], h->cfg.max_components) + min(ch.ncomp_saved[pass][1], h->cfg.max_components);
         return LFD_OK;
     }
-    case LFD_STAGE_LINES_EQU: *count = h->res_h[frame].n_lines_equ[pass]; return LFD_OK;
-    case LFD_STAGE_LINES_BOX: *count = h->res_h[frame].n_lines_box[pass]; return LFD_OK;
+    // the lines the tap holds: k_hough_sort keeps at most max_lines of them (n_lines in lfd_result is the full count)
+    case LFD_STAGE_LINES_EQU: *count = min(h->res_h[frame].n_lines_equ[pass], hb.max_lines); return LFD_OK;
+    case LFD_STAGE_LINES_BOX: *count = min(h->res_h[frame].n_lines_box[pass], hb.max_lines); return LFD_OK;
     case LFD_STAGE_ACCUM_EQU:
     case LFD_STAGE_ACCUM_BOX: *count = (int)hb.accum_stride; return LFD_OK;
     default: h->err = "stage has no count"; return LFD_E_ARG;
