@@ -164,6 +164,32 @@ typedef struct lfd_trail {
 
 #define LFD_MAX_INJECT_TRAILS 16   /* trails per batch slot */
 
+/* Tabulated trail shapes for lfd_submit_injected_shaped: a pool of float32 samples that the handle owns, and tables that
+ * name n samples of it, evenly spaced on [lo, hi] (samples[offset + i] at lo + i * (hi - lo) / (n - 1)).
+ * A cross-section profile's abscissa is the signed distance d of lfd_trail; with p = the profile's samples:
+ *   footprint 0 <= t <= L and lo <= d <= hi (asymmetric profiles are allowed)
+ *   u = (d - lo) * inv, inv = (float)((n - 1) / ((double)hi - (double)lo)), i = min(trunc(u), n - 2), f = u - i
+ *   P = p[i] + f * (p[i+1] - p[i])
+ * A light curve a of m samples spans the segment from (x0, y0) at t = 0 to (x1, y1) at t = L (its lo and hi are not
+ * used): v = t * c, c = (float)((m - 1) / (double)L), j = min(trunc(v), m - 2), g = v - j, A = a[j] + g * (a[j+1] - a[j]).
+ * The pixel gets (peak * P) * A added, or peak * P without a light curve; every operation is one float32 round-to-nearest
+ * step (tests/inject_shapes_ref.py::render_trails(..., tables) is bit-identical).  Profile -1 is lfd_trail's Gaussian (P =
+ * expf(...), footprint |d| <= ceil(5 sigma) + 1) and light curve -1 is A = 1, so shapes of all -1 give
+ * lfd_submit_injected's frames bit for bit.  `peak` is the flux at a sample value of 1; a tabulated profile ignores
+ * `sigma` (it is not validated). */
+typedef struct lfd_table {
+    int32_t offset, n;      /* samples[offset .. offset + n) of the pool, 2 <= n <= LFD_MAX_TABLE_SAMPLES */
+    float lo, hi;           /* finite, lo < hi, max(|lo|, |hi|) <= 1024 */
+} lfd_table;
+
+typedef struct lfd_trail_shape {
+    int32_t profile;        /* table index of the cross-section profile, -1 = Gaussian of lfd_trail.sigma */
+    int32_t lightcurve;     /* table index of the light curve, -1 = constant 1 */
+} lfd_trail_shape;
+
+#define LFD_MAX_TABLE_SAMPLES 4096
+#define LFD_MAX_TRAIL_TABLES 4096
+
 typedef struct lfd_handle lfd_handle;
 
 int lfd_abi_version(void);
@@ -221,6 +247,17 @@ int lfd_run_resident(lfd_handle* h, int n, int flags);
 int lfd_set_base(lfd_handle* h, const float* frames, int n_base, const int32_t* rects, const int32_t* rect_offsets);
 int lfd_submit_injected(lfd_handle* h, int n, const int32_t* base_index, const lfd_trail* trails,
                         const int32_t* trail_offsets, int flags);
+/* lfd_set_trail_tables uploads the pool of tabulated shapes (lfd_table) once, synchronously; a second call replaces it.
+ * LFD_E_STATE while a batch is pending; LFD_E_ARG when n_tables is outside 1..LFD_MAX_TRAIL_TABLES, a table's n is
+ * outside 2..LFD_MAX_TABLE_SAMPLES or it lies outside samples[0 .. n_samples), a sample, lo or hi is not finite,
+ * lo >= hi, or max(|lo|, |hi|) > 1024.
+ * lfd_submit_injected_shaped is lfd_submit_injected with one shapes entry per trail (NULL = all -1, which is
+ * lfd_submit_injected).  Beyond lfd_submit_injected's checks: LFD_E_ARG with nothing launched when a table index is
+ * below -1 or not in the current pool, LFD_E_STATE when a trail names a table and no pool has been set; sigma is only
+ * checked for Gaussian profiles. */
+int lfd_set_trail_tables(lfd_handle* h, const float* samples, int n_samples, const lfd_table* tables, int n_tables);
+int lfd_submit_injected_shaped(lfd_handle* h, int n, const int32_t* base_index, const lfd_trail* trails,
+                               const lfd_trail_shape* shapes, const int32_t* trail_offsets, int flags);
 
 /* One pass on one already flipped frame (process_field_bright / process_field_dim called directly).
  * If `writeback` != 0 the clipped float image is copied back into `img` (the reference mutates it). */

@@ -26,6 +26,9 @@ STAGES = {"mask": 0, "gray": 1, "equ": 2, "eroded": 3, "morph": 4, "canny": 5, "
           "lines_equ": 15, "lines_box": 16, "clipped": 17, "input": 18}
 MAX_INJECT_TRAILS = 16
 TRAIL_DTYPE = np.dtype([("x0", "<f4"), ("y0", "<f4"), ("x1", "<f4"), ("y1", "<f4"), ("sigma", "<f4"), ("peak", "<f4")])
+MAX_TABLE_SAMPLES, MAX_TRAIL_TABLES = 4096, 4096
+TABLE_DTYPE = np.dtype([("offset", "<i4"), ("n", "<i4"), ("lo", "<f4"), ("hi", "<f4")])
+SHAPE_DTYPE = np.dtype([("profile", "<i4"), ("lightcurve", "<i4")])
 
 
 class PassParams(ctypes.Structure):
@@ -139,12 +142,16 @@ def lib():
                                        ctypes.c_double, ctypes.c_double, ctypes.c_longlong, ctypes.c_double,
                                        ctypes.POINTER(ctypes.c_char_p), ctypes.c_int, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_int,
                                        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]
-        for sym in ("lfd_set_base", "lfd_submit_injected"):     # added within ABI version 1: a stale build lacks them
+        for sym in ("lfd_set_base", "lfd_submit_injected", "lfd_set_trail_tables", "lfd_submit_injected_shaped"):
+            # added within ABI version 1: a stale build lacks them
             if not hasattr(L, sym):
                 raise ImportError("liblfd_b200.so predates %s: rebuild it (`python -c 'import __graft_entry__ as g; g.build()'`)" % sym)
         L.lfd_set_base.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]
         L.lfd_submit_injected.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                           ctypes.c_int]
+        L.lfd_set_trail_tables.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
+        L.lfd_submit_injected_shaped.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                                 ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]
         if L.lfd_abi_version() != 1:
             raise ImportError("liblfd_b200.so ABI mismatch")
         _lib = L
@@ -392,17 +399,35 @@ class Handle:
         _flat, _offs, rp, op = self._rects_arrays(rects_per_frame)
         self._ck(self._L.lfd_set_base(self.h, frames.ctypes.data_as(ctypes.c_void_p), frames.shape[0], rp, op))
 
+    def set_trail_tables(self, tables):
+        """Upload the pool of tabulated trail shapes, a list of ``(lo, hi, samples)`` (``samples`` evenly spaced on
+        [lo, hi]); a trail dict's ``"profile"`` / ``"lightcurve"`` keys index it.  A second call replaces the pool
+        (include/lfd_b200.h: lfd_set_trail_tables, lfd_table)."""
+        arrs = [np.asarray(smp, np.float32).ravel() for _lo, _hi, smp in tables]
+        tab = np.zeros(len(arrs), TABLE_DTYPE)
+        off = 0
+        for i, ((lo, hi, _smp), a) in enumerate(zip(tables, arrs)):
+            tab[i] = (off, len(a), lo, hi)
+            off += len(a)
+        pool = np.ascontiguousarray(np.concatenate(arrs) if arrs else np.zeros(0, np.float32))
+        self._ck(self._L.lfd_set_trail_tables(self.h, pool.ctypes.data_as(ctypes.c_void_p), len(pool),
+                                              tab.ctypes.data_as(ctypes.c_void_p), len(tab)))
+
     @staticmethod
     def trails_array(trails):
-        """Trails as synth's dicts {p0: (x, y), p1: (x, y), sigma, peak} -> a TRAIL_DTYPE array (float32 fields)."""
+        """Trails as synth's dicts {p0: (x, y), p1: (x, y), sigma, peak} -> a TRAIL_DTYPE array (float32 fields).  A
+        trail with a tabulated ``"profile"`` may omit ``sigma`` (NaN here)."""
         out = np.zeros(len(trails), TRAIL_DTYPE)
         for i, t in enumerate(trails):
-            out[i] = (t["p0"][0], t["p0"][1], t["p1"][0], t["p1"][1], t["sigma"], t["peak"])
+            sigma = t["sigma"] if t.get("profile", -1) < 0 else t.get("sigma", np.nan)
+            out[i] = (t["p0"][0], t["p0"][1], t["p1"][0], t["p1"][1], sigma, t["peak"])
         return out
 
     def submit_injected(self, base_index, trails_per_slot=None, flags=0):
         """Run slot f on base base_index[f] plus the trails trails_per_slot[f] (synth's dicts), added on the device;
-        collect with wait() (include/lfd_b200.h: lfd_submit_injected)."""
+        collect with wait() (include/lfd_b200.h: lfd_submit_injected).  When a trail has an integer ``"profile"`` or
+        ``"lightcurve"`` key (an index into set_trail_tables' pool, -1 = Gaussian / constant) the batch goes through
+        lfd_submit_injected_shaped."""
         bidx = np.ascontiguousarray(base_index, np.int32)
         n = len(bidx)
         tp, op = None, None
@@ -416,6 +441,13 @@ class Handle:
             if offs[-1]:
                 arr[:offs[-1]] = np.concatenate([self.trails_array(ts) for ts in trails_per_slot if len(ts)])
             tp, op = arr.ctypes.data_as(ctypes.c_void_p), offs.ctypes.data_as(ctypes.c_void_p)
+            flat = [t for ts in trails_per_slot for t in ts]
+            if any("profile" in t or "lightcurve" in t for t in flat):
+                shapes = np.array([(t.get("profile", -1), t.get("lightcurve", -1)) for t in flat], SHAPE_DTYPE)
+                self._ck(self._L.lfd_submit_injected_shaped(self.h, n, bidx.ctypes.data_as(ctypes.c_void_p), tp,
+                                                            shapes.ctypes.data_as(ctypes.c_void_p), op, flags))
+                self._n = n
+                return
         self._ck(self._L.lfd_submit_injected(self.h, n, bidx.ctypes.data_as(ctypes.c_void_p), tp, op, flags))
         self._n = n
 

@@ -1,21 +1,27 @@
-// k_inject.cuh - on-device trail injection for completeness campaigns (lfd_set_base / lfd_submit_injected).
+// k_inject.cuh - on-device trail injection for completeness campaigns (lfd_set_base / lfd_submit_injected[_shaped]).
 //
-// in[f] = base[base_index[f]] + the Gaussian line segments of slot f, the trail of lfd_b200/synth.py::_add_trail with
-// the tails beyond |d| = ceil(5 sigma) + 1 dropped (oracle/inject_ref.py::render_trails is the checker).  Per pixel,
-// in float32 and in _add_trail's operation order:
+// in[f] = base[base_index[f]] + the line segments of slot f (the checkers are oracle/inject_ref.py::render_trails and,
+// for tabulated shapes, tests/inject_shapes_ref.py::render_trails).  Per pixel, in float32 and in
+// lfd_b200/synth.py::_add_trail's operation order:
 //   t = (x - x0) * ux + (y - y0) * uy,   d = -(x - x0) * uy + (y - y0) * ux
-//   pixel += peak * expf(-0.5f * (d / sigma)^2)   iff 0 <= t <= L and |d| <= pad
-// with ux, uy, L rounded to float32 from double on the host.  Every product and sum is an explicit round-to-nearest
-// intrinsic, so footprint membership is bit-identical to the NumPy reference and only expf may differ in the last bits.
+//   pixel += (peak * P(d)) * A(t)   iff 0 <= t <= L and dlo <= d <= dhi
+// with ux, uy, L rounded to float32 from double on the host.  P is _add_trail's Gaussian expf(-0.5f * (d / sigma)^2)
+// with [dlo, dhi] = [-pad, pad], pad = ceil(5 sigma) + 1, or the linear interpolation of a tabulated profile on
+// [dlo, dhi]; A is 1 or the linear interpolation of a tabulated light curve over [0, L] (include/lfd_b200.h, lfd_table).
+// Every product and sum is an explicit round-to-nearest intrinsic, so footprint membership and the tabulated shapes are
+// bit-identical to the NumPy reference and only expf may differ in the last bits.
 #pragma once
 #include "common.cuh"
 
 #define INJ_ROWS 8                  // frame rows per CTA
 #define INJ_THREADS 256
 
-// one trail as the kernel uses it (host-prepared from lfd_trail); L == 0 marks a zero-length trail (adds nothing)
+// one trail as the kernel uses it (host-prepared from lfd_trail and lfd_trail_shape); L == 0 marks a zero-length trail
+// (adds nothing).  pn == 0: Gaussian profile of sigma; else pn samples at poff on [dlo, dhi], inv = (pn - 1) / (dhi - dlo).
+// lm == 0: no light curve; else lm samples at loff over [0, L], c = (lm - 1) / L.
 struct InjTrail {
-    float x0, y0, ux, uy, L, sigma, peak, pad;
+    float x0, y0, ux, uy, L, sigma, peak, dlo, dhi, inv, c;
+    int poff, pn, loff, lm;
 };
 
 // Conservative x-range [lo, hi] of the pixels of row y the float32 test can accept: the exact interval of the rotated
@@ -25,11 +31,11 @@ __device__ __forceinline__ int2 inj_row_range(const InjTrail& T, int y, int W)
     const double slack = 1e-5 * (fabs((double)T.x0) + fabs((double)T.y0) + (double)W + (double)y) + 1e-3;
     double lo = 0.0, hi = (double)(W - 1);
     const double yy = (double)y - (double)T.y0;
-    // t(x) = ux * (x - x0) + yy * uy in [-slack, L + slack];  d(x) = -uy * (x - x0) + yy * ux in [-pad - slack, pad + slack]
+    // t(x) = ux * (x - x0) + yy * uy in [-slack, L + slack];  d(x) = -uy * (x - x0) + yy * ux in [dlo - slack, dhi + slack]
     const double c[2] = {(double)T.ux, -(double)T.uy};
     const double o[2] = {yy * (double)T.uy, yy * (double)T.ux};
-    const double a[2] = {-slack, -(double)T.pad - slack};
-    const double b[2] = {(double)T.L + slack, (double)T.pad + slack};
+    const double a[2] = {-slack, (double)T.dlo - slack};
+    const double b[2] = {(double)T.L + slack, (double)T.dhi + slack};
     for (int k = 0; k < 2; k++) {
         if (c[k] == 0.0) {
             if (o[k] < a[k] || o[k] > b[k]) return make_int2(1, 0);
@@ -44,10 +50,18 @@ __device__ __forceinline__ int2 inj_row_range(const InjTrail& T, int y, int W)
     return make_int2((int)floor(lo), (int)ceil(hi));
 }
 
+// a[i] + f * (a[i+1] - a[i]) at u >= 0, i = min(trunc(u), n - 2), f = u - i: the table value of lfd_table
+__device__ __forceinline__ float inj_lerp(const float* __restrict__ a, int n, float u)
+{
+    const int i = min((int)u, n - 2);
+    const float f = __fsub_rn(u, (float)i), a0 = __ldg(a + i), a1 = __ldg(a + i + 1);
+    return __fadd_rn(a0, __fmul_rn(f, __fsub_rn(a1, a0)));
+}
+
 // grid (ceil(H / INJ_ROWS), n), INJ_THREADS threads; W % 4 == 0 (lfd_create)
 __global__ void __launch_bounds__(INJ_THREADS)
 k_inject(const float* __restrict__ base, const int* __restrict__ base_index, const InjTrail* __restrict__ trails,
-         const int* __restrict__ trail_off, float* __restrict__ out, Dims d)
+         const int* __restrict__ trail_off, const float* __restrict__ samples, float* __restrict__ out, Dims d)
 {
     __shared__ InjTrail st[LFD_MAX_INJECT_TRAILS];
     __shared__ int2 rng[INJ_ROWS][LFD_MAX_INJECT_TRAILS];
@@ -101,9 +115,17 @@ k_inject(const float* __restrict__ base, const int* __restrict__ base_index, con
                         const float ax = __fsub_rn(xf, T.x0), by = __fsub_rn(yf, T.y0);
                         const float t = __fadd_rn(__fmul_rn(ax, T.ux), __fmul_rn(by, T.uy));
                         const float dd = __fadd_rn(-__fmul_rn(ax, T.uy), __fmul_rn(by, T.ux));
-                        if (t >= 0.f && t <= T.L && fabsf(dd) <= T.pad) {
-                            const float q2 = __fdiv_rn(dd, T.sigma);
-                            acc = __fadd_rn(acc, __fmul_rn(T.peak, expf(__fmul_rn(-0.5f, __fmul_rn(q2, q2)))));
+                        if (t >= 0.f && t <= T.L && dd >= T.dlo && dd <= T.dhi) {
+                            float p;
+                            if (T.pn == 0) {
+                                const float q2 = __fdiv_rn(dd, T.sigma);
+                                p = expf(__fmul_rn(-0.5f, __fmul_rn(q2, q2)));
+                            } else {
+                                p = inj_lerp(samples + T.poff, T.pn, __fmul_rn(__fsub_rn(dd, T.dlo), T.inv));
+                            }
+                            float add = __fmul_rn(T.peak, p);
+                            if (T.lm) add = __fmul_rn(add, inj_lerp(samples + T.loff, T.lm, __fmul_rn(t, T.c)));
+                            acc = __fadd_rn(acc, add);
                         }
                     }
                     e[c] = acc;

@@ -137,6 +137,9 @@ struct lfd_handle {
     InjTrail* inj_trails_h = nullptr; // pinned staging of the three above
     int* inj_off_h = nullptr;
     int* inj_base_h = nullptr;
+    float* tab_samples_d = nullptr;   // pool of tabulated trail shapes (lfd_set_trail_tables), [tab_cap] samples
+    int tab_cap = 0;
+    std::vector<lfd_table> tables;    // the pool's tables; empty: no pool set
     cudaEvent_t ev_inj[2] = {nullptr, nullptr};   // around k_inject; inj_recorded: the last run was lfd_submit_injected
     bool inj_recorded = false;
     float inj_ms = 0.f;
@@ -395,6 +398,7 @@ extern "C" int lfd_destroy(lfd_handle* h)
     if (h->rect_off_h) cudaFreeHost(h->rect_off_h);
     if (h->ctl_h) cudaFreeHost(h->ctl_h);
     if (h->base_d) cudaFree(h->base_d);
+    if (h->tab_samples_d) cudaFree(h->tab_samples_d);
     if (h->inj_trails_h) cudaFreeHost(h->inj_trails_h);
     if (h->inj_off_h) cudaFreeHost(h->inj_off_h);
     if (h->inj_base_h) cudaFreeHost(h->inj_base_h);
@@ -1106,8 +1110,48 @@ extern "C" int lfd_set_base(lfd_handle* h, const float* frames, int n_base, cons
     return LFD_OK;
 }
 
+extern "C" int lfd_set_trail_tables(lfd_handle* h, const float* samples, int n_samples, const lfd_table* tables, int n_tables)
+{
+    if (!h) return LFD_E_ARG;
+    cudaSetDevice(h->device);
+    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    if (!samples || !tables || n_samples < 2 || n_tables < 1 || n_tables > LFD_MAX_TRAIL_TABLES) {
+        h->err = "lfd_set_trail_tables: samples and tables must be non-NULL, n_samples >= 2, n_tables in 1..LFD_MAX_TRAIL_TABLES";
+        return LFD_E_ARG;
+    }
+    for (int i = 0; i < n_samples; i++)
+        if (!isfinite(samples[i])) { h->err = "trail table samples must be finite"; return LFD_E_ARG; }
+    for (int k = 0; k < n_tables; k++) {
+        const lfd_table& t = tables[k];
+        if (t.n < 2 || t.n > LFD_MAX_TABLE_SAMPLES || t.offset < 0 || (int64_t)t.offset + t.n > n_samples) {
+            h->err = "a trail table has n outside 2..LFD_MAX_TABLE_SAMPLES or lies outside the samples"; return LFD_E_ARG;
+        }
+        if (!isfinite(t.lo) || !isfinite(t.hi) || !(t.lo < t.hi) || fmaxf(fabsf(t.lo), fabsf(t.hi)) > 1024.f) {
+            h->err = "a trail table needs finite lo < hi with max(|lo|, |hi|) <= 1024"; return LFD_E_ARG;
+        }
+    }
+    if (n_samples > h->tab_cap) {
+        if (h->tab_samples_d) { cudaFree(h->tab_samples_d); h->tab_samples_d = nullptr; }
+        h->tab_cap = 0;
+        h->tables.clear();
+        CK(cudaMalloc((void**)&h->tab_samples_d, (size_t)n_samples * sizeof(float)));
+        h->tab_cap = n_samples;
+    }
+    h->tables.clear();
+    CK(cudaMemcpyAsync(h->tab_samples_d, samples, (size_t)n_samples * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));          // the caller may free `samples` on return
+    h->tables.assign(tables, tables + n_tables);
+    return LFD_OK;
+}
+
 extern "C" int lfd_submit_injected(lfd_handle* h, int n, const int32_t* base_index, const lfd_trail* trails,
                                    const int32_t* trail_offsets, int flags)
+{
+    return lfd_submit_injected_shaped(h, n, base_index, trails, nullptr, trail_offsets, flags);
+}
+
+extern "C" int lfd_submit_injected_shaped(lfd_handle* h, int n, const int32_t* base_index, const lfd_trail* trails,
+                                          const lfd_trail_shape* shapes, const int32_t* trail_offsets, int flags)
 {
     if (!h) return LFD_E_ARG;
     cudaSetDevice(h->device);
@@ -1116,6 +1160,7 @@ extern "C" int lfd_submit_injected(lfd_handle* h, int n, const int32_t* base_ind
     if (n < 1 || n > h->B || !base_index) { h->err = "bad batch size or base_index"; return LFD_E_ARG; }
     if (flags & LFD_INPUT_BIGENDIAN) { h->err = "injected frames are built in native byte order (LFD_INPUT_BIGENDIAN)"; return LFD_E_ARG; }
     if (!trails != !trail_offsets || (trail_offsets && trail_offsets[0] != 0)) { h->err = "bad trails / trail_offsets"; return LFD_E_ARG; }
+    const int ntab = (int)h->tables.size();
     // validate everything before anything is staged or launched
     for (int f = 0; f < n; f++) {
         if (base_index[f] < 0 || base_index[f] >= h->n_base) { h->err = "base_index out of range"; return LFD_E_ARG; }
@@ -1124,8 +1169,14 @@ extern "C" int lfd_submit_injected(lfd_handle* h, int n, const int32_t* base_ind
         if (c < 0 || c > LFD_MAX_INJECT_TRAILS) { h->err = "a slot has more than LFD_MAX_INJECT_TRAILS trails"; return LFD_E_ARG; }
         for (int k = trail_offsets[f]; k < trail_offsets[f + 1]; k++) {
             const lfd_trail& t = trails[k];
-            if (!isfinite(t.x0) || !isfinite(t.y0) || !isfinite(t.x1) || !isfinite(t.y1) || !isfinite(t.sigma) ||
-                !isfinite(t.peak) || !(t.sigma > 0.f)) { h->err = "trail values must be finite with sigma > 0"; return LFD_E_ARG; }
+            const lfd_trail_shape s = shapes ? shapes[k] : lfd_trail_shape{-1, -1};
+            if (s.profile < -1 || s.lightcurve < -1) { h->err = "a trail table index is below -1"; return LFD_E_ARG; }
+            if ((s.profile >= 0 || s.lightcurve >= 0) && ntab == 0) { h->err = "a trail names a table and no pool is set (call lfd_set_trail_tables)"; return LFD_E_STATE; }
+            if (s.profile >= ntab || s.lightcurve >= ntab) { h->err = "a trail table index is not in the pool"; return LFD_E_ARG; }
+            if (!isfinite(t.x0) || !isfinite(t.y0) || !isfinite(t.x1) || !isfinite(t.y1) || !isfinite(t.peak) ||
+                (s.profile < 0 && !(isfinite(t.sigma) && t.sigma > 0.f))) {
+                h->err = "trail values must be finite, with sigma > 0 for a Gaussian profile"; return LFD_E_ARG;
+            }
         }
     }
     // per-slot star rectangles from the slot's base, into the lfd_submit staging
@@ -1148,13 +1199,28 @@ extern "C" int lfd_submit_injected(lfd_handle* h, int n, const int32_t* base_ind
         for (int k = trail_offsets[f]; k < trail_offsets[f + 1]; k++) {
             const lfd_trail& t = trails[k];
             const double dx = (double)t.x1 - (double)t.x0, dy = (double)t.y1 - (double)t.y0, L = hypot(dx, dy);
+            const lfd_trail_shape s = shapes ? shapes[k] : lfd_trail_shape{-1, -1};
             InjTrail& q = h->inj_trails_h[nt++];
             q.x0 = t.x0; q.y0 = t.y0; q.sigma = t.sigma; q.peak = t.peak;
             q.L = (float)L;
             q.ux = L > 0 ? (float)(dx / L) : 0.f;
             q.uy = L > 0 ? (float)(dy / L) : 0.f;
-            q.pad = (float)(ceil(5.0 * (double)t.sigma) + 1.0);
             if (L == 0) q.L = 0.f;
+            if (s.profile < 0) {
+                const float pad = (float)(ceil(5.0 * (double)t.sigma) + 1.0);
+                q.dlo = -pad; q.dhi = pad; q.poff = q.pn = 0; q.inv = 0.f;
+            } else {
+                const lfd_table& p = h->tables[s.profile];
+                q.dlo = p.lo; q.dhi = p.hi; q.poff = p.offset; q.pn = p.n;
+                q.inv = (float)((double)(p.n - 1) / ((double)p.hi - (double)p.lo));
+            }
+            if (s.lightcurve < 0 || q.L == 0.f) {
+                q.loff = q.lm = 0; q.c = 0.f;
+            } else {
+                const lfd_table& a = h->tables[s.lightcurve];
+                q.loff = a.offset; q.lm = a.n;
+                q.c = (float)((double)(a.n - 1) / (double)q.L);
+            }
         }
     }
     h->inj_off_h[n] = nt;
@@ -1163,7 +1229,7 @@ extern "C" int lfd_submit_injected(lfd_handle* h, int n, const int32_t* base_ind
     CK(cudaMemcpyAsync(h->inj_base_d, h->inj_base_h, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, h->stream));
     CK(cudaEventRecord(h->ev_inj[0], h->stream));
     k_inject<<<dim3((h->d.H + INJ_ROWS - 1) / INJ_ROWS, n), INJ_THREADS, 0, h->stream>>>(h->base_d, h->inj_base_d, h->inj_trails_d,
-                                                                                       h->inj_off_d, h->in, h->d); LAUNCH_CHECK();
+                                                                                       h->inj_off_d, h->tab_samples_d, h->in, h->d); LAUNCH_CHECK();
     CK(cudaEventRecord(h->ev_inj[1], h->stream));
     int rc = run_pipeline(h, n, flags, 0, false);
     if (rc != LFD_OK) return rc;

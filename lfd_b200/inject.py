@@ -2,14 +2,18 @@
 passes find.  Synthetic trails (synth's dicts ``{p0: (x, y), p1: (x, y), sigma, peak}``, the Gaussian line segment of
 include/lfd_b200.h ``lfd_trail``) are added to resident real frames on the device (lfd_set_base /
 lfd_submit_injected), so a campaign that reuses a few dozen frames thousands of times never sends pixels over the host
-link."""
+link.
+
+Trails may also carry tabulated shapes (include/lfd_b200.h ``lfd_table``): a ``"profile"`` key indexes a cross-section
+profile and a ``"lightcurve"`` key a brightness along the segment in the ``tables`` passed to ``recovery``.
+``defocus_profile`` builds the cross-section of a meteor seen by a telescope focused at infinity."""
 import math
 
 import numpy as np
 
 from . import _lib
 
-__all__ = ["trail_line", "recovery", "RECOVERY_DTYPE"]
+__all__ = ["trail_line", "recovery", "defocus_profile", "RECOVERY_DTYPE"]
 
 _T = _lib.MAX_INJECT_TRAILS
 RECOVERY_DTYPE = np.dtype([
@@ -35,6 +39,50 @@ def trail_line(trail, shape):
     return x0 * math.cos(theta) + y0 * math.sin(theta), theta
 
 
+def _defocus_samples(r_outer, r_inner, seeing_fwhm, step):
+    """(d, samples) of defocus_profile before the normalisation to a maximum of 1 (float64)."""
+    ro, ri, fw, step = float(r_outer), float(r_inner), float(seeing_fwhm), float(step)
+    if not all(math.isfinite(v) for v in (ro, ri, fw, step)) or step <= 0 or fw < 0:
+        raise ValueError("r_outer, r_inner, seeing_fwhm and step must be finite, step > 0 and seeing_fwhm >= 0")
+    if ro <= 0 and fw == 0:
+        raise ValueError("r_outer must be > 0 when there is no seeing")
+    if ri < 0 or ri > ro:
+        raise ValueError("r_inner must lie in [0, r_outer]")
+    sig = fw / (2.0 * math.sqrt(2.0 * math.log(2.0)))
+    k = int(math.ceil((max(ro, 0.0) + 4.0 * sig) / step - 1e-9))
+    if 2 * k + 1 > _lib.MAX_TABLE_SAMPLES:
+        raise ValueError("%d samples exceed %d: use a larger step" % (2 * k + 1, _lib.MAX_TABLE_SAMPLES))
+    # with seeing, the convolution runs on a grid 8 times finer than the output, so the smooth result's samples keep
+    # the annulus' integral; without seeing the samples are the annulus' point values
+    sub = 8 if sig > 0 else 1
+    h = step / sub
+    kw = int(math.ceil(4.0 * sig / h)) if sig > 0 else 0
+    x = np.arange(-(k * sub + kw), k * sub + kw + 1) * h
+    if ro > 0:
+        a = np.sqrt(np.maximum(ro * ro - x * x, 0.0)) - np.sqrt(np.maximum(ri * ri - x * x, 0.0))
+    else:                                       # a point source: the seeing alone
+        a = np.zeros_like(x)
+        a[k * sub + kw] = 1.0 / h
+    if kw:
+        g = np.exp(-0.5 * (np.arange(-kw, kw + 1) * h / sig) ** 2)
+        a = np.convolve(a, g / g.sum(), mode="valid")[::sub]
+    return np.arange(-k, k + 1) * step, 0.5 * (a + a[::-1])     # exactly symmetric
+
+
+def defocus_profile(r_outer, r_inner=0.0, seeing_fwhm=0.0, step=0.25):
+    """Cross-section of a defocused trail as a ``(lo, hi, samples)`` table for ``recovery(..., tables=...)`` and
+    Handle.set_trail_tables: the telescope pupil, a uniform annulus of radii ``r_inner`` <= ``r_outer`` px, drawn along
+    a line, sqrt(max(ro² - d², 0)) - sqrt(max(ri² - d², 0)), convolved with the seeing, a Gaussian of FWHM
+    ``seeing_fwhm`` px (a 2-D Gaussian projects to a 1-D Gaussian of the same sigma).  Samples every ``step`` px on
+    ±(ro + 4 sigma), rounded out to the step, float32, normalised to a maximum of 1, so a trail's ``peak`` is the flux
+    at the brightest point of the cross-section.  A telescope focused at infinity images each point of a meteor at
+    distance D as its pupil of angular diameter aperture / D: a 2.5 m aperture at 100 km subtends 5.2 arcsec, 13 px at
+    0.396 arcsec per pixel, so ``r_outer = 6.5``.  Raises ValueError when r_outer <= 0 without seeing, or r_inner is
+    outside [0, r_outer]."""
+    d, a = _defocus_samples(r_outer, r_inner, seeing_fwhm, step)
+    return float(d[0]), float(d[-1]), (a / a.max()).astype(np.float32)
+
+
 def _first_match(rho, theta, lines, theta_tol, rho_tol):
     """Index of the first (rho_true, theta_true) the detected line matches, or -1.  Across the theta = 0 / pi wrap the
     same line has the opposite rho."""
@@ -46,11 +94,13 @@ def _first_match(rho, theta, lines, theta_tol, rho_tol):
 
 
 def recovery(frames, rects, injections, params_bright=None, params_dim=None, device=0, batch=64,
-             theta_tol=np.deg2rad(2), rho_tol=None):
+             theta_tol=np.deg2rad(2), rho_tol=None, tables=None):
     """Run every injection and every base without a trail; one RECOVERY_DTYPE row per injection.
 
     ``frames``: (n_base, H, W) un-flipped float32 bases; ``rects``: their star rectangles (lfd_submit's convention, one
-    array per base) or None; ``injections``: a sequence of ``(base_index, [trail, ...])`` with at most 16 trails each.
+    array per base) or None; ``injections``: a sequence of ``(base_index, [trail, ...])`` with at most 16 trails each;
+    ``tables``: the ``(lo, hi, samples)`` tables (e.g. ``defocus_profile``) that trails' ``"profile"`` and
+    ``"lightcurve"`` keys index.  The row's ``sigma`` is NaN for a tabulated profile that has none.
 
     A row holds the base, the injected trails (NaN past ``ntrails``), the device verdict of the injected frame
     (``detected``, ``pass``, ``status``, and ``rho``, ``theta`` = equhough[0][0] of the detecting pass), whether the base
@@ -87,6 +137,8 @@ def recovery(frames, rects, injections, params_bright=None, params_dim=None, dev
             hs.append(h)
             h.set_params(pb, pd)
             h.set_base(frames, rects)
+            if tables:
+                h.set_trail_tables(tables)
 
         def submit(k):
             hs[k & 1].submit_injected([jobs[i][0] for i in chunks[k]], [jobs[i][1] for i in chunks[k]])

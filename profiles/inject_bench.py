@@ -3,9 +3,14 @@ the device and a grid of single-trail injections (angles incl. 0 and 90 +- 1 deg
 lengths), run through lfd_submit_injected with one handle and with two alternating handles; k_inject's event time per
 64-slot step against the HBM copy peak; and, for comparison, the same injections rendered on the host with
 oracle/inject_ref.py::render_trails (one host thread) and sent through lfd_submit.  The host path renders ~10 ms a
-frame, so it runs on the first --host-steps steps of the grid only (stated in its line).
+frame, so it runs on the first --host-steps steps of the grid only (stated in its line; 0 skips it).
 
-    python profiles/inject_bench.py [--injections 20480] [--host-steps 8] [--out DIR]
+--shape picks the trail cross-sections, on the same bases and the same geometry grid: ``gaussian`` (synth's Gaussian,
+lfd_submit_injected), ``donut`` (lfd_b200.inject.defocus_profile with r_outer 4, 6.67, 9.33, 12 px in place of the four
+FWHMs, r_inner = 0.4 r_outer, seeing FWHM 3.5 px; lfd_submit_injected_shaped) and ``donut_lightcurve`` (the same with a
+64-sample rise-and-fade light curve).  Several shapes alternate within each round of handle counts.
+
+    python profiles/inject_bench.py [--injections 20480] [--host-steps 8] [--shape gaussian donut ...] [--out DIR]
 
 Prints one JSON line per measurement (and writes them to DIR/inject_bench.jsonl with --out).  The device name and
 power limit are read in the same run."""
@@ -61,15 +66,17 @@ def make_bases():
     return frames, rects, [j[0] for j in jobs]
 
 
+FWHM = (2.0, 4.0, 8.0, 15.0)
+R_OUTER = (4.0, 20.0 / 3.0, 28.0 / 3.0, 12.0)     # the donut that replaces FWHM[k]
+COMBOS = list(itertools.product((0.0, 1.0, 179.0, 89.0, 90.0, 91.0, 30.0, 45.0, 60.0, 120.0, 135.0, 150.0), FWHM,
+                                (0.1, 0.3, 1.0, 3.0, 10.0, 50.0), (200.0, 600.0, 1200.0, 2400.0)))
+
+
 def make_grid(n, seed=2026):
     """n single-trail injections: every combination of 12 angles, 4 FWHMs, 6 peaks and 4 lengths, repeated with random
     centres (middle half of the frame) and random bases."""
     rng = np.random.default_rng(seed)
-    angles = (0.0, 1.0, 179.0, 89.0, 90.0, 91.0, 30.0, 45.0, 60.0, 120.0, 135.0, 150.0)
-    fwhm = (2.0, 4.0, 8.0, 15.0)
-    peaks = (0.1, 0.3, 1.0, 3.0, 10.0, 50.0)
-    lengths = (200.0, 600.0, 1200.0, 2400.0)
-    combos = list(itertools.product(angles, fwhm, peaks, lengths))
+    combos = COMBOS
     out = []
     for i in range(n):
         ang, fw, pk, L = combos[i % len(combos)]
@@ -78,6 +85,28 @@ def make_grid(n, seed=2026):
         out.append((int(rng.integers(0, B)), [{"p0": (cx - L / 2 * math.cos(a), cy - L / 2 * math.sin(a)),
                                                "p1": (cx + L / 2 * math.cos(a), cy + L / 2 * math.sin(a)),
                                                "sigma": fw / 2.3548, "peak": pk}]))
+    return out
+
+
+def shape_tables():
+    """The donut profiles (table k replaces FWHM[k]) and, last, the rise-and-fade light curve."""
+    from lfd_b200.inject import defocus_profile
+    s = np.linspace(0.0, 1.0, 64)
+    rise_fade = np.where(s < 0.3, (s / 0.3) ** 2, np.exp(-(s - 0.3) / 0.35)).astype(np.float32)
+    return [defocus_profile(r, 0.4 * r, 3.5) for r in R_OUTER] + [(0.0, 1.0, rise_fade)]
+
+
+def shaped_grid(grid, shape):
+    """The grid with the trails of `shape`: the same end points and peaks, the Gaussian of FWHM[k] replaced by donut k."""
+    if shape == "gaussian":
+        return grid
+    out = []
+    for i, (b, (t,)) in enumerate(grid):
+        t = dict(t, profile=FWHM.index(COMBOS[i % len(COMBOS)][1]))
+        del t["sigma"]
+        if shape == "donut_lightcurve":
+            t["lightcurve"] = len(R_OUTER)
+        out.append((b, [t]))
     return out
 
 
@@ -108,6 +137,7 @@ def main():
     ap.add_argument("--injections", type=int, default=20480)
     ap.add_argument("--host-steps", type=int, default=8)
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--shape", nargs="+", default=["gaussian"], choices=["gaussian", "donut", "donut_lightcurve"])
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     from lfd_b200.detecttrails import default_params
@@ -125,9 +155,11 @@ def main():
     steps = [grid[i:i + B] for i in range(0, len(grid), B)]
     pb, pd, _ = default_params()
     hs = [_lib.Handle(H, W, max_batch=B) for _ in range(2)]
+    tables = shape_tables()
     for h in hs:
         h.set_params(pb, pd)
         h.set_base(frames, rects)
+        h.set_trail_tables(tables)
     common = dict(info, bases=B, base_kinds={k: kinds.count(k) for k in sorted(set(kinds))}, batch=B,
                   frame=[H, W], injections=len(grid))
 
@@ -161,12 +193,17 @@ def main():
     # kernel runs alone; with two it overlaps the other handle's passes, so its event time includes their contention.
     peak, src = hbm_peak()
     bytes_step = 8 * H * W * B
-    run_device(2, steps[:args.warmup])
-    for nh in (1, 2, 1, 2):
-        dt, kms, ndet = run_device(nh, steps)
+    shaped = {}
+    for sh in args.shape:
+        g = shaped_grid(grid, sh)
+        shaped[sh] = [g[i:i + B] for i in range(0, len(g), B)]
+    for sh in args.shape:
+        run_device(2, shaped[sh][:args.warmup])
+    for nh, sh in itertools.product((1, 2, 1, 2), args.shape):
+        dt, kms, ndet = run_device(nh, shaped[sh])
         ms = float(np.median(kms))
         step_ms = 1e3 * dt / len(steps)
-        emit(dict(common, metric="injections/s (lfd_submit_injected, bases resident)", handles=nh,
+        emit(dict(common, metric="injections/s (lfd_submit_injected, bases resident)", handles=nh, shape=sh,
                   value=len(grid) / dt, seconds=dt, steps=len(steps), detections=ndet, step_ms=step_ms,
                   k_inject={"ms_median": ms, "ms_min": float(np.min(kms)), "ms_max": float(np.max(kms)),
                             "bytes_per_step": bytes_step, "gbs": bytes_step / (ms * 1e6), "hbm_peak_gbs": peak,
@@ -182,18 +219,19 @@ def main():
             render_trails(h.host_frames[j], ts)
         h.submit(len(hsteps[k]), [rects[b] for b, _ in hsteps[k]])
 
-    host_stage(0)
-    hs[0].wait()
-    t0 = time.perf_counter()
-    host_stage(0)
-    for k in range(1, len(hsteps)):
-        host_stage(k)
-        hs[(k - 1) & 1].wait()
-    hs[(len(hsteps) - 1) & 1].wait()
-    dt = time.perf_counter() - t0
-    n = sum(len(s) for s in hsteps)
-    emit(dict(common, metric="injections/s (render_trails on the host, one thread, + lfd_submit)", handles=2,
-              value=n / dt, seconds=dt, injections=n, note="first %d steps of the grid" % len(hsteps)))
+    if hsteps:
+        host_stage(0)
+        hs[0].wait()
+        t0 = time.perf_counter()
+        host_stage(0)
+        for k in range(1, len(hsteps)):
+            host_stage(k)
+            hs[(k - 1) & 1].wait()
+        hs[(len(hsteps) - 1) & 1].wait()
+        dt = time.perf_counter() - t0
+        n = sum(len(s) for s in hsteps)
+        emit(dict(common, metric="injections/s (render_trails on the host, one thread, + lfd_submit)", handles=2,
+                  shape="gaussian", value=n / dt, seconds=dt, injections=n, note="first %d steps of the grid" % len(hsteps)))
     for h in hs:
         h.close()
     if args.out:
