@@ -60,7 +60,8 @@ extern "C" {
 
 /* lfd_submit flags */
 #define LFD_INPUT_NATIVE 0      /* host float32, native byte order (what fitsio.read returns) */
-#define LFD_INPUT_BIGENDIAN 1   /* raw FITS payload: big-endian float32, byte-swapped on the device */
+#define LFD_INPUT_BIGENDIAN 1   /* raw FITS payload: big-endian float32, byte-swapped on the device (lfd_submit,
+                                   lfd_upload, lfd_run_resident; lfd_run_pass and lfd_submit_injected refuse it) */
 #define LFD_KEEP_TAPS 2         /* materialise the uint8 stage images for lfd_get_stage */
 #define LFD_FULL_LINES 4        /* sort and keep the full HoughLines lists (taps / parity) */
 #define LFD_SERIAL_PASSES 8     /* run the dim pass after the bright pass on one stream (per-stage timings) */
@@ -260,7 +261,8 @@ int lfd_submit_injected_shaped(lfd_handle* h, int n, const int32_t* base_index, 
                                const lfd_trail_shape* shapes, const int32_t* trail_offsets, int flags);
 
 /* One pass on one already flipped frame (process_field_bright / process_field_dim called directly).
- * If `writeback` != 0 the clipped float image is copied back into `img` (the reference mutates it). */
+ * If `writeback` != 0 the clipped float image is copied back into `img` (the reference mutates it).  `img` is native
+ * float32 in and out: LFD_E_ARG with nothing launched when `flags` holds LFD_INPUT_BIGENDIAN. */
 int lfd_run_pass(lfd_handle* h, int pass, float* img, int flags, int writeback, lfd_result* out);
 
 /* remove_stars' blot on a host image, in place (UN-flipped orientation, same rect convention as lfd_submit). */

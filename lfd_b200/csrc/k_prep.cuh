@@ -53,6 +53,7 @@ __device__ __forceinline__ float bswapf(float v)
 
 // ---- generic variant: also emits the clipped float image (standalone pass functions with write-back).
 // mode 0: whole-frame pipeline: mask + flip + bright clip -> gray0 ; + dim threshold/offset -> gray1
+//         (the library runs k_prep<0, *> there; mode 0 is profiles/lab/prep_lab.cu's reference)
 // mode 1: standalone bright on an already flipped frame (no mask, no flip) -> gray0
 // mode 2: standalone dim on an already flipped frame (no bright clip)     -> gray1
 // Each thread converts 4 consecutive pixels (W % 4 == 0).  hist: [2][n][256].
@@ -60,7 +61,7 @@ __device__ __forceinline__ float bswapf(float v)
 __global__ void __launch_bounds__(256)
 k_prep_generic(const float* __restrict__ in, const u32* __restrict__ mask, u8* __restrict__ gray0,
        u8* __restrict__ gray1, u32* __restrict__ hist0, u32* __restrict__ hist1, float* __restrict__ clipped,
-       Dims d, int mode, int bigendian, float minFlux, float addFlux)
+       Dims d, int mode, float minFlux, float addFlux)
 {
     __shared__ u32 sh[2][256];
     int f = blockIdx.y;
@@ -94,7 +95,6 @@ k_prep_generic(const float* __restrict__ in, const u32* __restrict__ mask, u8* _
             if (q >= quads) continue;
             int y = yy[u], x = xx[u];
             float4 v = vv[u];
-            if (bigendian) { v.x = bswapf(v.x); v.y = bswapf(v.y); v.z = bswapf(v.z); v.w = bswapf(v.w); }
             float a[4] = {v.x, v.y, v.z, v.w};
             u32 mbits = 0;
             if (mode == 0) mbits = (mask[(size_t)f * d.NW + (size_t)y * d.WW + (x >> 5)] >> (x & 31)) & 0xf;
@@ -190,9 +190,8 @@ __device__ __forceinline__ u32 pack_low_bytes(u32 u0, u32 u1, u32 u2, u32 u3)
 
 // one float4: mask, clips, both conversions.  t[] are the un-flipped-source pixels of 4 consecutive columns.
 template <int MODE>
-__device__ __forceinline__ void prep4(float4 v, u32 mb, int bigendian, float minFlux, float addFlux, u32& g0, u32& g1)
+__device__ __forceinline__ void prep4(float4 v, u32 mb, float minFlux, float addFlux, u32& g0, u32& g1)
 {
-    if (bigendian) { v.x = bswapf(v.x); v.y = bswapf(v.y); v.z = bswapf(v.z); v.w = bswapf(v.w); }
     if (MODE == 0 && mb) {
         if (mb & 1u) v.x = 0.0f;
         if (mb & 2u) v.y = 0.0f;
@@ -350,6 +349,7 @@ __global__ void __launch_bounds__(PR_WARPS * 32, MINB)
 k_prep(const float* __restrict__ in, const u32* __restrict__ mask, u8* __restrict__ gray0, u8* __restrict__ gray1,
             u32* __restrict__ hist0, u32* __restrict__ hist1, Dims d, int nframes, float minFlux, float addFlux)
 {
+    static_assert(MODE == 0 || !BE, "the standalone passes (lfd_run_pass) read native float32 only");
     extern __shared__ __align__(128) unsigned char dsm[];
     float4* ring = reinterpret_cast<float4*>(dsm);                                       // [PR_WARPS][PR_S][PR_CF4]
     u32* sh = reinterpret_cast<u32*>(dsm + (size_t)PR_WARPS * PR_S * PR_CB);             // [2][256]
@@ -425,7 +425,7 @@ k_prep(const float* __restrict__ in, const u32* __restrict__ mask, u8* __restric
             u32 mb = 0;
             if (anym) mb = (__shfl_sync(FULLMASK, mcur, (lane >> 3) + 4 * k) >> ((lane & 7) << 2)) & 0xfu;
             if (MODE == 0) prep4_pipe<BE>(v[k], mb, thr, minFlux, addFlux, G0[k], G1[k]);
-            else prep4<MODE>(v[k], 0u, BE ? 1 : 0, minFlux, addFlux, G0[k], G1[k]);
+            else prep4<MODE>(v[k], 0u, minFlux, addFlux, G0[k], G1[k]);
         }
         if (nf4 == PR_CF4) {
 #pragma unroll

@@ -460,7 +460,7 @@ static int create_impl(lfd_handle* h, int device, int max_batch, int H, int W, c
         int per_sm[3] = {0, 0, 0};
         // k_prep keeps its TMA rings in dynamic shared memory (above the 48 KB default limit)
 #define PREP_ATTR(M, E) CK(cudaFuncSetAttribute(k_prep<M, E>, cudaFuncAttributeMaxDynamicSharedMemorySize, PR_SMEM))
-        PREP_ATTR(0, false); PREP_ATTR(0, true); PREP_ATTR(1, false); PREP_ATTR(1, true); PREP_ATTR(2, false); PREP_ATTR(2, true);
+        PREP_ATTR(0, false); PREP_ATTR(0, true); PREP_ATTR(1, false); PREP_ATTR(2, false);
 #undef PREP_ATTR
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], k_prep<0, false>, PR_WARPS * 32, PR_SMEM));
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], k_prep<1, false>, PR_WARPS * 32, PR_SMEM));
@@ -890,7 +890,7 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
     u32* hist1 = h->hist + (size_t)h->B * 256;
     if (clipped) {
         int pblocks = (d.N / 4 + 255) / 256; if (pblocks > 1184) pblocks = 1184;
-        k_prep_generic<<<dim3(pblocks, n), 256, 0, s>>>(h->in, h->starmask, h->gray[0], h->gray[1], h->hist, hist1, clipped, d, mode, be,
+        k_prep_generic<<<dim3(pblocks, n), 256, 0, s>>>(h->in, h->starmask, h->gray[0], h->gray[1], h->hist, hist1, clipped, d, mode,
                                                       (float)pd.minFlux, (float)pd.addFlux); LAUNCH_CHECK();
     } else {
         // one wave of resident CTAs spread over the frames of the batch (a second, partial wave would double the time)
@@ -904,8 +904,8 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
         dim3 pg(rb, gy);
 #define PREP_LAUNCH(M, E) k_prep<M, E><<<pg, PR_WARPS * 32, PR_SMEM, s>>>(h->in, h->starmask, h->gray[0], h->gray[1], h->hist, hist1, d, n, mf, af)
         if (mode == 0) { if (be) PREP_LAUNCH(0, true); else PREP_LAUNCH(0, false); }
-        else if (mode == 1) { if (be) PREP_LAUNCH(1, true); else PREP_LAUNCH(1, false); }
-        else { if (be) PREP_LAUNCH(2, true); else PREP_LAUNCH(2, false); }
+        else if (mode == 1) PREP_LAUNCH(1, false);         // lfd_run_pass: native order only
+        else PREP_LAUNCH(2, false);
 #undef PREP_LAUNCH
         LAUNCH_CHECK();
     }
@@ -1293,6 +1293,7 @@ extern "C" int lfd_run_pass(lfd_handle* h, int pass, float* img, int flags, int 
     if (!h || !img || (pass != 0 && pass != 1)) { if (h) h->err = "bad argument"; return LFD_E_ARG; }
     cudaSetDevice(h->device);
     if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    if (flags & LFD_INPUT_BIGENDIAN) { h->err = "lfd_run_pass reads and writes back native float32 (LFD_INPUT_BIGENDIAN)"; return LFD_E_ARG; }
     h->rect_off_h[0] = h->rect_off_h[1] = 0;
     CK(cudaMemcpyAsync(h->in, img, (size_t)h->d.N * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     int rc = run_pipeline(h, 1, flags, pass == 0 ? 1 : 2, writeback != 0);
