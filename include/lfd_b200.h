@@ -89,9 +89,11 @@ enum lfd_stage {
                                 lfd_get_stage_count: n_lines, capped at the handle's max_lines */
     LFD_STAGE_LINES_BOX = 16,
     LFD_STAGE_CLIPPED = 17,  /* float32 H*W: the frame after the pass's in-place clip (processfield.py:342,453-454) */
-    LFD_STAGE_INPUT = 18     /* float32 H*W: the un-flipped frame of a batch slot as the last whole-frame run read it, native
+    LFD_STAGE_INPUT = 18,    /* float32 H*W: the un-flipped frame of a batch slot as the last whole-frame run read it, native
                                 byte order (swapped back after an LFD_INPUT_BIGENDIAN run); needs no LFD_KEEP_TAPS; `pass` is
                                 ignored.  LFD_E_STATE after lfd_run_pass / lfd_blot / a bare lfd_upload, which overwrite the slots */
+    LFD_STAGE_RECT_SCREEN = 19 /* int32[n]: 1 where the aspect screen (DESIGN.md §7) rejected the contour, same order and
+                                  count as LFD_STAGE_RECTS; recorded with and without LFD_KEEP_TAPS */
 };
 
 /* one pass's parameters: the keys of params_bright / params_dim (detecttrails.py:202-230) */
@@ -137,7 +139,9 @@ typedef struct lfd_result {
 /* a minimum-area rectangle as cv2.minAreaRect returns it (processfield.py:249) */
 typedef struct lfd_rect {
     float cx, cy, w, h, angle;
-    int32_t kind;               /* 0 = outer border of an edge component, 1 = hole border, 2 = not retrieved (RETR_EXTERNAL) */
+    int32_t kind;               /* 0 = outer border of an edge component, 1 = hole border, 2 = not retrieved (RETR_EXTERNAL),
+                                   3 = not fitted: its aspect bound (DESIGN.md §7) proves it cannot pass; only in runs without
+                                   LFD_KEEP_TAPS, which fit every contour.  cx .. angle and box are 0, key is set */
     int32_t key;                /* raster-first pixel index (y*W+x) of the component / hole */
     int32_t passed;             /* 1 if it passed the length/width filter (processfield.py:256-257) */
     int32_t box[8];             /* int32(boxPoints(rect)) x0,y0..x3,y3 (processfield.py:259-260); valid if passed */
@@ -348,7 +352,8 @@ int lfd_ingest_batch(void* staging, int height, int width, int n, const char* co
 /* Work counters of the last run, summed over the batch: [0] nonzero px voted equ, [1] box, [2] votes,
  * [3] runs fg, [4] runs bg, [5] contours, [6] passing rects, [7] frames that ran dim, [8] frames that ran Hough,
  * [11] contours whose rectangle a whole warp computed, [12] of those, short contours handed over because their thread's hull stack was full,
- * [14] labelling bands whose run-id look-back gave up waiting (frame reported LFD_FRAME_OVERFLOW; expected 0). */
+ * [14] labelling bands whose run-id look-back gave up waiting (frame reported LFD_FRAME_OVERFLOW; expected 0),
+ * [15] contours the aspect screen proved unable to pass (fitted anyway with LFD_KEEP_TAPS). */
 int lfd_get_counters(lfd_handle* h, int64_t* out, int n);
 
 #ifdef __cplusplus

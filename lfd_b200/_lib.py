@@ -23,7 +23,7 @@ MAX_SET_LINES = 16
 
 STAGES = {"mask": 0, "gray": 1, "equ": 2, "eroded": 3, "morph": 4, "canny": 5, "box": 6, "hist": 7, "lut": 8,
           "nms": 9, "fg_labels": 10, "bg_labels": 11, "rects": 12, "accum_equ": 13, "accum_box": 14,
-          "lines_equ": 15, "lines_box": 16, "clipped": 17, "input": 18}
+          "lines_equ": 15, "lines_box": 16, "clipped": 17, "input": 18, "rect_screen": 19}
 MAX_INJECT_TRAILS = 16
 TRAIL_DTYPE = np.dtype([("x0", "<f4"), ("y0", "<f4"), ("x1", "<f4"), ("y1", "<f4"), ("sigma", "<f4"), ("peak", "<f4")])
 MAX_TABLE_SAMPLES, MAX_TRAIL_TABLES = 4096, 4096
@@ -485,6 +485,8 @@ class Handle:
             out = np.empty((H, W), np.float32)
         elif stage == "rects":
             out = np.zeros(self.stage_count(frame, pass_, stage), RECT_DTYPE)
+        elif stage == "rect_screen":
+            out = np.zeros(self.stage_count(frame, pass_, stage), np.int32)
         elif stage in ("accum_equ", "accum_box"):
             out = np.empty(self.stage_count(frame, pass_, stage), np.int32)
         elif stage in ("lines_equ", "lines_box"):
@@ -563,7 +565,7 @@ class Handle:
         self._ck(self._L.lfd_get_counters(self.h, c, 16))
         names = ["nnz_equ", "nnz_box", "votes", "runs_fg", "runs_bg", "contours", "passing_rects", "frames_dim",
                  "frames_hough", "frames_bright_run", "frames_dim_run", "rects_warp_path", "rects_thread_overflow",
-                 "hough_smem_atomics", "ccl_lookback_stalls"]
+                 "hough_smem_atomics", "ccl_lookback_stalls", "rects_screened"]
         return {k: int(c[i]) for i, k in enumerate(names)}
 
     def timer_mark(self, slot):

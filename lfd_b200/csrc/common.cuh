@@ -29,6 +29,7 @@ struct FrameCtl {
     int status;           // LFD_FRAME_* bits
     int detected;         // this pass accepted a line (k_check_theta)
     int ncomp_saved[2][2]; // [pass][kind] contour counts kept for the RECTS tap
+    int nsurv;            // contours k_rects_screen kept in the rectangle launch whose first frame this is
 };
 
 // A run of set bits in one mask row.

@@ -12,6 +12,7 @@
 struct RectBuf {
     lfd_rect* rects;     // [2*maxcomp]  same indexing as CompBuf entries
     int* passing;        // [2*maxcomp]  entry indices of rectangles that passed
+    int* screened;       // [2*maxcomp]  1 = k_rects_screen proved that the contour cannot pass (recorded in every mode)
     lfdgeom::Pt* hull;   // [hullcap]
     float* hullf;        // [3*hullcap]
 };
@@ -39,6 +40,117 @@ struct RectBuf {
 #define RECT_WARP_WORDS (RECT_WARP_WORDS_T > RECT_WARP_WORDS_W ? RECT_WARP_WORDS_T : RECT_WARP_WORDS_W)
 
 __host__ __device__ inline size_t rects_smem(int nframes) { return (size_t)RECT_WARPS * RECT_WARP_WORDS * 4 + ((size_t)nframes + 1) * 4; }
+
+// Flat task numbering of the contours of a launch: pre[f] = contours of the active frames before f (fg entries of a
+// frame first, then its bg entries).  Warp 0 of the block fills pre[0..nframes]; the caller synchronises.
+__device__ __forceinline__ void rect_task_prefix(const CompBuf* __restrict__ comps, const FrameCtl* __restrict__ ctl, int pass,
+                                                 int nframes, int* pre)
+{
+    const int lane = lane_id();
+    if ((threadIdx.x >> 5) != 0) return;
+    int carry = 0;
+    for (int f0 = 0; f0 < nframes; f0 += 32) {
+        int ff = f0 + lane, c = 0;
+        if (ff < nframes && ctl[ff].active[pass]) {
+            int mc = comps[ff].maxcomp;
+            c = min(ctl[ff].ncomp[0], mc) + min(ctl[ff].ncomp[1], mc);
+        }
+        int inc = c;
+        for (int o = 1; o < 32; o <<= 1) { int v = __shfl_up_sync(FULLMASK, inc, o); if (lane >= o) inc += v; }
+        if (ff < nframes) pre[ff + 1] = carry + inc;
+        carry += __shfl_sync(FULLMASK, inc, 31);
+    }
+    if (lane == 0) pre[0] = 0;
+}
+
+// task -> (frame, entry, kind): the largest f with pre[f] <= task
+__device__ __forceinline__ void rect_task_decode(const int* pre, int nframes, const CompBuf* __restrict__ comps,
+                                                 const FrameCtl* __restrict__ ctl, int task, int* f, int* e, int* kind)
+{
+    int flo = 0, fhi = nframes;
+    while (fhi - flo > 1) { int mid = (flo + fhi) >> 1; if (pre[mid] <= task) flo = mid; else fhi = mid; }
+    const int i = task - pre[flo];
+    const int mc = comps[flo].maxcomp;
+    const int n0 = min(ctl[flo].ncomp[0], mc);
+    *f = flo;
+    *kind = i >= n0;
+    *e = *kind ? mc + (i - n0) : i;
+}
+
+// ---- aspect screen -------------------------------------------------------------------------------------------------
+// A contour passes only if length / width > lwTresh for its minimum-area rectangle.  With P the contour's points, every
+// side of that rectangle is P's extent along some direction, so length <= diam(P) <= D (D^2 = bw^2 + bh^2, the squared
+// diagonal of P's bounding box) and width >= w(P), the minimum width of P's hull.  The hull lies in a strip of width w(P)
+// and length at most diam(P), so area(hull) <= w(P) * D; and the polygon through the row extremes of P (down the
+// rowmin side, up the rowmax side) has its vertices in P, so its area A <= area(hull).  Hence
+//   length / width <= D^2 / A,
+// and a contour with D^2 < lwTresh * A cannot pass, whatever its hull.  2A = sum over consecutive non-empty rows of
+// dy * (w_k + w_k+1) with w = rowmax - rowmin, an exact integer.  The test keeps a relative margin of 1e-4 for the float
+// rounding of the fitted sides; lwTresh <= 1 or NaN rejects nothing (A <= bw * bh <= D^2 / 2).  It needs no minLen.
+#define SCREEN_THREADS 256
+#define SCREEN_MARGIN 1e-4
+
+__host__ __device__ inline size_t screen_smem(int nframes) { return ((size_t)nframes + 1) * 4; }
+
+// One thread per contour over the flat task list.  Every contour's verdict goes to rb.screened[e].  With `tasks`
+// (production runs), a rejected contour gets its lfd_rect record here (kind 3, never passes) and the others are appended
+// to tasks[0 .. ctl[0].nsurv) for k_rects_warp; without it (taps, the standalone fit) k_rects_warp fits every contour.
+// counters[15] counts the rejected contours in every mode.
+__global__ void __launch_bounds__(SCREEN_THREADS)
+k_rects_screen(const CompBuf* __restrict__ comps, RectBuf* __restrict__ rbufs, const CclBuf* __restrict__ ccl0,
+               const CclBuf* __restrict__ ccl1, FrameCtl* __restrict__ ctl, int pass, int nframes, Dims d, double lwTresh,
+               int* __restrict__ tasks, unsigned long long* __restrict__ counters)
+{
+    extern __shared__ int spre[];      // [nframes + 1]
+    rect_task_prefix(comps, ctl, pass, nframes, spre);
+    __syncthreads();
+    const int total = spre[nframes], lane = lane_id();
+    for (int base = blockIdx.x * SCREEN_THREADS; base < total; base += gridDim.x * SCREEN_THREADS) {
+        const int task = base + (int)threadIdx.x;
+        const bool valid = task < total;
+        bool drop = false;
+        int f = 0, e = 0, kind = 0;
+        if (valid) {
+            rect_task_decode(spre, nframes, comps, ctl, task, &f, &e, &kind);
+            const CompBuf& cb = comps[f];
+            const int hh = cb.h[e], slot = cb.slot[e];
+            const int* __restrict__ rmin = cb.rowmin + slot;
+            const int* __restrict__ rmax = cb.rowmax + slot;
+            int xlo = 0x7fffffff, xhi = -1, ylo = -1, py = -1, pw = 0;
+            long long a2 = 0;
+#pragma unroll 4
+            for (int r = 0; r < hh; r++) {
+                const int a = rmin[r], b = rmax[r];
+                if (a > b) continue;                         // empty row
+                xlo = min(xlo, a); xhi = max(xhi, b);
+                const int w = b - a;
+                if (py >= 0) a2 += (long long)(r - py) * (w + pw);
+                else ylo = r;
+                py = r; pw = w;
+            }
+            const long long bw = (long long)xhi - xlo, bh = (long long)py - ylo;
+            drop = py >= 0 && (double)(bw * bw + bh * bh) * (1.0 + SCREEN_MARGIN) < lwTresh * (0.5 * (double)a2);
+            rbufs[f].screened[e] = drop ? 1 : 0;
+            if (drop && tasks) {
+                lfd_rect o;
+                memset(&o, 0, sizeof(o));
+                o.kind = 3;                                  // screened: no fit, cannot pass
+                Run rr = (kind ? ccl1[f] : ccl0[f]).runs[cb.root[e]];
+                o.key = (int)rr.y * d.W + (int)rr.xs;
+                rbufs[f].rects[e] = o;
+            }
+        }
+        const unsigned dropped = __ballot_sync(FULLMASK, valid && drop);
+        if (lane == 0 && dropped) atomicAdd(&counters[15], (unsigned long long)__popc(dropped));
+        if (tasks) {
+            const unsigned keep = __ballot_sync(FULLMASK, valid && !drop);
+            int slot0 = 0;
+            if (lane == 0 && keep) slot0 = atomicAdd(&ctl[0].nsurv, __popc(keep));
+            slot0 = __shfl_sync(FULLMASK, slot0, 0);
+            if (valid && !drop) tasks[slot0 + __popc(keep & ((1u << lane) - 1u))] = task;
+        }
+    }
+}
 
 __device__ __forceinline__ u32 pt_pack(int x, int y) { return (u32)(x & 0xffff) | ((u32)y << 16); }
 __device__ __forceinline__ lfdgeom::Pt pt_unpack(u32 v) { lfdgeom::Pt p; p.x = (int)(v & 0xffffu); p.y = (int)(v >> 16); return p; }
@@ -321,46 +433,30 @@ __device__ __forceinline__ void rect_warp_path(const int* __restrict__ rmin, con
     }
 }
 
-// grid = (any, 1); dynamic smem = rects_smem(nframes)
+// grid = (any, 1); dynamic smem = rects_smem(nframes).  `tasks`: the survivors of k_rects_screen (ctl[0].nsurv of them),
+// one per warp; nullptr = every contour of the launch, RECT_TPW per warp.
 __global__ void __launch_bounds__(RECT_WARPS * 32)
 k_rects_warp(CompBuf* __restrict__ comps, RectBuf* __restrict__ rbufs, const CclBuf* __restrict__ ccl0,
              const CclBuf* __restrict__ ccl1, FrameCtl* __restrict__ ctl, int pass, int nframes,
-             Dims d, double minLen, double lwTresh, unsigned long long* __restrict__ counters, int external_only)
+             Dims d, double minLen, double lwTresh, unsigned long long* __restrict__ counters, int external_only,
+             const int* __restrict__ tasks)
 {
     extern __shared__ u32 rsm[];
     const int warp = threadIdx.x >> 5, lane = lane_id();
     u32* wsm = rsm + warp * RECT_WARP_WORDS;
     int* pre = reinterpret_cast<int*>(rsm + RECT_WARPS * RECT_WARP_WORDS);      // [nframes + 1]
-    if (warp == 0) {
-        int carry = 0;
-        for (int f0 = 0; f0 < nframes; f0 += 32) {
-            int ff = f0 + lane, c = 0;
-            if (ff < nframes && ctl[ff].active[pass]) {
-                int mc = comps[ff].maxcomp;
-                c = min(ctl[ff].ncomp[0], mc) + min(ctl[ff].ncomp[1], mc);
-            }
-            int inc = c;
-            for (int o = 1; o < 32; o <<= 1) { int v = __shfl_up_sync(FULLMASK, inc, o); if (lane >= o) inc += v; }
-            if (ff < nframes) pre[ff + 1] = carry + inc;
-            carry += __shfl_sync(FULLMASK, inc, 31);
-        }
-        if (lane == 0) pre[0] = 0;
-    }
+    rect_task_prefix(comps, ctl, pass, nframes, pre);
     __syncthreads();
-    const int total_all = pre[nframes];
-    for (int base = (blockIdx.x * RECT_WARPS + warp) * RECT_TPW; base < total_all; base += gridDim.x * RECT_WARPS * RECT_TPW) {
-        const int task = base + lane;
-        const bool valid = lane < RECT_TPW && task < total_all;
+    const int ntasks = tasks ? ctl[0].nsurv : pre[nframes];
+    // Survivors are few (a few % of the contours) and mostly the tall ones that take the serial warp path: one per warp,
+    // so that they run side by side instead of up to RECT_TPW after one another in one warp.
+    const int tpw = tasks ? 1 : RECT_TPW;
+    for (int base = (blockIdx.x * RECT_WARPS + warp) * tpw; base < ntasks; base += gridDim.x * RECT_WARPS * tpw) {
+        const bool valid = lane < tpw && base + lane < ntasks;
         int f = 0, e = 0, kind = 0, hh = 0, slot = 0, ho = 0, y0 = 0;
         if (valid) {
-            int flo = 0, fhi = nframes;           // largest f with pre[f] <= task
-            while (fhi - flo > 1) { int mid = (flo + fhi) >> 1; if (pre[mid] <= task) flo = mid; else fhi = mid; }
-            f = flo;
-            const int i = task - pre[f];
-            const int mc = comps[f].maxcomp;
-            const int n0 = min(ctl[f].ncomp[0], mc);
-            kind = i >= n0;
-            e = kind ? mc + (i - n0) : i;
+            const int task = tasks ? tasks[base + lane] : base + lane;
+            rect_task_decode(pre, nframes, comps, ctl, task, &f, &e, &kind);
             const CompBuf& cbr = comps[f];
             hh = cbr.h[e]; slot = cbr.slot[e]; ho = cbr.hulloff[e]; y0 = cbr.y0[e];
         }

@@ -33,7 +33,7 @@ static std::string g_create_error;
 
 // dynamic shared-memory opt-in (cudaFuncSetAttribute) is per function AND per device: high-water marks per device
 #define LFD_MAX_DEVICES 64
-struct DevLimits { size_t band_max = 48 * 1024, rects_max = 48 * 1024, anyk_max = 48 * 1024; };
+struct DevLimits { size_t band_max = 48 * 1024, rects_max = 48 * 1024, screen_max = 48 * 1024, anyk_max = 48 * 1024; };
 static DevLimits g_dev_limits[LFD_MAX_DEVICES];
 
 // with the two passes overlapped, a batch of >= 16 frames is cut in this many parts (1 / 2 / 3 / 4 parts measured
@@ -54,9 +54,9 @@ static const char* k_timing_names[] = {
 // Brackets: a CUDA event on each side of the launches that carry the step (recorded on the launching stream, also
 // inside the captured graph), so that bench.py can quote the average launch duration of the time-dominant kernel
 // measured live in the timed region (lfd_get_kernel_times).
-enum { KB_MORPH = 0, KB_NMS, KB_CCL_BAND_FG, KB_CCL_BAND_BG, KB_RECTS, KB_HOUGH_VOTE, KB_COUNT };
+enum { KB_MORPH = 0, KB_NMS, KB_CCL_BAND_FG, KB_CCL_BAND_BG, KB_RECTS_SCREEN, KB_RECTS, KB_HOUGH_VOTE, KB_COUNT };
 static const char* k_bracket_names[KB_COUNT] = {"k_morph_march", "k_nms_march", "k_ccl_band(fg)", "k_ccl_band(bg)",
-                                                "k_rects_warp", "k_hough_vote"};
+                                                "k_rects_screen", "k_rects_warp", "k_hough_vote"};
 
 struct HoughBufs {
     HoughCfg hc;
@@ -121,6 +121,7 @@ struct lfd_handle {
     CclBuf* ccl_d[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};   // [pass][kind] -> [B]
     CompBuf* comp_d[2] = {nullptr, nullptr}; // per pass: [B]
     RectBuf* rbuf_d[2] = {nullptr, nullptr}; // per pass: [B]
+    int* rtasks[2] = {nullptr, nullptr};     // per pass: [B][2*max_components] k_rects_screen's survivors, a launch's from its first frame
     std::vector<CclBuf> ccl_h[2][2];
     std::vector<CompBuf> comp_h[2];
     std::vector<RectBuf> rbuf_h[2];
@@ -479,6 +480,10 @@ static int create_impl(lfd_handle* h, int device, int max_batch, int H, int W, c
             CK(cudaFuncSetAttribute(k_rects_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rects_smem(max_batch)));
             L.rects_max = rects_smem(max_batch);
         }
+        if (screen_smem(max_batch) > L.screen_max) {
+            CK(cudaFuncSetAttribute(k_rects_screen, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)screen_smem(max_batch)));
+            L.screen_max = screen_smem(max_batch);
+        }
     }
     for (int i = 0; i <= N_TIMINGS; i++) { CK(cudaEventCreate(&h->ev[i])); h->ev_valid[i] = true; }
     for (int i = 0; i < 4; i++) { CK(cudaEventCreate(&h->mark[i])); h->mark_valid[i] = true; }
@@ -555,11 +560,12 @@ static int create_impl(lfd_handle* h, int device, int max_batch, int H, int W, c
         h->rbuf_h[p].resize(B);
         lfdgeom::Pt* hulls; float* hullfs;
         DA(hulls, (size_t)B * hullcap); DA(hullfs, (size_t)B * 3 * hullcap);
-        lfd_rect* rects; int* passing;
-        DA(rects, (size_t)B * 2 * MC); DA(passing, (size_t)B * 2 * MC);
+        lfd_rect* rects; int *passing, *screened;
+        DA(rects, (size_t)B * 2 * MC); DA(passing, (size_t)B * 2 * MC); DA(screened, (size_t)B * 2 * MC);
+        DA(h->rtasks[p], (size_t)B * 2 * MC);
         for (int f = 0; f < B; f++) {
             RectBuf& r = h->rbuf_h[p][f];
-            r.rects = rects + (size_t)f * 2 * MC; r.passing = passing + (size_t)f * 2 * MC;
+            r.rects = rects + (size_t)f * 2 * MC; r.passing = passing + (size_t)f * 2 * MC; r.screened = screened + (size_t)f * 2 * MC;
             r.hull = hulls + (size_t)f * hullcap; r.hullf = hullfs + (size_t)f * 3 * hullcap;
         }
         DA(h->rbuf_d[p], (size_t)B);
@@ -819,9 +825,15 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
     k_ccl_alloc_flat<<<flat, 256, 0, s>>>(v_ccl1, nullptr, v_comp, C, pass, d, 1); LAUNCH_CHECK();
     k_ccl_extremes_flat<<<flat, 256, 0, s>>>(v_edges, v_ccl1, v_comp, C, pass, d, 1); LAUNCH_CHECK();
     STAGE_EVENT(tbase + 4);
-    // rectangles + box image
+    // rectangles + box image.  The screen rejects the contours whose aspect bound proves they cannot pass (most of them:
+    // the NMS rings around stars and their holes); only the survivors are fitted.  With taps, and in the standalone fit
+    // (part 1), whose RECTS tap is its output, every contour is fitted and the screen only records its verdicts.
+    int* const v_tasks = (!taps && part == 0) ? h->rtasks[pass] + (size_t)f0 * 2 * h->cfg.max_components : nullptr;
+    KB_MARK(KB_RECTS_SCREEN, 0);
+    k_rects_screen<<<h->sm_count * 2, SCREEN_THREADS, screen_smem(n), s>>>(v_comp, v_rbuf, v_ccl0, v_ccl1, C, pass, n, d, pp.lwTresh, v_tasks, cnt); LAUNCH_CHECK();
+    KB_MARK(KB_RECTS_SCREEN, 1);
     KB_MARK(KB_RECTS, 0);
-    k_rects_warp<<<h->sm_count * 16, RECT_WARPS * 32, rects_smem(n), s>>>(v_comp, v_rbuf, v_ccl0, v_ccl1, C, pass, n, d, pp.minAreaRectMinLen, pp.lwTresh, (unsigned long long*)h->counters_d, pp.contoursMode == 0 ? 1 : 0); LAUNCH_CHECK();
+    k_rects_warp<<<h->sm_count * 16, RECT_WARPS * 32, rects_smem(n), s>>>(v_comp, v_rbuf, v_ccl0, v_ccl1, C, pass, n, d, pp.minAreaRectMinLen, pp.lwTresh, cnt, pp.contoursMode == 0 ? 1 : 0, v_tasks); LAUNCH_CHECK();
     KB_MARK(KB_RECTS, 1);
     CK(cudaMemsetAsync(v_box, 0, (size_t)n * d.NW * sizeof(u32), s));
     k_fill_boxes<<<dim3(16, n), 128, 0, s>>>(v_rbuf, v_box, C, pass, d); LAUNCH_CHECK();
@@ -1340,7 +1352,8 @@ extern "C" int lfd_get_stage_count(lfd_handle* h, int frame, int pass, int stage
     cudaSetDevice(h->device);
     const HoughBufs& hb = h->hb[pass];
     switch (stage) {
-    case LFD_STAGE_RECTS: {
+    case LFD_STAGE_RECTS:
+    case LFD_STAGE_RECT_SCREEN: {
         const FrameCtl& ch = h->ctl_h[(size_t)pass * h->B + frame];
         *count = min(ch.ncomp_saved[pass][0], h->cfg.max_components) + min(ch.ncomp_saved[pass][1], h->cfg.max_components);
         return LFD_OK;
@@ -1404,6 +1417,17 @@ extern "C" int lfd_get_stage(lfd_handle* h, int frame, int pass, int stage, void
         const RectBuf& rb = h->rbuf_h[pass][frame];
         if (n0) CK(cudaMemcpyAsync(host_out, rb.rects, (size_t)n0 * sizeof(lfd_rect), cudaMemcpyDeviceToHost, s));
         if (n1) CK(cudaMemcpyAsync((char*)host_out + (size_t)n0 * sizeof(lfd_rect), rb.rects + h->cfg.max_components, (size_t)n1 * sizeof(lfd_rect), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        return LFD_OK;
+    }
+    case LFD_STAGE_RECT_SCREEN: {
+        const FrameCtl& ch = h->ctl_h[(size_t)pass * h->B + frame];
+        int n0 = min(ch.ncomp_saved[pass][0], h->cfg.max_components), n1 = min(ch.ncomp_saved[pass][1], h->cfg.max_components);
+        need = (size_t)(n0 + n1) * sizeof(int);
+        if (bytes < need) { h->err = "buffer too small"; return LFD_E_ARG; }
+        const RectBuf& rb = h->rbuf_h[pass][frame];
+        if (n0) CK(cudaMemcpyAsync(host_out, rb.screened, (size_t)n0 * sizeof(int), cudaMemcpyDeviceToHost, s));
+        if (n1) CK(cudaMemcpyAsync((char*)host_out + (size_t)n0 * sizeof(int), rb.screened + h->cfg.max_components, (size_t)n1 * sizeof(int), cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
         return LFD_OK;
     }
