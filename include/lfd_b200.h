@@ -304,8 +304,8 @@ int lfd_get_timings(lfd_handle* h, float* ms, int max_entries, int* n_entries);
 /* Bracketed kernels (the ones that carry the step: morphology, Sobel/NMS, the band CCL kernels, rectangles, Hough vote)
    of the last collected batch: CUDA events recorded on the launching stream on both sides of the launch - also inside
    the captured graph of the production path - so the durations are measured live, with the other streams running.
-   index = 0 .. 11 (6 kernels x 2 passes); ms is summed over the batch parts, launches = number of parts.
-   index 12 = k_inject of the last collected lfd_submit_injected batch (always bracketed; launches 0 otherwise).
+   index = 0 .. 13 (7 kernels x 2 passes); ms is summed over the batch parts, launches = number of parts.
+   index 14 = k_inject of the last collected lfd_submit_injected batch (always bracketed; launches 0 otherwise).
    Returns LFD_E_ARG past the last index. */
 int lfd_get_kernel_times(lfd_handle* h, int index, const char** name, int* pass, float* ms, int* launches);
 const char* lfd_timing_name(int i);

@@ -70,6 +70,13 @@ struct HoughBufs {
     size_t smem = 0;
 };
 
+// lfd_hough_lines' buffers, sized for the image of its last call
+struct HoughScratch {
+    int H = 0, W = 0;
+    u8* img = nullptr; u32* mask = nullptr; uint2* segs = nullptr; FrameCtl* ctl = nullptr; lfd_result* res = nullptr;
+    HoughBufs hb;
+};
+
 struct lfd_handle {
     int device = 0, B = 0, sm_count = 148;
     Dims d;
@@ -127,6 +134,7 @@ struct lfd_handle {
     std::vector<RectBuf> rbuf_h[2];
     std::vector<void*> allocs;
     HoughBufs hb[2];
+    HoughScratch hs;                  // lfd_hough_lines, allocated on first use
     // injection campaigns (lfd_set_base / lfd_submit_injected): resident base frames and per-slot trails
     float* base_d = nullptr;          // [base_cap][N], replaced by lfd_set_base
     int n_base = 0, base_cap = 0;
@@ -202,6 +210,9 @@ struct lfd_handle {
         }                                                                                          \
     } while (0)
 
+// propagate an LFD_* error code
+#define TRY(call) do { int rc_ = (call); if (rc_ != LFD_OK) return rc_; } while (0)
+
 static void ktime_mark(lfd_handle* h, int line)
 {
     if (h->kn >= (int)h->kev.size()) { cudaEvent_t e; cudaEventCreate(&e); h->kev.push_back(e); h->kline.push_back(0); }
@@ -223,6 +234,14 @@ static int dev_alloc(lfd_handle* h, T** p, size_t count)
 }
 
 static int next_pow2(int v) { int p = 1; while (p < v) p <<= 1; return p; }
+
+// prologue of the entry points that enqueue work: the handle's device, and no batch in flight
+static int enter(lfd_handle* h)
+{
+    cudaSetDevice(h->device);
+    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    return LFD_OK;
+}
 
 // ------------------------------------------------------------------------------------------------
 // small bookkeeping kernels
@@ -309,6 +328,19 @@ static void hough_dims_host(int H, int W, double rho_, double theta_, int* numan
     *numrho = (int)lrint(((max_rho - min_rho) + 1) / rho);
 }
 
+static void hough_free(HoughBufs& hb)
+{
+    cudaFree(hb.accum); cudaFree(hb.keys); cudaFree(hb.lines); cudaFree(hb.tabSin);   // tabCos lies in tabSin's block
+    hb.accum = nullptr; hb.keys = nullptr; hb.lines = nullptr; hb.tabSin = hb.tabCos = nullptr;
+}
+
+static void hough_scratch_free(HoughScratch& hs)
+{
+    cudaFree(hs.img); cudaFree(hs.mask); cudaFree(hs.segs); cudaFree(hs.ctl); cudaFree(hs.res);
+    hs.img = nullptr; hs.mask = nullptr; hs.segs = nullptr; hs.ctl = nullptr; hs.res = nullptr; hs.H = hs.W = 0;
+    hough_free(hs.hb);
+}
+
 static int hough_setup(lfd_handle* h, HoughBufs* hb, int H, int W, double rho_, double theta_, int threshold,
                        int nframes, bool want_lines, int max_lines_cfg)
 {
@@ -346,11 +378,7 @@ static int hough_setup(lfd_handle* h, HoughBufs* hb, int H, int W, double rho_, 
     size_t key_stride = (size_t)next_pow2((int)cells);
     bool realloc_needed = (accum_stride != hb->accum_stride) || (key_stride != hb->key_stride) || !hb->accum;
     if (realloc_needed) {
-        if (hb->accum) cudaFree(hb->accum);
-        if (hb->keys) cudaFree(hb->keys);
-        if (hb->lines) cudaFree(hb->lines);
-        if (hb->tabSin) cudaFree(hb->tabSin);
-        hb->accum = nullptr; hb->keys = nullptr; hb->lines = nullptr; hb->tabSin = nullptr;
+        hough_free(*hb);
         CK(cudaMalloc((void**)&hb->accum, (size_t)nframes * 2 * accum_stride * sizeof(int)));
         CK(cudaMalloc((void**)&hb->keys, (size_t)nframes * 2 * key_stride * sizeof(u64)));
         CK(cudaMalloc((void**)&hb->tabSin, (size_t)2 * hc.numangle * sizeof(float)));
@@ -387,24 +415,13 @@ extern "C" int lfd_destroy(lfd_handle* h)
             if (h->xs[k][p] && h->xs[k][p] != h->stream) cudaStreamSynchronize(h->xs[k][p]);
     if (h->gate_fd >= 0) { flock(h->gate_fd, LOCK_UN); close(h->gate_fd); h->gate_fd = -1; }
     for (void* p : h->allocs) cudaFree(p);
-    for (int p = 0; p < 2; p++) {
-        if (h->hb[p].accum) cudaFree(h->hb[p].accum);
-        if (h->hb[p].keys) cudaFree(h->hb[p].keys);
-        if (h->hb[p].lines) cudaFree(h->hb[p].lines);
-        if (h->hb[p].tabSin) cudaFree(h->hb[p].tabSin);
-    }
-    if (h->frames_h) cudaFreeHost(h->frames_h);
-    if (h->res_h) cudaFreeHost(h->res_h);
-    if (h->rects_h) cudaFreeHost(h->rects_h);
-    if (h->rect_off_h) cudaFreeHost(h->rect_off_h);
-    if (h->ctl_h) cudaFreeHost(h->ctl_h);
-    if (h->base_d) cudaFree(h->base_d);
-    if (h->tab_samples_d) cudaFree(h->tab_samples_d);
-    if (h->inj_trails_h) cudaFreeHost(h->inj_trails_h);
-    if (h->inj_off_h) cudaFreeHost(h->inj_off_h);
-    if (h->inj_base_h) cudaFreeHost(h->inj_base_h);
+    for (int p = 0; p < 2; p++) hough_free(h->hb[p]);
+    hough_scratch_free(h->hs);
+    cudaFree(h->base_d); cudaFree(h->tab_samples_d);
+    for (void* p : {(void*)h->frames_h, (void*)h->res_h, (void*)h->rects_h, (void*)h->rect_off_h, (void*)h->ctl_h,
+                    (void*)h->inj_trails_h, (void*)h->inj_off_h, (void*)h->inj_base_h, (void*)h->counters_h})
+        cudaFreeHost(p);
     for (int i = 0; i < 2; i++) if (h->ev_inj[i]) cudaEventDestroy(h->ev_inj[i]);
-    if (h->counters_h) cudaFreeHost(h->counters_h);
     for (int i = 0; i <= N_TIMINGS; i++) if (h->ev_valid[i]) cudaEventDestroy(h->ev[i]);
     for (int k = 0; k < LFD_BATCH_PARTS; k++)
         for (int p = 0; p < 2; p++)
@@ -616,11 +633,17 @@ extern "C" int lfd_host_frames(lfd_handle* h, float** out)
 // ------------------------------------------------------------------------------------------------
 // parameters
 // ------------------------------------------------------------------------------------------------
+static int check_contours_args(lfd_handle* h, int mode, int method)
+{
+    if (mode < 0 || mode > 3) { h->err = "unknown contoursMode"; return LFD_E_ARG; }
+    if (method != 1 && method != 2) { h->err = "contoursMethod CHAIN_APPROX_TC89_* is not implemented"; return LFD_E_UNSUPPORTED; }
+    return LFD_OK;
+}
+
 static int check_pass_params(lfd_handle* h, const lfd_pass_params& p, bool dim)
 {
     if (p.nlinesInSet < 1 || p.nlinesInSet > LFD_MAX_SET_LINES) { h->err = "nlinesInSet must be in 1..16"; return LFD_E_UNSUPPORTED; }
-    if (p.contoursMode < 0 || p.contoursMode > 3) { h->err = "unknown contoursMode"; return LFD_E_ARG; }
-    if (p.contoursMethod != 1 && p.contoursMethod != 2) { h->err = "contoursMethod CHAIN_APPROX_TC89_* is not implemented"; return LFD_E_UNSUPPORTED; }
+    TRY(check_contours_args(h, p.contoursMode, p.contoursMethod));
     if (p.dilate_h < 1 || p.dilate_w < 1) { h->err = "dilateKernel missing"; return LFD_E_ARG; }
     int eh = dim ? p.erode_h : 0, ew = dim ? p.erode_w : 0;
     if ((eh > 0) != (ew > 0)) { h->err = "bad erodeKernel"; return LFD_E_ARG; }
@@ -638,15 +661,13 @@ extern "C" int lfd_set_params(lfd_handle* h, const lfd_params* p)
 {
     if (!h || !p) return LFD_E_ARG;
     cudaSetDevice(h->device);
-    int rc;
-    if ((rc = check_pass_params(h, p->bright, false)) != LFD_OK) return rc;
-    if ((rc = check_pass_params(h, p->dim, true)) != LFD_OK) return rc;
+    TRY(check_pass_params(h, p->bright, false));
+    TRY(check_pass_params(h, p->dim, true));
     CK(cudaStreamSynchronize(h->stream));
     for (int pass = 0; pass < 2; pass++) {
         const lfd_pass_params& pp = pass ? p->dim : p->bright;
         // theta = np.pi/180 and threshold = 1 are literals in the reference (processfield.py:370, :488)
-        rc = hough_setup(h, &h->hb[pass], h->d.H, h->d.W, pp.houghMethod, M_PI / 180, 1, h->B, false, h->cfg.max_lines);
-        if (rc != LFD_OK) return rc;
+        TRY(hough_setup(h, &h->hb[pass], h->d.H, h->d.W, pp.houghMethod, M_PI / 180, 1, h->B, false, h->cfg.max_lines));
     }
     h->params = *p;
     h->have_params = true;
@@ -681,9 +702,8 @@ extern "C" int lfd_set_kernels(lfd_handle* h, int pass, const uint8_t* erode_mas
     cudaSetDevice(h->device);
     if (!h->have_params) { h->err = "lfd_set_params has not been called"; return LFD_E_STATE; }
     CK(cudaStreamSynchronize(h->stream));
-    int rc;
-    if ((rc = fill_anykernel(h, &h->anyk_h[pass][0], pass == 1 ? erode_mask : nullptr, eh, ew, "erodeKernel")) != LFD_OK) return rc;
-    if ((rc = fill_anykernel(h, &h->anyk_h[pass][1], dilate_mask, dh, dw, "dilateKernel")) != LFD_OK) return rc;
+    TRY(fill_anykernel(h, &h->anyk_h[pass][0], pass == 1 ? erode_mask : nullptr, eh, ew, "erodeKernel"));
+    TRY(fill_anykernel(h, &h->anyk_h[pass][1], dilate_mask, dh, dw, "dilateKernel"));
     CK(cudaMemcpy(h->anyk_d + pass * 2, &h->anyk_h[pass][0], 2 * sizeof(AnyKernel), cudaMemcpyHostToDevice));
     h->anyk_on[pass] = true;
     if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
@@ -696,60 +716,151 @@ extern "C" int lfd_set_kernels(lfd_handle* h, int pass, const uint8_t* erode_mas
 // ------------------------------------------------------------------------------------------------
 // the pipeline
 // ------------------------------------------------------------------------------------------------
-// frames [f0, f0 + n) of the batch: every per-frame array is entered at frame f0, kernels index frames from 0
-// `part`: 0 = the whole pass ; 1 = only the contour part (NMS .. box fill) on a morph plane + nz mask the caller put in place
-static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, cudaStream_t s, bool stage_events, int part = 0)
+// frames [f0, f0 + n) of one pass, launched on stream s: every per-frame array is entered at frame f0, kernels index
+// frames from 0
+struct PassView {
+    lfd_handle* h;
+    int f0, n, pass, flags;
+    cudaStream_t s;
+    FrameCtl* C;                      // this pass's bookkeeping block
+    u8 *gray, *morph;
+    u32 *nz, *cand, *strong, *edges, *box;
+    CclBuf* ccl[2]; CompBuf* comp; RectBuf* rbuf;   // ccl: [kind]
+};
+
+static PassView pass_view(lfd_handle* h, int f0, int n, int pass, int flags, cudaStream_t s)
 {
-#define STAGE_EVENT(i) do { if (stage_events) CK(cudaEventRecord(h->ev[i], s)); } while (0)
-#define KB_MARK(id, e) do {                                                                          \
-        if (!(flags & LFD_KERNEL_TIMES)) break;                                                        \
-        cudaEvent_t& kev_ = h->kb[h->cur_part][pass][id][e];                                           \
-        /* under stream capture a plain record is a dependency marker, not a node: ask for an external record node */ \
-        CK(cudaEventRecordWithFlags(kev_, s, capturing ? cudaEventRecordExternal : cudaEventRecordDefault)); \
-        h->kb_used[h->cur_part][pass][id] = true;                                                      \
-    } while (0)
+    const size_t fN = (size_t)f0 * h->d.N, fNW = (size_t)f0 * h->d.NW;
+    return {h, f0, n, pass, flags, s, h->ctl + (size_t)pass * h->B + f0, h->gray[pass] + fN, h->morph[pass] + fN,
+            h->nz[pass] + fNW, h->cand[pass] + fNW, h->strong[pass] + fNW, h->edges[pass] + fNW, h->box[pass] + fNW,
+            {h->ccl_d[pass][0] + f0, h->ccl_d[pass][1] + f0}, h->comp_d[pass] + f0, h->rbuf_d[pass] + f0};
+}
+
+// One side (e = 0 begin, 1 end) of the bracket of kernel `id`, with LFD_KERNEL_TIMES only
+static int kb_mark(const PassView& V, int id, int e)
+{
+    lfd_handle* h = V.h;
+    if (!(V.flags & LFD_KERNEL_TIMES)) return LFD_OK;
+    cudaStreamCaptureStatus cst = cudaStreamCaptureStatusNone;
+    const bool capturing = cudaStreamIsCapturing(V.s, &cst) == cudaSuccess && cst == cudaStreamCaptureStatusActive;
+    // under stream capture a plain record is a dependency marker, not a node: ask for an external record node
+    CK(cudaEventRecordWithFlags(h->kb[h->cur_part][V.pass][id][e], V.s, capturing ? cudaEventRecordExternal : cudaEventRecordDefault));
+    h->kb_used[h->cur_part][V.pass][id] = true;
+    return LFD_OK;
+}
+
+// Sobel + NMS of the morphology plane into the candidate / strong edge masks; ntap: per-pixel class tap, or nullptr
+static int launch_nms(const PassView& V, int low, int high, u8* ntap)
+{
+    lfd_handle* h = V.h;
+    const Dims d = h->d; const int n = V.n;
+    if ((d.W % 8) == 0) {        // k_nms_march stores only non-zero mask words
+        CK(cudaMemsetAsync(V.cand, 0, (size_t)n * d.NW * sizeof(u32), V.s));
+        CK(cudaMemsetAsync(V.strong, 0, (size_t)n * d.NW * sizeof(u32), V.s));
+    }
+    TRY(kb_mark(V, KB_NMS, 0));
+    if ((d.W % 8) == 0) {
+        const int nstrips = ((d.W >> 2) + MARCH_UW - 1) / MARCH_UW, nchunks = (d.H + NMS_R - 1) / NMS_R;
+        const int nunits = nstrips * nchunks;
+        dim3 gg((nunits + NMS_WPC - 1) / NMS_WPC, n);
+        if (ntap) k_nms_march<true><<<gg, NMS_WPC * 32, 0, V.s>>>(V.morph, V.nz, V.cand, V.strong, ntap, V.C, V.pass, d, nstrips, nunits, low, high);
+        else k_nms_march<false><<<gg, NMS_WPC * 32, 0, V.s>>>(V.morph, V.nz, V.cand, V.strong, ntap, V.C, V.pass, d, nstrips, nunits, low, high);
+    } else {
+        dim3 cg((d.W + CANNY_TW - 1) / CANNY_TW, (d.H + CANNY_TH - 1) / CANNY_TH, n);
+        k_canny_nms<<<cg, 256, 0, V.s>>>(V.morph, V.nz, V.cand, V.strong, ntap, V.C, V.pass, d, low, high);
+    }
+    LAUNCH_CHECK();
+    return kb_mark(V, KB_NMS, 1);
+}
+
+// Run labelling.  kind 0: the candidate edges, a component kept (hysteresis) and written to the edge mask where it holds
+// a strong pixel (outer contours); kind 1: the background of the edge mask (holes).  k_ccl_extremes_flat is the caller's.
+static int launch_labels(const PassView& V, int kind)
+{
+    lfd_handle* h = V.h;
+    const Dims d = h->d; const int n = V.n;
+    const int nbands = (d.H + CCL_BAND - 1) / CCL_BAND;
+    const dim3 bands((n >= 16 && nbands > CCL_BAND_CTAS) ? CCL_BAND_CTAS : nbands, n), seams((nbands + CCL_WARPS - 1) / CCL_WARPS, n),
+        flat(CCL_FLAT_CTAS, n);
+    unsigned long long* const cnt = (unsigned long long*)h->counters_d;
+    CclBuf* const ccl = V.ccl[kind];
+    TRY(kb_mark(V, KB_CCL_BAND_FG + kind, 0));
+    k_ccl_band<<<bands, 256, ccl_band_smem(d.WW), V.s>>>(kind ? V.edges : V.cand, ccl, V.C, V.pass, d, kind, h->cfg.max_runs, cnt); LAUNCH_CHECK();
+    TRY(kb_mark(V, KB_CCL_BAND_FG + kind, 1));
+    k_ccl_merge<<<seams, CCL_WARPS * 32, 0, V.s>>>(ccl, V.C, V.pass, d, kind); LAUNCH_CHECK();
+    if (kind == 0) CK(cudaMemsetAsync(V.edges, 0, (size_t)n * d.NW * sizeof(u32), V.s));
+    k_ccl_stats_flat<<<flat, 256, 0, V.s>>>(kind ? nullptr : V.strong, ccl, V.C, V.pass, d, kind); LAUNCH_CHECK();
+    k_ccl_alloc_flat<<<flat, 256, 0, V.s>>>(ccl, kind ? nullptr : V.edges, V.comp, V.C, V.pass, d, kind); LAUNCH_CHECK();
+    return LFD_OK;
+}
+
+// fit_minAreaRect's arguments (processfield.py:201); external: cv2.RETR_EXTERNAL, outermost outer borders only
+struct ContourArgs { double minAreaRectMinLen, lwTresh; bool external; };
+
+// Rectangles of both contour kinds + box image.  The screen rejects the contours whose aspect bound proves they cannot
+// pass (most of them: the NMS rings around stars and their holes); only the survivors are fitted.  With `fit_all`
+// every contour is fitted and the screen only records its verdicts, so that the RECTS tap holds every rectangle.
+static int launch_contours(const PassView& V, const ContourArgs& a, bool fit_all)
+{
+    lfd_handle* h = V.h;
+    const Dims d = h->d; const int n = V.n;
+    unsigned long long* const cnt = (unsigned long long*)h->counters_d;
+    int* const tasks = fit_all ? nullptr : h->rtasks[V.pass] + (size_t)V.f0 * 2 * h->cfg.max_components;
+    TRY(kb_mark(V, KB_RECTS_SCREEN, 0));
+    k_rects_screen<<<h->sm_count * 2, SCREEN_THREADS, screen_smem(n), V.s>>>(V.comp, V.rbuf, V.ccl[0], V.ccl[1], V.C, V.pass, n, d, a.lwTresh, tasks, cnt); LAUNCH_CHECK();
+    TRY(kb_mark(V, KB_RECTS_SCREEN, 1));
+    TRY(kb_mark(V, KB_RECTS, 0));
+    k_rects_warp<<<h->sm_count * 16, RECT_WARPS * 32, rects_smem(n), V.s>>>(V.comp, V.rbuf, V.ccl[0], V.ccl[1], V.C, V.pass, n, d, a.minAreaRectMinLen, a.lwTresh, cnt, a.external ? 1 : 0, tasks); LAUNCH_CHECK();
+    TRY(kb_mark(V, KB_RECTS, 1));
+    CK(cudaMemsetAsync(V.box, 0, (size_t)n * d.NW * sizeof(u32), V.s));
+    k_fill_boxes<<<dim3(16, n), 128, 0, V.s>>>(V.rbuf, V.box, V.C, V.pass, d); LAUNCH_CHECK();
+    return LFD_OK;
+}
+
+// k_hough_vote of the segment lists of `nimg` images (of size d) into their accumulators
+static int launch_hough_vote(lfd_handle* h, const HoughBufs& hb, Dims d, const uint2* segs, int* accum, const FrameCtl* C,
+                             int pass, int nimg, cudaStream_t s)
+{
+    unsigned long long* const cnt = (unsigned long long*)h->counters_d;
+    if (hough_magic_ok(d.H, d.W, hb.hc.rho))
+        k_hough_vote<true><<<dim3(32, hb.hc.ngroups, nimg), HOUGH_THREADS, hb.smem, s>>>(segs, accum, hb.tabSin, hb.tabCos, C, pass, hb.hc, (size_t)d.NW, hb.accum_stride, cnt);
+    else
+        k_hough_vote<false><<<dim3(32, hb.hc.ngroups, nimg), HOUGH_THREADS, hb.smem, s>>>(segs, accum, hb.tabSin, hb.tabCos, C, pass, hb.hc, (size_t)d.NW, hb.accum_stride, cnt);
+    LAUNCH_CHECK();
+    return LFD_OK;
+}
+
+// the whole pass on frames [f0, f0 + n)
+static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, cudaStream_t s, bool stage_events)
+{
     const Dims d = h->d;
-    bool capturing = false;
-    { cudaStreamCaptureStatus cst = cudaStreamCaptureStatusNone; if (cudaStreamIsCapturing(s, &cst) == cudaSuccess) capturing = cst == cudaStreamCaptureStatusActive; }
     const lfd_pass_params& pp = pass ? h->params.dim : h->params.bright;
-    FrameCtl* const C = h->ctl + (size_t)pass * h->B + f0;      // this pass's bookkeeping block
-    const size_t fN = (size_t)f0 * d.N, fNW = (size_t)f0 * d.NW;
-    u8* const v_gray = h->gray[pass] + fN;
-    u8* const v_morph = h->morph[pass] + fN;
-    u32* const v_nz = h->nz[pass] + fNW;
-    u32* const v_cand = h->cand[pass] + fNW;
-    u32* const v_strong = h->strong[pass] + fNW;
-    u32* const v_edges = h->edges[pass] + fNW;
-    u32* const v_box = h->box[pass] + fNW;
-    CclBuf* const v_ccl0 = h->ccl_d[pass][0] + f0;
-    CclBuf* const v_ccl1 = h->ccl_d[pass][1] + f0;
-    CompBuf* const v_comp = h->comp_d[pass] + f0;
-    RectBuf* const v_rbuf = h->rbuf_d[pass] + f0;
+    const PassView V = pass_view(h, f0, n, pass, flags, s);
+    FrameCtl* const C = V.C;
+    const size_t fN = (size_t)f0 * d.N;
     uint2* const v_segs = h->segs[pass] + (size_t)f0 * 2 * d.NW;
     lfd_result* const v_res = h->res_d + f0;
     const bool taps = flags & LFD_KEEP_TAPS;
     const int tbase = 2 + pass * (T_PER_PASS - 1);   // event index preceding this pass's first stage
+    auto stage_event = [&](int i) -> int { if (stage_events) CK(cudaEventRecord(h->ev[tbase + i], s)); return LFD_OK; };
     HoughBufs& hb = h->hb[pass];
-    const int nbands = (d.H + CCL_BAND - 1) / CCL_BAND;
-    dim3 bands((n >= 16 && nbands > CCL_BAND_CTAS) ? CCL_BAND_CTAS : nbands, n), seams((nbands + CCL_WARPS - 1) / CCL_WARPS, n);
 
     // NMS tap (class per pixel) only with LFD_KEEP_TAPS
     u8* ntap = nullptr;
     if (taps) {
-        if (!h->nms_tap[pass]) { int rc = dev_alloc(h, &h->nms_tap[pass], (size_t)h->B * d.N); if (rc) return rc; }
+        if (!h->nms_tap[pass]) TRY(dev_alloc(h, &h->nms_tap[pass], (size_t)h->B * d.N));
         ntap = h->nms_tap[pass] + fN;
     }
-    if (part == 0) {
     // LUT + morphology
     k_lut<<<dim3(n, 1), 256, 0, s>>>(h->hist + (size_t)f0 * 256, h->lut + (size_t)f0 * 256, C, h->B, d.N, pass); LAUNCH_CHECK();
     MorphCfg mc;
     mc.eh = pass ? pp.erode_h : 0; mc.ew = pass ? pp.erode_w : 0; mc.dh = pp.dilate_h; mc.dw = pp.dilate_w;
     u8* etap = nullptr;
     if (taps && pass == 1 && mc.eh > 0) {
-        if (!h->eroded_tap) { int rc = dev_alloc(h, &h->eroded_tap, (size_t)h->B * d.N); if (rc) return rc; }
+        if (!h->eroded_tap) TRY(dev_alloc(h, &h->eroded_tap, (size_t)h->B * d.N));
         etap = h->eroded_tap + fN;
     }
-    KB_MARK(KB_MORPH, 0);
+    TRY(kb_mark(V, KB_MORPH, 0));
     {
         const u8* lutp = h->lut + ((size_t)pass * h->B + f0) * 256;
         const int nstrips = ((d.W >> 2) + MARCH_UW - 1) / MARCH_UW, nchunks = (d.H + MARCH_R - 1) / MARCH_R;
@@ -761,12 +872,12 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
             const AnyKernel* dkd = h->anyk_d + pass * 2 + 1;
             const int re = ekd ? h->anyk_h[pass][0].reach : 0, rd = h->anyk_h[pass][1].reach;
             dim3 ag((d.W + ANYK_TW - 1) / ANYK_TW, (d.H + ANYK_TH - 1) / ANYK_TH, n);
-            k_morph_any<<<ag, 256, anyk_smem(re, rd), s>>>(v_gray, lutp, v_morph, v_nz, etap, C, pass, d, ekd, dkd);
+            k_morph_any<<<ag, 256, anyk_smem(re, rd), s>>>(V.gray, lutp, V.morph, V.nz, etap, C, pass, d, ekd, dkd);
             done = true;
         }
 #define MORPH_CASE(EH_, EW_, DH_, DW_)                                                                              \
         if (!done && (d.W % 8) == 0 && mc.eh == EH_ && mc.ew == EW_ && mc.dh == DH_ && mc.dw == DW_) {                \
-            k_morph_march<EH_, EW_, DH_, DW_><<<gg, MARCH_WPC * 32, 0, s>>>(v_gray, lutp, v_morph, v_nz, etap, \
+            k_morph_march<EH_, EW_, DH_, DW_><<<gg, MARCH_WPC * 32, 0, s>>>(V.gray, lutp, V.morph, V.nz, etap, \
                                                                C, pass, d, nstrips, nunits);                    \
             done = true;                                                                                             \
         }
@@ -778,82 +889,30 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
 #undef MORPH_CASE
         if (!done) {                // any other all-ones rectangle: shared-memory tile kernel
             dim3 mg((d.W + MORPH_TW - 1) / MORPH_TW, (d.H + MORPH_TH - 1) / MORPH_TH, n);
-            k_morph<<<mg, 256, 0, s>>>(v_gray, lutp, v_morph, v_nz, etap, C, pass, d, mc);
+            k_morph<<<mg, 256, 0, s>>>(V.gray, lutp, V.morph, V.nz, etap, C, pass, d, mc);
         }
         LAUNCH_CHECK();
     }
-    KB_MARK(KB_MORPH, 1);
-    STAGE_EVENT(tbase + 1);
+    TRY(kb_mark(V, KB_MORPH, 1));
+    TRY(stage_event(1));
+    TRY(launch_nms(V, 0, 255, ntap));
+    TRY(stage_event(2));
+    for (int kind = 0; kind < 2; kind++) {
+        TRY(launch_labels(V, kind));
+        k_ccl_extremes_flat<<<dim3(CCL_FLAT_CTAS, n), 256, 0, s>>>(V.edges, V.ccl[kind], V.comp, C, pass, d, kind); LAUNCH_CHECK();
+        TRY(stage_event(3 + kind));
     }
-    // Sobel + NMS
-    if ((d.W % 8) == 0) {        // k_nms_march stores only non-zero mask words
-        CK(cudaMemsetAsync(v_cand, 0, (size_t)n * d.NW * sizeof(u32), s));
-        CK(cudaMemsetAsync(v_strong, 0, (size_t)n * d.NW * sizeof(u32), s));
-    }
-    KB_MARK(KB_NMS, 0);
-    if ((d.W % 8) == 0) {
-        const int nstrips = ((d.W >> 2) + MARCH_UW - 1) / MARCH_UW, nchunks = (d.H + NMS_R - 1) / NMS_R;
-        const int nunits = nstrips * nchunks;
-        dim3 gg((nunits + NMS_WPC - 1) / NMS_WPC, n);
-        if (ntap) k_nms_march<true><<<gg, NMS_WPC * 32, 0, s>>>(v_morph, v_nz, v_cand, v_strong, ntap, C, pass, d, nstrips, nunits, 0, 255);
-        else k_nms_march<false><<<gg, NMS_WPC * 32, 0, s>>>(v_morph, v_nz, v_cand, v_strong, ntap, C, pass, d, nstrips, nunits, 0, 255);
-    } else {
-        dim3 cg((d.W + CANNY_TW - 1) / CANNY_TW, (d.H + CANNY_TH - 1) / CANNY_TH, n);
-        k_canny_nms<<<cg, 256, 0, s>>>(v_morph, v_nz, v_cand, v_strong, ntap, C, pass, d, 0, 255);
-    }
-    LAUNCH_CHECK();
-    KB_MARK(KB_NMS, 1);
-    STAGE_EVENT(tbase + 2);
-    // foreground runs: hysteresis + outer contours
-    unsigned long long* const cnt = (unsigned long long*)h->counters_d;
-    KB_MARK(KB_CCL_BAND_FG, 0);
-    k_ccl_band<<<bands, 256, ccl_band_smem(d.WW), s>>>(v_cand, v_ccl0, C, pass, d, 0, h->cfg.max_runs, cnt); LAUNCH_CHECK();
-    KB_MARK(KB_CCL_BAND_FG, 1);
-    k_ccl_merge<<<seams, CCL_WARPS * 32, 0, s>>>(v_ccl0, C, pass, d, 0); LAUNCH_CHECK();
-    const dim3 flat(CCL_FLAT_CTAS, n);
-    CK(cudaMemsetAsync(v_edges, 0, (size_t)n * d.NW * sizeof(u32), s));
-    k_ccl_stats_flat<<<flat, 256, 0, s>>>(v_strong, v_ccl0, C, pass, d, 0); LAUNCH_CHECK();
-    k_ccl_alloc_flat<<<flat, 256, 0, s>>>(v_ccl0, v_edges, v_comp, C, pass, d, 0); LAUNCH_CHECK();
-    k_ccl_extremes_flat<<<flat, 256, 0, s>>>(v_edges, v_ccl0, v_comp, C, pass, d, 0); LAUNCH_CHECK();
-    STAGE_EVENT(tbase + 3);
-    // background runs: hole contours
-    KB_MARK(KB_CCL_BAND_BG, 0);
-    k_ccl_band<<<bands, 256, ccl_band_smem(d.WW), s>>>(v_edges, v_ccl1, C, pass, d, 1, h->cfg.max_runs, cnt); LAUNCH_CHECK();
-    KB_MARK(KB_CCL_BAND_BG, 1);
-    k_ccl_merge<<<seams, CCL_WARPS * 32, 0, s>>>(v_ccl1, C, pass, d, 1); LAUNCH_CHECK();
-    k_ccl_stats_flat<<<flat, 256, 0, s>>>(nullptr, v_ccl1, C, pass, d, 1); LAUNCH_CHECK();
-    k_ccl_alloc_flat<<<flat, 256, 0, s>>>(v_ccl1, nullptr, v_comp, C, pass, d, 1); LAUNCH_CHECK();
-    k_ccl_extremes_flat<<<flat, 256, 0, s>>>(v_edges, v_ccl1, v_comp, C, pass, d, 1); LAUNCH_CHECK();
-    STAGE_EVENT(tbase + 4);
-    // rectangles + box image.  The screen rejects the contours whose aspect bound proves they cannot pass (most of them:
-    // the NMS rings around stars and their holes); only the survivors are fitted.  With taps, and in the standalone fit
-    // (part 1), whose RECTS tap is its output, every contour is fitted and the screen only records its verdicts.
-    int* const v_tasks = (!taps && part == 0) ? h->rtasks[pass] + (size_t)f0 * 2 * h->cfg.max_components : nullptr;
-    KB_MARK(KB_RECTS_SCREEN, 0);
-    k_rects_screen<<<h->sm_count * 2, SCREEN_THREADS, screen_smem(n), s>>>(v_comp, v_rbuf, v_ccl0, v_ccl1, C, pass, n, d, pp.lwTresh, v_tasks, cnt); LAUNCH_CHECK();
-    KB_MARK(KB_RECTS_SCREEN, 1);
-    KB_MARK(KB_RECTS, 0);
-    k_rects_warp<<<h->sm_count * 16, RECT_WARPS * 32, rects_smem(n), s>>>(v_comp, v_rbuf, v_ccl0, v_ccl1, C, pass, n, d, pp.minAreaRectMinLen, pp.lwTresh, cnt, pp.contoursMode == 0 ? 1 : 0, v_tasks); LAUNCH_CHECK();
-    KB_MARK(KB_RECTS, 1);
-    CK(cudaMemsetAsync(v_box, 0, (size_t)n * d.NW * sizeof(u32), s));
-    k_fill_boxes<<<dim3(16, n), 128, 0, s>>>(v_rbuf, v_box, C, pass, d); LAUNCH_CHECK();
-    STAGE_EVENT(tbase + 5);
-    if (part == 1) return LFD_OK;
+    TRY(launch_contours(V, {pp.minAreaRectMinLen, pp.lwTresh, pp.contoursMode == 0}, taps));
+    TRY(stage_event(5));
     // Hough on the morphology output and on the box image
     int* const v_accum = hb.accum + (size_t)f0 * 2 * hb.accum_stride;
     u64* const v_keys = hb.keys + (size_t)f0 * 2 * hb.key_stride;
     CK(cudaMemsetAsync(v_accum, 0, (size_t)n * 2 * hb.accum_stride * sizeof(int), s));
     // a thread's iterations are a serial chain (load -> ballot -> slot atomic -> store): many CTAs, few iterations each
-    k_hough_compact<<<dim3(128, n, 2), 256, 0, s>>>(v_nz, v_box, v_segs, C, pass, d, (size_t)d.NW); LAUNCH_CHECK();
-    KB_MARK(KB_HOUGH_VOTE, 0);
-    if (hough_magic_ok(d.H, d.W, hb.hc.rho))
-        k_hough_vote<true><<<dim3(32, hb.hc.ngroups, 2 * n), HOUGH_THREADS, hb.smem, s>>>(v_segs, v_accum, hb.tabSin, hb.tabCos, C, pass,
-                                                                                  hb.hc, (size_t)d.NW, hb.accum_stride, (unsigned long long*)h->counters_d);
-    else
-        k_hough_vote<false><<<dim3(32, hb.hc.ngroups, 2 * n), HOUGH_THREADS, hb.smem, s>>>(v_segs, v_accum, hb.tabSin, hb.tabCos, C, pass,
-                                                                                   hb.hc, (size_t)d.NW, hb.accum_stride, (unsigned long long*)h->counters_d);
-    LAUNCH_CHECK();
-    KB_MARK(KB_HOUGH_VOTE, 1);
+    k_hough_compact<<<dim3(128, n, 2), 256, 0, s>>>(V.nz, V.box, v_segs, C, pass, d, (size_t)d.NW); LAUNCH_CHECK();
+    TRY(kb_mark(V, KB_HOUGH_VOTE, 0));
+    TRY(launch_hough_vote(h, hb, d, v_segs, v_accum, C, pass, 2 * n, s));
+    TRY(kb_mark(V, KB_HOUGH_VOTE, 1));
     int cells = hb.hc.numangle * hb.hc.numrho;
     int pblocks = (cells + 255) / 256; if (pblocks > 64) pblocks = 64;
     k_hough_peaks<<<dim3(pblocks, 2 * n), 256, 0, s>>>(v_accum, v_keys, C, pass, hb.hc, hb.accum_stride, hb.key_stride); LAUNCH_CHECK();
@@ -862,13 +921,10 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
         if (!hb.lines) CK(cudaMalloc((void**)&hb.lines, (size_t)h->B * 2 * hb.line_stride * sizeof(float)));
         k_hough_sort<<<dim3(2, n), 1024, 0, s>>>(v_keys, hb.lines + (size_t)f0 * 2 * hb.line_stride, C, pass, hb.hc, hb.key_stride, hb.line_stride, hb.max_lines); LAUNCH_CHECK();
     }
-    STAGE_EVENT(tbase + 6);
+    TRY(stage_event(6));
     k_check_theta<<<(n + 63) / 64, 64, 0, s>>>(v_res, C, pass, n, pp.nlinesInSet, pp.dro, pp.thetaTresh, pp.lineSetTresh,
                                               hb.hc.numangle, (unsigned long long*)h->counters_d); LAUNCH_CHECK();
-    STAGE_EVENT(tbase + 7);
-    return LFD_OK;
-#undef STAGE_EVENT
-#undef KB_MARK
+    return stage_event(7);
 }
 
 // mode 0: whole-frame pipeline on h->in (un-flipped) ; mode 1/2: standalone bright/dim on frame slot 0
@@ -893,7 +949,7 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
     }
     float* clipped = nullptr;
     if (want_clipped) {
-        if (!h->clipped) { int rc = dev_alloc(h, &h->clipped, (size_t)d.N); if (rc) return rc; }
+        if (!h->clipped) TRY(dev_alloc(h, &h->clipped, (size_t)d.N));
         clipped = h->clipped;
     }
     const lfd_pass_params& pd = h->params.dim;
@@ -922,7 +978,6 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
         LAUNCH_CHECK();
     }
     CK(cudaEventRecord(h->ev[2], s));
-    int rc;
     // The bright and the dim pass of a batch are independent until the verdict (the reference runs dim only
     // when bright finds nothing, detecttrails.py:125-129; here dim runs for every frame on a second stream and
     // k_finalize drops it where bright detected).  Most kernels after the morphology are latency-bound, so the
@@ -935,7 +990,6 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
     // independent chains (bright / dim x part) keep the SMs busy through the latency-bound CCL / geometry phases
     const int nsplit = (overlap && n >= 16) ? LFD_BATCH_PARTS : 1;
     auto passes = [&](bool stage_events) -> int {
-        int rc2;
         if (overlap) {
             CK(cudaEventRecord(h->ev_fork, s));
             for (int k = 0; k < nsplit; k++)
@@ -948,9 +1002,9 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
             cudaStream_t sb = overlap ? h->xs[k][0] : s, sd = overlap ? h->xs[k][1] : s;
             const bool ev = stage_events && k == 0;
             h->cur_part = k;
-            if (mode != 2) { if ((rc2 = run_pass_kernels(h, fstart, cnt, 0, flags, sb, ev)) != LFD_OK) return rc2; }
+            if (mode != 2) TRY(run_pass_kernels(h, fstart, cnt, 0, flags, sb, ev));
             else if (k == 0) for (int i = 3; i <= T_PER_PASS + 1; i++) CK(cudaEventRecord(h->ev[i], s));
-            if (mode != 1) { if ((rc2 = run_pass_kernels(h, fstart, cnt, 1, flags, sd, ev)) != LFD_OK) return rc2; }
+            if (mode != 1) TRY(run_pass_kernels(h, fstart, cnt, 1, flags, sd, ev));
             else if (k == 0) for (int i = T_PER_PASS + 2; i < N_TIMINGS; i++) CK(cudaEventRecord(h->ev[i], s));
             fstart += cnt;
         }
@@ -970,7 +1024,7 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
             if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
             const int64_t l0 = h->launches;
             CK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-            rc = passes(false);
+            const int rc = passes(false);
             cudaGraph_t g = nullptr;
             cudaError_t ce = cudaStreamEndCapture(s, &g);
             if (rc != LFD_OK) { if (g) cudaGraphDestroy(g); cudaGetLastError(); return rc; }
@@ -985,7 +1039,7 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
         CK(cudaGraphLaunch(h->graph_exec, s));
         h->launches += h->graph_launches;
     } else {
-        if ((rc = passes(true)) != LFD_OK) return rc;
+        TRY(passes(true));
     }
     CK(cudaEventRecord(h->ev[N_TIMINGS], s));
     h->last_n = n; h->last_flags = flags; h->pending = true;
@@ -995,16 +1049,23 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
 
 static void CUDART_CB gate_release_cb(void* p) { flock((int)(intptr_t)p, LOCK_UN); }
 
+// star-rectangle offsets of n frames: rect_offsets[0] == 0 and at most max_star_rects per frame
+static int check_rect_offsets(lfd_handle* h, int n, const int32_t* rect_offsets)
+{
+    if (rect_offsets[0] != 0) { h->err = "rect_offsets[0] must be 0"; return LFD_E_ARG; }
+    for (int f = 0; f < n; f++) {
+        int c = rect_offsets[f + 1] - rect_offsets[f];
+        if (c < 0 || c > h->cfg.max_star_rects) { h->err = "too many star rectangles for a frame (lfd_config.max_star_rects)"; return LFD_E_CAPACITY; }
+    }
+    return LFD_OK;
+}
+
 static int stage_rects(lfd_handle* h, int n, const int32_t* rects, const int32_t* rect_offsets)
 {
     if (!rects || !rect_offsets) {
         for (int f = 0; f <= n; f++) h->rect_off_h[f] = 0;
     } else {
-        if (rect_offsets[0] != 0) { h->err = "rect_offsets[0] must be 0"; return LFD_E_ARG; }
-        for (int f = 0; f < n; f++) {
-            int c = rect_offsets[f + 1] - rect_offsets[f];
-            if (c < 0 || c > h->cfg.max_star_rects) { h->err = "too many star rectangles for a frame (lfd_config.max_star_rects)"; return LFD_E_CAPACITY; }
-        }
+        TRY(check_rect_offsets(h, n, rect_offsets));
         memcpy(h->rect_off_h, rect_offsets, ((size_t)n + 1) * sizeof(int));
         memcpy(h->rects_h, rects, (size_t)rect_offsets[n] * sizeof(int4));
         CK(cudaMemcpyAsync(h->rects_d, h->rects_h, (size_t)rect_offsets[n] * sizeof(int4), cudaMemcpyHostToDevice, h->stream));
@@ -1016,10 +1077,8 @@ static int stage_rects(lfd_handle* h, int n, const int32_t* rects, const int32_t
 extern "C" int lfd_upload(lfd_handle* h, const float* frames, int n, const int32_t* rects, const int32_t* rect_offsets, int flags)
 {
     if (!h || n < 1 || n > h->B) { if (h) h->err = "bad batch size"; return LFD_E_ARG; }
-    cudaSetDevice(h->device);
-    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
-    int rc = stage_rects(h, n, rects, rect_offsets);
-    if (rc != LFD_OK) return rc;
+    TRY(enter(h));
+    TRY(stage_rects(h, n, rects, rect_offsets));
     const float* src = frames ? frames : h->frames_h;
     // Copy gate: wait (bounded) for this rank's slot of its host bridge, copy, and let a host callback on the stream free
     // the slot when the copy has completed.  With four GPUs behind one ~117 GB/s bridge the four concurrent 781 MB copies
@@ -1063,16 +1122,14 @@ extern "C" int lfd_set_h2d_gate(lfd_handle* h, const char* lock_path)
 
 extern "C" int lfd_submit(lfd_handle* h, const float* frames, int n, const int32_t* rects, const int32_t* rect_offsets, int flags)
 {
-    int rc = lfd_upload(h, frames, n, rects, rect_offsets, flags);
-    if (rc != LFD_OK) return rc;
+    TRY(lfd_upload(h, frames, n, rects, rect_offsets, flags));
     return run_pipeline(h, n, flags, 0, false);
 }
 
 extern "C" int lfd_run_resident(lfd_handle* h, int n, int flags)
 {
     if (!h || n < 1 || n > h->B) { if (h) h->err = "bad batch size"; return LFD_E_ARG; }
-    cudaSetDevice(h->device);
-    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    TRY(enter(h));
     return run_pipeline(h, n, flags, 0, false);
 }
 
@@ -1083,15 +1140,8 @@ extern "C" int lfd_set_base(lfd_handle* h, const float* frames, int n_base, cons
 {
     if (!h) return LFD_E_ARG;
     if (!frames || n_base < 1) { h->err = "lfd_set_base: frames must be non-NULL and n_base >= 1"; return LFD_E_ARG; }
-    cudaSetDevice(h->device);
-    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
-    if (rects && rect_offsets) {
-        if (rect_offsets[0] != 0) { h->err = "rect_offsets[0] must be 0"; return LFD_E_ARG; }
-        for (int f = 0; f < n_base; f++) {
-            int c = rect_offsets[f + 1] - rect_offsets[f];
-            if (c < 0 || c > h->cfg.max_star_rects) { h->err = "too many star rectangles for a frame (lfd_config.max_star_rects)"; return LFD_E_CAPACITY; }
-        }
-    }
+    TRY(enter(h));
+    if (rects && rect_offsets) TRY(check_rect_offsets(h, n_base, rect_offsets));
     const size_t N = h->d.N;
     if (n_base > h->base_cap) {
         if (h->base_d) { cudaFree(h->base_d); h->base_d = nullptr; }
@@ -1100,10 +1150,9 @@ extern "C" int lfd_set_base(lfd_handle* h, const float* frames, int n_base, cons
         h->base_cap = n_base;
     }
     if (!h->inj_trails_d) {
-        int rc;
-        if ((rc = dev_alloc(h, &h->inj_trails_d, (size_t)h->B * LFD_MAX_INJECT_TRAILS)) != LFD_OK) return rc;
-        if ((rc = dev_alloc(h, &h->inj_off_d, (size_t)h->B + 1)) != LFD_OK) return rc;
-        if ((rc = dev_alloc(h, &h->inj_base_d, (size_t)h->B)) != LFD_OK) return rc;
+        TRY(dev_alloc(h, &h->inj_trails_d, (size_t)h->B * LFD_MAX_INJECT_TRAILS));
+        TRY(dev_alloc(h, &h->inj_off_d, (size_t)h->B + 1));
+        TRY(dev_alloc(h, &h->inj_base_d, (size_t)h->B));
         CK(cudaMallocHost((void**)&h->inj_trails_h, (size_t)h->B * LFD_MAX_INJECT_TRAILS * sizeof(InjTrail)));
         CK(cudaMallocHost((void**)&h->inj_off_h, ((size_t)h->B + 1) * sizeof(int)));
         CK(cudaMallocHost((void**)&h->inj_base_h, (size_t)h->B * sizeof(int)));
@@ -1125,8 +1174,7 @@ extern "C" int lfd_set_base(lfd_handle* h, const float* frames, int n_base, cons
 extern "C" int lfd_set_trail_tables(lfd_handle* h, const float* samples, int n_samples, const lfd_table* tables, int n_tables)
 {
     if (!h) return LFD_E_ARG;
-    cudaSetDevice(h->device);
-    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    TRY(enter(h));
     if (!samples || !tables || n_samples < 2 || n_tables < 1 || n_tables > LFD_MAX_TRAIL_TABLES) {
         h->err = "lfd_set_trail_tables: samples and tables must be non-NULL, n_samples >= 2, n_tables in 1..LFD_MAX_TRAIL_TABLES";
         return LFD_E_ARG;
@@ -1166,8 +1214,7 @@ extern "C" int lfd_submit_injected_shaped(lfd_handle* h, int n, const int32_t* b
                                           const lfd_trail_shape* shapes, const int32_t* trail_offsets, int flags)
 {
     if (!h) return LFD_E_ARG;
-    cudaSetDevice(h->device);
-    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    TRY(enter(h));
     if (h->n_base < 1) { h->err = "no base frames (call lfd_set_base)"; return LFD_E_STATE; }
     if (n < 1 || n > h->B || !base_index) { h->err = "bad batch size or base_index"; return LFD_E_ARG; }
     if (flags & LFD_INPUT_BIGENDIAN) { h->err = "injected frames are built in native byte order (LFD_INPUT_BIGENDIAN)"; return LFD_E_ARG; }
@@ -1243,8 +1290,7 @@ extern "C" int lfd_submit_injected_shaped(lfd_handle* h, int n, const int32_t* b
     k_inject<<<dim3((h->d.H + INJ_ROWS - 1) / INJ_ROWS, n), INJ_THREADS, 0, h->stream>>>(h->base_d, h->inj_base_d, h->inj_trails_d,
                                                                                        h->inj_off_d, h->tab_samples_d, h->in, h->d); LAUNCH_CHECK();
     CK(cudaEventRecord(h->ev_inj[1], h->stream));
-    int rc = run_pipeline(h, n, flags, 0, false);
-    if (rc != LFD_OK) return rc;
+    TRY(run_pipeline(h, n, flags, 0, false));
     h->inj_recorded = true;
     return LFD_OK;
 }
@@ -1303,13 +1349,11 @@ extern "C" int lfd_get_kernel_times(lfd_handle* h, int index, const char** name,
 extern "C" int lfd_run_pass(lfd_handle* h, int pass, float* img, int flags, int writeback, lfd_result* out)
 {
     if (!h || !img || (pass != 0 && pass != 1)) { if (h) h->err = "bad argument"; return LFD_E_ARG; }
-    cudaSetDevice(h->device);
-    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    TRY(enter(h));
     if (flags & LFD_INPUT_BIGENDIAN) { h->err = "lfd_run_pass reads and writes back native float32 (LFD_INPUT_BIGENDIAN)"; return LFD_E_ARG; }
     h->rect_off_h[0] = h->rect_off_h[1] = 0;
     CK(cudaMemcpyAsync(h->in, img, (size_t)h->d.N * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-    int rc = run_pipeline(h, 1, flags, pass == 0 ? 1 : 2, writeback != 0);
-    if (rc != LFD_OK) return rc;
+    TRY(run_pipeline(h, 1, flags, pass == 0 ? 1 : 2, writeback != 0));
     if (writeback) CK(cudaMemcpyAsync(img, h->clipped, (size_t)h->d.N * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     return lfd_wait(h, out);
 }
@@ -1329,8 +1373,7 @@ __global__ void k_blot(float* img, const int4* rects, int nrects, Dims d)
 extern "C" int lfd_blot(lfd_handle* h, float* img, const int32_t* rects, int nrects)
 {
     if (!h || !img || nrects < 0 || (nrects > 0 && !rects)) { if (h) h->err = "bad argument"; return LFD_E_ARG; }
-    cudaSetDevice(h->device);
-    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    TRY(enter(h));
     if (nrects > h->B * h->cfg.max_star_rects) { h->err = "too many rectangles"; return LFD_E_CAPACITY; }
     if (nrects == 0) return LFD_OK;
     memcpy(h->rects_h, rects, (size_t)nrects * sizeof(int4));
@@ -1346,6 +1389,13 @@ extern "C" int lfd_blot(lfd_handle* h, float* img, const int32_t* rects, int nre
 // ------------------------------------------------------------------------------------------------
 // taps
 // ------------------------------------------------------------------------------------------------
+// entries of the RECTS / RECT_SCREEN taps: x outer contours then y holes, each kind's list at its own offset
+static int2 rect_tap_counts(const lfd_handle* h, int frame, int pass)
+{
+    const FrameCtl& ch = h->ctl_h[(size_t)pass * h->B + frame];
+    return make_int2(min(ch.ncomp_saved[pass][0], h->cfg.max_components), min(ch.ncomp_saved[pass][1], h->cfg.max_components));
+}
+
 extern "C" int lfd_get_stage_count(lfd_handle* h, int frame, int pass, int stage, int* count)
 {
     if (!h || !count || frame < 0 || frame >= h->last_n || (pass != 0 && pass != 1)) { if (h) h->err = "bad argument"; return LFD_E_ARG; }
@@ -1354,8 +1404,8 @@ extern "C" int lfd_get_stage_count(lfd_handle* h, int frame, int pass, int stage
     switch (stage) {
     case LFD_STAGE_RECTS:
     case LFD_STAGE_RECT_SCREEN: {
-        const FrameCtl& ch = h->ctl_h[(size_t)pass * h->B + frame];
-        *count = min(ch.ncomp_saved[pass][0], h->cfg.max_components) + min(ch.ncomp_saved[pass][1], h->cfg.max_components);
+        const int2 nc = rect_tap_counts(h, frame, pass);
+        *count = nc.x + nc.y;
         return LFD_OK;
     }
     // the lines the tap holds: k_hough_sort keeps at most max_lines of them (n_lines in lfd_result is the full count)
@@ -1375,28 +1425,25 @@ extern "C" int lfd_get_stage(lfd_handle* h, int frame, int pass, int stage, void
     const Dims d = h->d;
     cudaStream_t s = h->stream;
     const size_t N = d.N;
-    Dims d1 = d;
     const void* src = nullptr;
     size_t need = N;
     HoughBufs& hb = h->hb[pass];
     switch (stage) {
     case LFD_STAGE_MASK:
-        k_expand_mask<<<dim3(256, 1), 256, 0, s>>>(h->starmask + (size_t)frame * d.NW, h->tap_u8, d1); LAUNCH_CHECK();
+    case LFD_STAGE_CANNY:
+    case LFD_STAGE_BOX: {
+        const u32* m = stage == LFD_STAGE_MASK ? h->starmask : stage == LFD_STAGE_CANNY ? h->edges[pass] : h->box[pass];
+        k_expand_mask<<<dim3(256, 1), 256, 0, s>>>(m + (size_t)frame * d.NW, h->tap_u8, d); LAUNCH_CHECK();
         src = h->tap_u8; break;
+    }
     case LFD_STAGE_GRAY: src = h->gray[pass] + (size_t)frame * N; break;
     case LFD_STAGE_EQU:
-        k_apply_lut<<<dim3(256, 1), 256, 0, s>>>(h->gray[pass] + (size_t)frame * N, h->lut + ((size_t)pass * h->B + frame) * 256, h->tap_u8, d1); LAUNCH_CHECK();
+        k_apply_lut<<<dim3(256, 1), 256, 0, s>>>(h->gray[pass] + (size_t)frame * N, h->lut + ((size_t)pass * h->B + frame) * 256, h->tap_u8, d); LAUNCH_CHECK();
         src = h->tap_u8; break;
     case LFD_STAGE_ERODED:
         if (!h->eroded_tap || pass != 1) { h->err = "eroded tap not recorded (dim pass with LFD_KEEP_TAPS)"; return LFD_E_STATE; }
         src = h->eroded_tap + (size_t)frame * N; break;
     case LFD_STAGE_MORPH: src = h->morph[pass] + (size_t)frame * N; break;
-    case LFD_STAGE_CANNY:
-        k_expand_mask<<<dim3(256, 1), 256, 0, s>>>(h->edges[pass] + (size_t)frame * d.NW, h->tap_u8, d1); LAUNCH_CHECK();
-        src = h->tap_u8; break;
-    case LFD_STAGE_BOX:
-        k_expand_mask<<<dim3(256, 1), 256, 0, s>>>(h->box[pass] + (size_t)frame * d.NW, h->tap_u8, d1); LAUNCH_CHECK();
-        src = h->tap_u8; break;
     case LFD_STAGE_HIST: src = h->hist + ((size_t)pass * h->B + frame) * 256; need = 256 * sizeof(u32); break;
     case LFD_STAGE_LUT: src = h->lut + ((size_t)pass * h->B + frame) * 256; need = 256; break;
     case LFD_STAGE_NMS:
@@ -1404,30 +1451,23 @@ extern "C" int lfd_get_stage(lfd_handle* h, int frame, int pass, int stage, void
         src = h->nms_tap[pass] + (size_t)frame * N; break;
     case LFD_STAGE_FG_LABELS:
     case LFD_STAGE_BG_LABELS: {
-        if (!h->labels_tap) { int rc = dev_alloc(h, &h->labels_tap, N); if (rc) return rc; }
+        if (!h->labels_tap) TRY(dev_alloc(h, &h->labels_tap, N));
         int kind = stage == LFD_STAGE_BG_LABELS;
         k_ccl_labels<<<(d.H + CCL_WARPS - 1) / CCL_WARPS, CCL_WARPS * 32, 0, s>>>(h->ccl_d[pass][kind], h->labels_tap, h->ctl + (size_t)pass * h->B, pass, d, kind, frame); LAUNCH_CHECK();
         src = h->labels_tap; need = N * sizeof(int); break;
     }
-    case LFD_STAGE_RECTS: {
-        const FrameCtl& ch = h->ctl_h[(size_t)pass * h->B + frame];
-        int n0 = min(ch.ncomp_saved[pass][0], h->cfg.max_components), n1 = min(ch.ncomp_saved[pass][1], h->cfg.max_components);
-        need = (size_t)(n0 + n1) * sizeof(lfd_rect);
-        if (bytes < need) { h->err = "buffer too small"; return LFD_E_ARG; }
-        const RectBuf& rb = h->rbuf_h[pass][frame];
-        if (n0) CK(cudaMemcpyAsync(host_out, rb.rects, (size_t)n0 * sizeof(lfd_rect), cudaMemcpyDeviceToHost, s));
-        if (n1) CK(cudaMemcpyAsync((char*)host_out + (size_t)n0 * sizeof(lfd_rect), rb.rects + h->cfg.max_components, (size_t)n1 * sizeof(lfd_rect), cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        return LFD_OK;
-    }
+    case LFD_STAGE_RECTS:
     case LFD_STAGE_RECT_SCREEN: {
-        const FrameCtl& ch = h->ctl_h[(size_t)pass * h->B + frame];
-        int n0 = min(ch.ncomp_saved[pass][0], h->cfg.max_components), n1 = min(ch.ncomp_saved[pass][1], h->cfg.max_components);
-        need = (size_t)(n0 + n1) * sizeof(int);
-        if (bytes < need) { h->err = "buffer too small"; return LFD_E_ARG; }
+        const int2 nc = rect_tap_counts(h, frame, pass);
+        const int n0 = nc.x, n1 = nc.y;
         const RectBuf& rb = h->rbuf_h[pass][frame];
-        if (n0) CK(cudaMemcpyAsync(host_out, rb.screened, (size_t)n0 * sizeof(int), cudaMemcpyDeviceToHost, s));
-        if (n1) CK(cudaMemcpyAsync((char*)host_out + (size_t)n0 * sizeof(int), rb.screened + h->cfg.max_components, (size_t)n1 * sizeof(int), cudaMemcpyDeviceToHost, s));
+        const bool rects = stage == LFD_STAGE_RECTS;
+        const size_t esz = rects ? sizeof(lfd_rect) : sizeof(int);
+        const char* list = rects ? (const char*)rb.rects : (const char*)rb.screened;
+        need = (size_t)(n0 + n1) * esz;
+        if (bytes < need) { h->err = "buffer too small"; return LFD_E_ARG; }
+        if (n0) CK(cudaMemcpyAsync(host_out, list, (size_t)n0 * esz, cudaMemcpyDeviceToHost, s));
+        if (n1) CK(cudaMemcpyAsync((char*)host_out + (size_t)n0 * esz, list + (size_t)h->cfg.max_components * esz, (size_t)n1 * esz, cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
         return LFD_OK;
     }
@@ -1468,13 +1508,6 @@ extern "C" int lfd_get_stage(lfd_handle* h, int frame, int pass, int stage, void
 // ------------------------------------------------------------------------------------------------
 // standalone cv2.HoughLines
 // ------------------------------------------------------------------------------------------------
-struct HoughScratch {
-    int H = 0, W = 0;
-    u8* img = nullptr; u32* mask = nullptr; uint2* segs = nullptr; FrameCtl* ctl = nullptr; lfd_result* res = nullptr;
-    HoughBufs hb;
-};
-static HoughScratch g_hs;   // one per process is enough for the microbenchmark entry point
-
 extern "C" int lfd_hough_dims(int height, int width, double rho, double theta, int* numangle, int* numrho)
 {
     if (!numangle || !numrho || !(rho > 0) || !(theta > 0)) return LFD_E_ARG;
@@ -1486,14 +1519,12 @@ extern "C" int lfd_hough_lines(lfd_handle* h, const uint8_t* img, int height, in
                                int threshold, float* lines, int max_lines, int* n_lines, int32_t* accum)
 {
     if (!h || !img || height < 1 || width < 1 || height > 65535 || width > 65535 * 32) { if (h) h->err = "bad argument"; return LFD_E_ARG; }
-    cudaSetDevice(h->device);
-    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    TRY(enter(h));
     cudaStream_t s = h->stream;
     Dims d; d.H = height; d.W = width; d.WW = (width + 31) / 32; d.N = height * width; d.NW = height * d.WW;
-    HoughScratch& hs = g_hs;
+    HoughScratch& hs = h->hs;
     if (hs.H != height || hs.W != width) {
-        if (hs.img) { cudaFree(hs.img); cudaFree(hs.mask); cudaFree(hs.segs); cudaFree(hs.ctl); cudaFree(hs.res); }
-        hs.img = nullptr;
+        hough_scratch_free(hs);
         CK(cudaMalloc((void**)&hs.img, (size_t)d.N));
         CK(cudaMalloc((void**)&hs.mask, (size_t)d.NW * sizeof(u32)));
         CK(cudaMalloc((void**)&hs.segs, (size_t)2 * d.NW * sizeof(uint2)));
@@ -1501,8 +1532,7 @@ extern "C" int lfd_hough_lines(lfd_handle* h, const uint8_t* img, int height, in
         CK(cudaMalloc((void**)&hs.res, sizeof(lfd_result)));
         hs.H = height; hs.W = width;
     }
-    int rc = hough_setup(h, &hs.hb, height, width, rho, theta, threshold, 1, true, 0);
-    if (rc != LFD_OK) return rc;
+    TRY(hough_setup(h, &hs.hb, height, width, rho, theta, threshold, 1, true, 0));
     HoughBufs& hb = hs.hb;
     CK(cudaMemcpyAsync(hs.img, img, (size_t)d.N, cudaMemcpyHostToDevice, s));
     CK(cudaMemsetAsync(h->counters_d, 0, 16 * sizeof(int64_t), s));
@@ -1517,13 +1547,7 @@ extern "C" int lfd_hough_lines(lfd_handle* h, const uint8_t* img, int height, in
     // which = 0 only: pass the same mask twice and ignore slot 1
     k_hough_compact<<<dim3(64, 1, 1), 256, 0, s>>>(hs.mask, hs.mask, hs.segs, hs.ctl, 0, d, (size_t)d.NW); LAUNCH_CHECK();
     CK(cudaEventRecord(h->ev[1], s));
-    if (hough_magic_ok(height, width, hb.hc.rho))
-        k_hough_vote<true><<<dim3(32, hb.hc.ngroups, 1), HOUGH_THREADS, hb.smem, s>>>(hs.segs, hb.accum, hb.tabSin, hb.tabCos, hs.ctl, 0, hb.hc,
-                                                                               (size_t)d.NW, hb.accum_stride, (unsigned long long*)h->counters_d);
-    else
-        k_hough_vote<false><<<dim3(32, hb.hc.ngroups, 1), HOUGH_THREADS, hb.smem, s>>>(hs.segs, hb.accum, hb.tabSin, hb.tabCos, hs.ctl, 0, hb.hc,
-                                                                                (size_t)d.NW, hb.accum_stride, (unsigned long long*)h->counters_d);
-    LAUNCH_CHECK();
+    TRY(launch_hough_vote(h, hb, d, hs.segs, hb.accum, hs.ctl, 0, 1, s));
     CK(cudaEventRecord(h->ev[2], s));
     long long cells = (long long)hb.hc.numangle * hb.hc.numrho;
     int pblocks = (int)((cells + 255) / 256); if (pblocks > 1184) pblocks = 1184;
@@ -1556,42 +1580,22 @@ extern "C" int lfd_hough_lines(lfd_handle* h, const uint8_t* img, int height, in
 extern "C" int lfd_canny(lfd_handle* h, const uint8_t* img, int low, int high, uint8_t* edges_out)
 {
     if (!h || !img || !edges_out || low < 0 || high < low) { if (h) h->err = "bad argument"; return LFD_E_ARG; }
-    cudaSetDevice(h->device);
-    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    TRY(enter(h));
     const Dims d = h->d;
     cudaStream_t s = h->stream;
-    const int pass = 0, n = 1;
-    FrameCtl* const C = h->ctl;
-    CK(cudaMemcpyAsync(h->morph[pass], img, (size_t)d.N, cudaMemcpyHostToDevice, s));
+    const PassView V = pass_view(h, 0, 1, 0, 0, s);      // frame 0 of the bright pass
+    CK(cudaMemcpyAsync(V.morph, img, (size_t)d.N, cudaMemcpyHostToDevice, s));
     k_ctl_init<<<1, 32, 0, s>>>(h->ctl, h->B, h->res_d, 1, 1, 0, h->look, h->look_stride); LAUNCH_CHECK();
     // device times -> lfd_get_timings entries 0..1 (Sobel + NMS incl. the input mask, hysteresis by run CCL)
     CK(cudaEventRecord(h->ev[0], s));
-    k_pack_mask<<<592, 256, 0, s>>>(h->morph[pass], h->nz[pass], d); LAUNCH_CHECK();
-    if ((d.W % 8) == 0) {
-        const int nstrips = ((d.W >> 2) + MARCH_UW - 1) / MARCH_UW, nchunks = (d.H + NMS_R - 1) / NMS_R;
-        const int nunits = nstrips * nchunks;
-        CK(cudaMemsetAsync(h->cand[pass], 0, (size_t)d.NW * sizeof(u32), s));
-        CK(cudaMemsetAsync(h->strong[pass], 0, (size_t)d.NW * sizeof(u32), s));
-        k_nms_march<false><<<dim3((nunits + NMS_WPC - 1) / NMS_WPC, n), NMS_WPC * 32, 0, s>>>(h->morph[pass], h->nz[pass], h->cand[pass], h->strong[pass], nullptr, C, pass, d,
-                                                                  nstrips, nunits, low, high);
-    } else {
-        dim3 cg((d.W + CANNY_TW - 1) / CANNY_TW, (d.H + CANNY_TH - 1) / CANNY_TH, n);
-        k_canny_nms<<<cg, 256, 0, s>>>(h->morph[pass], h->nz[pass], h->cand[pass], h->strong[pass], nullptr, C, pass, d, low, high);
-    }
-    LAUNCH_CHECK();
+    k_pack_mask<<<592, 256, 0, s>>>(V.morph, V.nz, d); LAUNCH_CHECK();
+    TRY(launch_nms(V, low, high, nullptr));
     CK(cudaEventRecord(h->ev[1], s));
-    const int nbands = (d.H + CCL_BAND - 1) / CCL_BAND;
-    dim3 bands(nbands, n), seams((nbands + CCL_WARPS - 1) / CCL_WARPS, n);
-    k_ccl_band<<<bands, 256, ccl_band_smem(d.WW), s>>>(h->cand[pass], h->ccl_d[pass][0], C, pass, d, 0, h->cfg.max_runs,
-                                                      (unsigned long long*)h->counters_d); LAUNCH_CHECK();
-    k_ccl_merge<<<seams, CCL_WARPS * 32, 0, s>>>(h->ccl_d[pass][0], C, pass, d, 0); LAUNCH_CHECK();
-    CK(cudaMemsetAsync(h->edges[pass], 0, (size_t)d.NW * sizeof(u32), s));
-    k_ccl_stats_flat<<<dim3(CCL_FLAT_CTAS, n), 256, 0, s>>>(h->strong[pass], h->ccl_d[pass][0], C, pass, d, 0); LAUNCH_CHECK();
-    k_ccl_alloc_flat<<<dim3(CCL_FLAT_CTAS, n), 256, 0, s>>>(h->ccl_d[pass][0], h->edges[pass], h->comp_d[pass], C, pass, d, 0); LAUNCH_CHECK();
+    TRY(launch_labels(V, 0));
     CK(cudaEventRecord(h->ev[2], s));
-    k_expand_mask<<<dim3(592, 1), 256, 0, s>>>(h->edges[pass], h->tap_u8, d); LAUNCH_CHECK();
+    k_expand_mask<<<dim3(592, 1), 256, 0, s>>>(V.edges, h->tap_u8, d); LAUNCH_CHECK();
     FrameCtl out;
-    CK(cudaMemcpyAsync(&out, C, sizeof(out), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(&out, V.C, sizeof(out), cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpyAsync(edges_out, h->tap_u8, (size_t)d.N, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     memset(h->timings, 0, sizeof(h->timings));
@@ -1608,42 +1612,36 @@ extern "C" int lfd_fit_min_area_rect(lfd_handle* h, const uint8_t* img, int cont
                                      double minAreaRectMinLen, double lwTresh, uint8_t* box_out, int* detection)
 {
     if (!h || !img || !box_out || !detection) { if (h) h->err = "bad argument"; return LFD_E_ARG; }
-    cudaSetDevice(h->device);
-    if (h->pending) { h->err = "previous batch not collected (call lfd_wait)"; return LFD_E_STATE; }
+    TRY(enter(h));
     if (!h->have_params) { h->err = "lfd_set_params has not been called"; return LFD_E_STATE; }
-    if (contoursMode < 0 || contoursMode > 3) { h->err = "unknown contoursMode"; return LFD_E_ARG; }
-    if (contoursMethod != 1 && contoursMethod != 2) { h->err = "contoursMethod CHAIN_APPROX_TC89_* is not implemented"; return LFD_E_UNSUPPORTED; }
+    TRY(check_contours_args(h, contoursMode, contoursMethod));
     const Dims d = h->d;
     cudaStream_t s = h->stream;
-    const lfd_pass_params saved = h->params.bright;
-    h->params.bright.contoursMode = contoursMode; h->params.bright.contoursMethod = contoursMethod;
-    h->params.bright.minAreaRectMinLen = minAreaRectMinLen; h->params.bright.lwTresh = lwTresh;
-    int rc = LFD_OK;
-    do {
-        cudaError_t ce;
-        if ((ce = cudaMemcpyAsync(h->morph[0], img, (size_t)d.N, cudaMemcpyHostToDevice, s)) != cudaSuccess ||
-            (ce = cudaMemsetAsync(h->counters_d, 0, 16 * sizeof(int64_t), s)) != cudaSuccess) { h->err = cudaGetErrorString(ce); rc = LFD_E_CUDA; break; }
-        k_ctl_init<<<1, 32, 0, s>>>(h->ctl, h->B, h->res_d, 1, 1, 0, h->look, h->look_stride);
-        k_pack_mask<<<592, 256, 0, s>>>(h->morph[0], h->nz[0], d);
-        h->launches += 2;
-        h->cur_part = 0;
-        if ((rc = run_pass_kernels(h, 0, 1, 0, 0, s, false, 1)) != LFD_OK) break;
-        k_expand_mask<<<dim3(592, 1), 256, 0, s>>>(h->box[0], h->tap_u8, d);
-        h->launches++;
-        FrameCtl out;
-        if ((ce = cudaMemcpyAsync(&out, h->ctl, sizeof(out), cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
-            (ce = cudaMemcpyAsync(box_out, h->tap_u8, (size_t)d.N, cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
-            (ce = cudaMemcpyAsync(h->counters_h, h->counters_d, 16 * sizeof(int64_t), cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
-            (ce = cudaStreamSynchronize(s)) != cudaSuccess) { h->err = cudaGetErrorString(ce); rc = LFD_E_CUDA; break; }
-        // the RECTS tap of (frame 0, bright pass) reads its counts from the host copy of the frame's control block; no
-        // k_check_theta runs here to save them, so save this call's own counts
-        h->ctl_h[0].ncomp_saved[0][0] = out.ncomp[0];
-        h->ctl_h[0].ncomp_saved[0][1] = out.ncomp[1];
-        if (out.status & LFD_FRAME_OVERFLOW) { h->err = "per-frame work list overflow (lfd_config.max_runs / max_components)"; rc = LFD_E_CAPACITY; break; }
-        *detection = out.hough[0] ? 1 : 0;
-    } while (0);
-    h->params.bright = saved;
-    return rc;
+    const PassView V = pass_view(h, 0, 1, 0, 0, s);      // frame 0 of the bright pass
+    CK(cudaMemcpyAsync(V.morph, img, (size_t)d.N, cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(h->counters_d, 0, 16 * sizeof(int64_t), s));
+    k_ctl_init<<<1, 32, 0, s>>>(h->ctl, h->B, h->res_d, 1, 1, 0, h->look, h->look_stride); LAUNCH_CHECK();
+    k_pack_mask<<<592, 256, 0, s>>>(V.morph, V.nz, d); LAUNCH_CHECK();
+    TRY(launch_nms(V, 0, 255, nullptr));
+    for (int kind = 0; kind < 2; kind++) {
+        TRY(launch_labels(V, kind));
+        k_ccl_extremes_flat<<<dim3(CCL_FLAT_CTAS, 1), 256, 0, s>>>(V.edges, V.ccl[kind], V.comp, V.C, 0, d, kind); LAUNCH_CHECK();
+    }
+    // the box image is the call's output and its RECTS tap every rectangle: fit every contour
+    TRY(launch_contours(V, {minAreaRectMinLen, lwTresh, contoursMode == 0}, true));
+    k_expand_mask<<<dim3(592, 1), 256, 0, s>>>(V.box, h->tap_u8, d); LAUNCH_CHECK();
+    FrameCtl out;
+    CK(cudaMemcpyAsync(&out, V.C, sizeof(out), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(box_out, h->tap_u8, (size_t)d.N, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(h->counters_h, h->counters_d, 16 * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    // the RECTS tap of (frame 0, bright pass) reads its counts from the host copy of the frame's control block; no
+    // k_check_theta runs here to save them, so save this call's own counts
+    h->ctl_h[0].ncomp_saved[0][0] = out.ncomp[0];
+    h->ctl_h[0].ncomp_saved[0][1] = out.ncomp[1];
+    if (out.status & LFD_FRAME_OVERFLOW) { h->err = "per-frame work list overflow (lfd_config.max_runs / max_components)"; return LFD_E_CAPACITY; }
+    *detection = out.hough[0] ? 1 : 0;
+    return LFD_OK;
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -554,6 +554,51 @@ def test_shared_memory_and_accumulator_limits(handle, cv2mod):
         assert not errs, errs
 
 
+@pytest.mark.gpu
+def test_standalone_handles_keep_their_own_buffers(cv2mod):
+    """Two handles of different frame sizes on one device, their calls interleaved across image sizes, rho and theta
+    (theta = 3.0: a single angle), are each exact; after one handle is closed the other is exact again."""
+    from lfd_b200 import _lib
+    a, b = _lib.Handle(8, 8, max_batch=1), _lib.Handle(64, 96, max_batch=1)
+    try:
+        calls = [(a, img_edges(37, 33), 3, np.pi / 180), (b, img_ties(), 2, np.pi / 180), (a, img_ties(), 1, 3.0),
+                 (b, img_edges(37, 33), 1, 3.0), (a, img_edges(120, 200), 1, np.pi / 90), (b, img_ties(), 5, np.pi / 180),
+                 (a, img_edges(120, 200), 5, np.pi / 180), (b, img_edges(120, 200), 2, 3.0)]
+        for h, img, rho, theta in calls + calls:
+            errs, _, _ = _check_standalone(h, cv2mod, img, rho, theta, 0)
+            assert not errs, (img.shape, rho, theta, errs)
+        a.close()
+        for h, img, rho, theta in calls:
+            if h is b:
+                errs, _, _ = _check_standalone(b, cv2mod, img, rho, theta, 0)
+                assert not errs, (img.shape, rho, theta, errs)
+    finally:
+        a.close()
+        b.close()
+
+
+@pytest.mark.gpu
+def test_standalone_handles_on_two_devices(cv2mod):
+    """One handle on each of two devices, the same image size on both: every call runs on its own device's buffers."""
+    from lfd_b200 import _lib
+    handles = []
+    try:
+        for dev in (0, 1):
+            try:
+                handles.append(_lib.Handle(8, 8, max_batch=1, device=dev))
+            except _lib.LfdError as e:
+                if "no such CUDA device" not in str(e):
+                    raise
+                pytest.skip("fewer than two CUDA devices visible")
+        for img, rho, theta in ((img_ties(), 2, np.pi / 180), (img_ties(), 1, 3.0), (img_edges(64, 96), 5, np.pi / 90)):
+            for h in handles + handles:
+                errs, _, _ = _check_standalone(h, cv2mod, img, rho, theta, 0)
+                assert not errs, (h.device, img.shape, rho, theta, errs)
+    finally:
+        for h in handles:
+            h.close()
+
+
 # ---- the pipeline's Hough, k_check_theta and k_finalize --------------------------------------------------------------
 # (H, W, frames, houghMethod values): W % 32 == 12 (handles need W % 4 == 0), and the production frame
 BATCHES = [(160, 332, 24, (20, 5, 2, 1)), (1489, 2048, 6, (20,))]
