@@ -109,7 +109,9 @@ typedef struct lfd_pass_params {
     int32_t nlinesInSet;        /* <= LFD_MAX_SET_LINES */
     int32_t contoursMode;       /* cv2.RETR_*: LIST(1), CCOMP(2), TREE(3) give the same contour set; EXTERNAL(0) = outermost outer borders only */
     int32_t contoursMethod;     /* cv2.CHAIN_APPROX_NONE(1) or SIMPLE(2) (same hulls); TC89_* unsupported */
-    int32_t erode_h, erode_w;   /* 0,0 = no erosion (bright).  All-ones rectangles; other shapes: lfd_set_kernels. */
+    int32_t erode_h, erode_w;   /* 0,0 = no erosion (bright).  All-ones rectangles whose erode + dilate reach fits the
+                                   rectangle kernels' halo (rows <= 16, columns <= 12 left / 11 right); any other
+                                   element, up to 255 x 255: lfd_set_kernels. */
     int32_t dilate_h, dilate_w;
     int32_t reserved;
 } lfd_pass_params;
@@ -216,8 +218,12 @@ int lfd_set_params(lfd_handle* h, const lfd_params* p);
  * lfd/createjobs/createjobs.py:173-218). */
 int lfd_set_h2d_gate(lfd_handle* h, const char* lock_path);
 
-/* Structuring elements that are not all-ones rectangles (cv2.getStructuringElement crosses / ellipses, hand-made
- * masks), for one pass: row-major uint8 masks, non-zero = member, cv2's default anchor (kw/2, kh/2), sides 1..31.
+/* Flat structuring elements of any shape (cv2.getStructuringElement crosses / ellipses, rings, hand-made masks, and
+ * all-ones rectangles past the rectangle kernels' halo), for one pass: row-major uint8 masks, non-zero = member, any
+ * parity, cv2's default anchor (kw/2, kh/2) whether or not it is a member, sides 1..255 (larger: LFD_E_UNSUPPORTED; a
+ * mask without a member: LFD_E_ARG).  Semantics of cv2.erode / cv2.dilate with the default border: out-of-frame samples
+ * are ignored, also in frames smaller than the element; the erosion (dim pass only) runs first.  Evaluated by chord
+ * decomposition (DESIGN.md §3): the cost per pixel grows with the element's rows and runs, not with its area.
  * Call after lfd_set_params (which resets both passes to the all-ones rectangles of lfd_pass_params).
  * erode_mask may be NULL (no erosion; always ignored for the bright pass, processfield.py:354). */
 int lfd_set_kernels(lfd_handle* h, int pass, const uint8_t* erode_mask, int erode_h, int erode_w,

@@ -1,4 +1,5 @@
-// k_morph.cuh - erode / dilate with all-ones rectangular kernels, fused with the equalisation LUT.
+// k_morph.cuh - erode / dilate fused with the equalisation LUT: all-ones rectangles (k_morph_march, k_morph) and flat
+// structuring elements of any shape up to 255 x 255 (k_morph_any, chord decomposition).
 //
 // Reference: cv2.erode(equ, erodeKernel) processfield.py:464 ; cv2.dilate(., dilateKernel) :354, :471
 // (paths under /root/reference/lfd/detecttrails/).  cv2 semantics: anchor = (kw/2, kh/2), window rows
@@ -13,6 +14,7 @@
 // byte-wise SIMD min/max (__vminu4/__vmaxu4) with funnel shifts for the horizontal window.
 #pragma once
 #include "common.cuh"
+#include "chords.cuh"
 
 #define MORPH_TW 128                // tile width in pixels
 #define MORPH_TWW (MORPH_TW / 4)    // in 4-pixel words
@@ -427,83 +429,119 @@ k_morph_march(const u8* __restrict__ gray, const u8* __restrict__ lut, u8* __res
 }
 
 // ================================================================================================
-// Arbitrary structuring elements (cv2.getStructuringElement crosses / ellipses, hand-made masks):
-// direct evaluation over the list of non-zero kernel offsets on a shared-memory tile.  Slow path by
-// design - the all-ones rectangles the reference's defaults use never come here.
+// Arbitrary flat structuring elements (cv2.getStructuringElement ellipses / crosses, rings, hand-made masks, all-ones
+// rectangles past the tile halo), sides 1..CHORD_MAX_SIDE: the chord decomposition of chords.cuh, one launch per
+// operation (erosion into a scratch plane, then dilation + LUT + mask bits).
+//
+// A CTA owns a strip of CHORD_SW output columns (one per thread) and a chunk of CHORD_R output rows.  It reads each
+// input row the chunk needs once, with the element's horizontal reach on both sides, and builds that row's sparse-table
+// levels P_0 .. P_{nlev-1} in shared memory.  Mask row i of the element folds its chords' result into output row
+// y = r - (i - ay), held in a ring of kh partial rows; a row leaves the ring when mask row kh - 1 has contributed.
+// Per output pixel that is 2 * #chords + 1 shared-memory loads per mask row plus nlev per input row, against |M| for
+// the direct evaluation (DESIGN.md §3).  Out-of-frame samples are the identity (255 for min, 0 for max), so they are
+// ignored as cv2 ignores them; an input row holding only the identity (all outside the frame, or a zero row of a
+// dilation) contributes nothing and is skipped.
 // ================================================================================================
-#define ANYK_MAX 31                    // largest kernel side
-#define ANYK_TW 64
-#define ANYK_TH 16
+#define CHORD_SW 256                   // strip width in pixels = threads per CTA
+#define CHORD_R 64                     // output rows per chunk
 
-struct AnyKernel {
-    int n;                             // number of non-zero elements (0 = stage absent)
-    int reach;                         // max |offset|
-    signed char dx[ANYK_MAX * ANYK_MAX], dy[ANYK_MAX * ANYK_MAX];     // offsets relative to the anchor (kw/2, kh/2)
+struct ChordSet {
+    const int* rowoff;                 // [kh + 1] first chord of each mask row (chords.cuh)
+    const u32* code;                   // chord codes
+    int kh, kw, ay, ax, nlev;          // nlev: sparse-table levels the chords read
 };
 
-// dynamic smem: A = (TH + 2(re+rd)) x (TW + 2(re+rd)) bytes, B = (TH + 2rd) x (TW + 2rd) bytes
-__host__ __device__ inline size_t anyk_smem(int re, int rd)
+__host__ __device__ inline int chord_lw(int kw) { return (CHORD_SW + kw - 1 + 3) & ~3; }
+
+// dynamic smem: nlev level rows of chord_lw(kw) bytes, the kh-row ring, the LUT
+__host__ __device__ inline size_t chord_smem(int kh, int kw, int nlev)
 {
-    return (size_t)(ANYK_TH + 2 * (re + rd)) * (ANYK_TW + 2 * (re + rd)) + (size_t)(ANYK_TH + 2 * rd) * (ANYK_TW + 2 * rd) + 256;
+    return (size_t)nlev * chord_lw(kw) + (size_t)kh * CHORD_SW + 256;
 }
 
-__global__ void __launch_bounds__(256)
-k_morph_any(const u8* __restrict__ gray, const u8* __restrict__ lut, u8* __restrict__ morph, u32* __restrict__ nz,
-            u8* __restrict__ eroded_tap, const FrameCtl* __restrict__ ctl, int pass, Dims d,
-            const AnyKernel* __restrict__ ek, const AnyKernel* __restrict__ dk)
+template <bool IS_MAX> __device__ __forceinline__ u32 op8(u32 a, u32 b) { return IS_MAX ? max(a, b) : min(a, b); }
+
+// IS_MAX = false: erosion of `src` into `dst` (raw values), eroded tap = lut[dst].
+// IS_MAX = true: dilation of `src`, lut -> `dst` (the morphology plane) + nz; eroded_tap (runs without an erosion only)
+// = lut[src], as the pass's eroded plane is then its input.
+template <bool IS_MAX>
+__global__ void __launch_bounds__(CHORD_SW)
+k_morph_any(const u8* __restrict__ src, const u8* __restrict__ lut, u8* __restrict__ dst, u32* __restrict__ nz,
+            u8* __restrict__ eroded_tap, const FrameCtl* __restrict__ ctl, int pass, Dims d, ChordSet cs)
 {
     const int f = blockIdx.z;
     if (!ctl[f].active[pass]) return;
-    extern __shared__ u8 anysm[];
-    const int re = ek ? ek->reach : 0, rd = dk->reach;
-    const int ra = re + rd;
-    const int AW = ANYK_TW + 2 * ra, AH = ANYK_TH + 2 * ra, BW = ANYK_TW + 2 * rd, BH = ANYK_TH + 2 * rd;
-    u8* A = anysm;
-    u8* B = A + AW * AH;
-    u8* slut = B + BW * BH;
-    slut[threadIdx.x] = lut[(size_t)f * 256 + threadIdx.x];
-    const int tx0 = blockIdx.x * ANYK_TW, ty0 = blockIdx.y * ANYK_TH;
-    const u8* src = gray + (size_t)f * d.N;
-    if (ek && ek->n > 0) {
-        for (int i = threadIdx.x; i < AW * AH; i += blockDim.x) {
-            int r = i / AW, c = i - r * AW;
-            int y = ty0 - ra + r, x = tx0 - ra + c;
-            A[i] = (y >= 0 && y < d.H && x >= 0 && x < d.W) ? src[(size_t)y * d.W + x] : (u8)255;     // ignored by min
-        }
-        __syncthreads();
-        const int n = ek->n;
-        for (int i = threadIdx.x; i < BW * BH; i += blockDim.x) {
-            int r = i / BW, c = i - r * BW;
-            int y = ty0 - rd + r, x = tx0 - rd + c;
-            int v = 0;                                              // outside the frame: ignored by max
-            if (y >= 0 && y < d.H && x >= 0 && x < d.W) {
-                v = 255;
-                for (int k = 0; k < n; k++) v = min(v, (int)A[(r + re + ek->dy[k]) * AW + (c + re + ek->dx[k])]);
+    extern __shared__ u32 chsm_[];
+    const int LW = chord_lw(cs.kw), kh = cs.kh, ay = cs.ay;
+    u8* lv = reinterpret_cast<u8*>(chsm_);
+    u8* ring = lv + cs.nlev * LW;
+    u8* slut = ring + kh * CHORD_SW;
+    const int tx = threadIdx.x;
+    slut[tx] = lut[(size_t)f * 256 + tx];
+    const u32 ID = IS_MAX ? 0u : 255u;
+    for (int i = 0; i < kh; i++) ring[i * CHORD_SW + tx] = (u8)ID;      // a thread's ring column is its own
+    const int x0 = blockIdx.x * CHORD_SW, y0 = blockIdx.y * CHORD_R, y1 = min(y0 + CHORD_R, d.H);
+    const int x = x0 + tx, xs = x0 - cs.ax;                              // xs: frame column of level column 0
+    const bool xin = x < d.W;
+    const u8* in = src + (size_t)f * d.N;
+    u8* out = dst + (size_t)f * d.N;
+    u8* et = eroded_tap ? eroded_tap + (size_t)f * d.N : nullptr;
+    const int rlast = y1 - 1 + (kh - 1 - ay);
+    for (int r = y0 - ay; r <= rlast; r++) {
+        bool any = false;
+        if (r >= 0 && r < d.H) {
+            const u8* row = in + (size_t)r * d.W;
+            for (int c = tx; c < LW; c += CHORD_SW) {
+                const int xc = xs + c;
+                const u32 v = (xc >= 0 && xc < d.W) ? row[xc] : ID;
+                lv[c] = (u8)v;
+                any |= v != ID;
             }
-            B[i] = (u8)v;
         }
-    } else {
-        for (int i = threadIdx.x; i < BW * BH; i += blockDim.x) {
-            int r = i / BW, c = i - r * BW;
-            int y = ty0 - rd + r, x = tx0 - rd + c;
-            B[i] = (y >= 0 && y < d.H && x >= 0 && x < d.W) ? src[(size_t)y * d.W + x] : (u8)0;
+        const bool busy = __syncthreads_or(any);
+        if (IS_MAX && et && r >= y0 && r < y1 && xin) et[(size_t)r * d.W + x] = slut[lv[tx + cs.ax]];
+        if (busy) {
+            for (int k = 1; k < cs.nlev; k++) {
+                const u8* p = lv + (k - 1) * LW;
+                u8* q = lv + k * LW;
+                const int s = 1 << (k - 1);
+                for (int c = tx; c + 2 * s <= LW; c += CHORD_SW) q[c] = (u8)op8<IS_MAX>(p[c], p[c + s]);
+                __syncthreads();
+            }
+            // mask rows i whose output row y = r - i + ay lies in the chunk; ring slot (y - y0) % kh
+            const int ilo = max(0, r + ay - y1 + 1), ihi = min(kh - 1, r + ay - y0);
+            int slot = (r + ay - ilo - y0) % kh;
+            for (int i = ilo; i <= ihi; i++) {
+                const int c0 = __ldg(cs.rowoff + i), c1 = __ldg(cs.rowoff + i + 1);
+                if (c0 < c1) {
+                    u32 acc = ID;
+                    for (int c = c0; c < c1; c++) {
+                        const u32 q = __ldg(cs.code + c);
+                        const u8* P = lv + (q >> 16) * LW + tx;
+                        acc = op8<IS_MAX>(acc, op8<IS_MAX>(P[q & 255u], P[(q >> 8) & 255u]));
+                    }
+                    u8* rv = ring + slot * CHORD_SW + tx;
+                    *rv = (u8)op8<IS_MAX>(*rv, acc);
+                }
+                slot = slot == 0 ? kh - 1 : slot - 1;
+            }
         }
-    }
-    __syncthreads();
-    const int n = dk->n;
-    for (int i = threadIdx.x; i < ANYK_TW * ANYK_TH; i += blockDim.x) {
-        int r = i / ANYK_TW, c = i - r * ANYK_TW;          // a warp covers 32 consecutive pixels of one row
-        int y = ty0 + r, x = tx0 + c;
-        const bool in = y < d.H && x < d.W;
-        int o = 0;
-        if (in) {
-            int v = 0;
-            for (int k = 0; k < n; k++) v = max(v, (int)B[(r + rd + dk->dy[k]) * BW + (c + rd + dk->dx[k])]);
-            o = slut[v];
-            morph[(size_t)f * d.N + (size_t)y * d.W + x] = (u8)o;
-            if (eroded_tap) eroded_tap[(size_t)f * d.N + (size_t)y * d.W + x] = slut[B[(r + rd) * BW + (c + rd)]];
+        const int y = r - (kh - 1 - ay);                 // complete: mask row kh - 1 has contributed
+        if (y >= y0) {
+            u8* rv = ring + ((y - y0) % kh) * CHORD_SW + tx;
+            const u32 v = *rv;
+            *rv = (u8)ID;
+            if (IS_MAX) {
+                const u32 o = slut[v];
+                if (xin) out[(size_t)y * d.W + x] = (u8)o;
+                const u32 b = __ballot_sync(FULLMASK, xin && o != 0u);
+                const int mw = (x0 >> 5) + (tx >> 5);
+                if (lane_id() == 0 && mw < d.WW) nz[(size_t)f * d.NW + (size_t)y * d.WW + mw] = b;
+            } else if (xin) {
+                out[(size_t)y * d.W + x] = (u8)v;
+                if (et) et[(size_t)y * d.W + x] = slut[v];
+            }
         }
-        u32 b = __ballot_sync(FULLMASK, in && o != 0);
-        if (lane_id() == 0 && y < d.H && (x >> 5) < d.WW) nz[(size_t)f * d.NW + (size_t)y * d.WW + (x >> 5)] = b;
+        __syncthreads();                                 // the next row overwrites the levels
     }
 }

@@ -176,10 +176,11 @@ struct lfd_handle {
     int graph_n = 0, graph_flags = 0;
     int64_t graph_launches = 0;
     bool stage_timings_valid = true;
-    // arbitrary structuring elements (lfd_set_kernels): [pass][0 erode / 1 dilate]; n == 0 -> the all-ones rectangle of lfd_pass_params
-    AnyKernel* anyk_d = nullptr;      // [2][2]
-    AnyKernel anyk_h[2][2];
+    // arbitrary structuring elements (lfd_set_kernels): [pass][0 erode / 1 dilate] chord lists (chords.cuh) in device
+    // buffers sized by the element; kh == 0: no erosion.  anyk_on[pass] false: the all-ones rectangles of lfd_pass_params
+    struct AnyElem { int kh = 0, kw = 0, nlev = 0; int* buf = nullptr; size_t cap = 0; } anyk[2][2];
     bool anyk_on[2] = {false, false};
+    u8* anyk_eroded = nullptr;        // [B][N] the dim pass's erosion, allocated with its first erosion element
     int prep_grid[3] = {0, 0, 0};     // resident CTAs of k_prep<mode> on this device (one full wave)
     cudaEvent_t mark[4];              // caller-placed timestamps on the handle's stream (lfd_timer_mark)
     bool mark_valid[4];
@@ -418,6 +419,7 @@ extern "C" int lfd_destroy(lfd_handle* h)
     for (int p = 0; p < 2; p++) hough_free(h->hb[p]);
     hough_scratch_free(h->hs);
     cudaFree(h->base_d); cudaFree(h->tab_samples_d);
+    for (int p = 0; p < 2; p++) for (int k = 0; k < 2; k++) cudaFree(h->anyk[p][k].buf);
     for (void* p : {(void*)h->frames_h, (void*)h->res_h, (void*)h->rects_h, (void*)h->rect_off_h, (void*)h->ctl_h,
                     (void*)h->inj_trails_h, (void*)h->inj_off_h, (void*)h->inj_base_h, (void*)h->counters_h})
         cudaFreeHost(p);
@@ -530,8 +532,6 @@ static int create_impl(lfd_handle* h, int device, int max_batch, int H, int W, c
     }
     DA(h->tap_u8, N);
     DA(h->ctl, (size_t)2 * B);
-    DA(h->anyk_d, 4);
-    memset(h->anyk_h, 0, sizeof(h->anyk_h));
     DA(h->res_d, (size_t)B);
     DA(h->counters_d, 16);
     DA(h->segs[0], (size_t)B * 2 * NW);
@@ -676,20 +676,28 @@ extern "C" int lfd_set_params(lfd_handle* h, const lfd_params* p)
     return LFD_OK;
 }
 
-static int fill_anykernel(lfd_handle* h, AnyKernel* k, const uint8_t* mask, int kh, int kw, const char* what)
+// The chord list of one element (chords.cuh) into its device buffer: rowoff[kh + 1], then the chord codes
+static int fill_anykernel(lfd_handle* h, lfd_handle::AnyElem* k, const uint8_t* mask, int kh, int kw, const char* what)
 {
-    memset(k, 0, sizeof(*k));
+    k->kh = k->kw = k->nlev = 0;
     if (!mask || kh == 0 || kw == 0) return LFD_OK;
-    if (kh < 1 || kw < 1 || kh > ANYK_MAX || kw > ANYK_MAX) { h->err = std::string(what) + ": kernel side must be 1..31"; return LFD_E_UNSUPPORTED; }
-    const int ay = kh / 2, ax = kw / 2;        // cv2's default anchor
-    for (int i = 0; i < kh; i++)
-        for (int j = 0; j < kw; j++)
-            if (mask[i * kw + j]) {
-                k->dy[k->n] = (signed char)(i - ay); k->dx[k->n] = (signed char)(j - ax);
-                k->reach = std::max(k->reach, std::max(abs(i - ay), abs(j - ax)));
-                k->n++;
-            }
-    if (k->n == 0) { h->err = std::string(what) + ": structuring element has no non-zero entry"; return LFD_E_ARG; }
+    if (kh < 1 || kw < 1 || kh > CHORD_MAX_SIDE || kw > CHORD_MAX_SIDE) {
+        h->err = std::string(what) + ": kernel side must be 1.." + std::to_string(CHORD_MAX_SIDE);
+        return LFD_E_UNSUPPORTED;
+    }
+    std::vector<int> buf(kh + 1 + chord_capacity(kh, kw));
+    int nlev = 0;
+    const int n = chord_decompose(mask, kh, kw, buf.data(), reinterpret_cast<uint32_t*>(buf.data() + kh + 1), &nlev);
+    if (n == 0) { h->err = std::string(what) + ": structuring element has no non-zero entry"; return LFD_E_ARG; }
+    const size_t need = (size_t)(kh + 1 + n) * sizeof(int);
+    if (need > k->cap) {
+        cudaFree(k->buf);
+        k->buf = nullptr; k->cap = 0;
+        CK(cudaMalloc(&k->buf, need));
+        k->cap = need;
+    }
+    CK(cudaMemcpy(k->buf, buf.data(), need, cudaMemcpyHostToDevice));
+    k->kh = kh; k->kw = kw; k->nlev = nlev;
     return LFD_OK;
 }
 
@@ -702,14 +710,23 @@ extern "C" int lfd_set_kernels(lfd_handle* h, int pass, const uint8_t* erode_mas
     cudaSetDevice(h->device);
     if (!h->have_params) { h->err = "lfd_set_params has not been called"; return LFD_E_STATE; }
     CK(cudaStreamSynchronize(h->stream));
-    TRY(fill_anykernel(h, &h->anyk_h[pass][0], pass == 1 ? erode_mask : nullptr, eh, ew, "erodeKernel"));
-    TRY(fill_anykernel(h, &h->anyk_h[pass][1], dilate_mask, dh, dw, "dilateKernel"));
-    CK(cudaMemcpy(h->anyk_d + pass * 2, &h->anyk_h[pass][0], 2 * sizeof(AnyKernel), cudaMemcpyHostToDevice));
+    h->anyk_on[pass] = false;                    // until both elements are in place
+    TRY(fill_anykernel(h, &h->anyk[pass][0], pass == 1 ? erode_mask : nullptr, eh, ew, "erodeKernel"));
+    TRY(fill_anykernel(h, &h->anyk[pass][1], dilate_mask, dh, dw, "dilateKernel"));
+    if (h->anyk[pass][0].kh > 0 && !h->anyk_eroded) TRY(dev_alloc(h, &h->anyk_eroded, (size_t)h->B * h->d.N));
     h->anyk_on[pass] = true;
     if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
-    size_t need = anyk_smem(h->anyk_h[pass][0].reach, h->anyk_h[pass][1].reach);
+    size_t need = 0;
+    for (int k = 0; k < 2; k++) {
+        const lfd_handle::AnyElem& e = h->anyk[pass][k];
+        if (e.kh > 0) need = std::max(need, chord_smem(e.kh, e.kw, e.nlev));
+    }
     DevLimits& L = g_dev_limits[h->device % LFD_MAX_DEVICES];
-    if (need > L.anyk_max) { CK(cudaFuncSetAttribute(k_morph_any, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need)); L.anyk_max = need; }
+    if (need > L.anyk_max) {
+        CK(cudaFuncSetAttribute(k_morph_any<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
+        CK(cudaFuncSetAttribute(k_morph_any<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
+        L.anyk_max = need;
+    }
     return LFD_OK;
 }
 
@@ -867,12 +884,23 @@ static int run_pass_kernels(lfd_handle* h, int f0, int n, int pass, int flags, c
         const int nunits = nstrips * nchunks;
         dim3 gg((nunits + MARCH_WPC - 1) / MARCH_WPC, n);
         bool done = false;
-        if (h->anyk_on[pass]) {
-            const AnyKernel* ekd = (pass == 1 && h->anyk_h[pass][0].n > 0) ? h->anyk_d + pass * 2 : nullptr;
-            const AnyKernel* dkd = h->anyk_d + pass * 2 + 1;
-            const int re = ekd ? h->anyk_h[pass][0].reach : 0, rd = h->anyk_h[pass][1].reach;
-            dim3 ag((d.W + ANYK_TW - 1) / ANYK_TW, (d.H + ANYK_TH - 1) / ANYK_TH, n);
-            k_morph_any<<<ag, 256, anyk_smem(re, rd), s>>>(V.gray, lutp, V.morph, V.nz, etap, C, pass, d, ekd, dkd);
+        if (h->anyk_on[pass]) {     // erosion into the scratch plane, then dilation of it (or of gray)
+            const dim3 ag((d.W + CHORD_SW - 1) / CHORD_SW, (d.H + CHORD_R - 1) / CHORD_R, n);
+            auto chords = [](const lfd_handle::AnyElem& e) {
+                return ChordSet{e.buf, reinterpret_cast<const u32*>(e.buf + e.kh + 1), e.kh, e.kw, e.kh / 2, e.kw / 2, e.nlev};
+            };
+            const lfd_handle::AnyElem &ee = h->anyk[pass][0], &de = h->anyk[pass][1];
+            const u8* dsrc = V.gray;
+            if (pass == 1 && ee.kh > 0) {
+                u8* er = h->anyk_eroded + fN;
+                k_morph_any<false><<<ag, CHORD_SW, chord_smem(ee.kh, ee.kw, ee.nlev), s>>>(V.gray, lutp, er, nullptr, etap, C,
+                                                                                         pass, d, chords(ee));
+                LAUNCH_CHECK();
+                dsrc = er;
+                etap = nullptr;
+            }
+            k_morph_any<true><<<ag, CHORD_SW, chord_smem(de.kh, de.kw, de.nlev), s>>>(dsrc, lutp, V.morph, V.nz, etap, C, pass,
+                                                                                    d, chords(de));
             done = true;
         }
 #define MORPH_CASE(EH_, EW_, DH_, DW_)                                                                              \
