@@ -254,8 +254,17 @@ int lfd_run_resident(lfd_handle* h, int n, int flags);
  * k_inject just before the pipeline, so no pixel data crosses the host link.  It takes lfd_submit's flags except
  * LFD_INPUT_BIGENDIAN; collect with lfd_wait.  LFD_E_ARG with nothing launched when n is outside 1..max_batch, a base
  * index is out of range, a slot has more than LFD_MAX_INJECT_TRAILS trails, or a trail value is not finite or
- * sigma <= 0; LFD_E_STATE when no base has been set.  k_inject's duration is lfd_get_kernel_times index 12. */
+ * sigma <= 0; LFD_E_STATE when no base has been set.  k_inject's duration is lfd_get_kernel_times index 14. */
 int lfd_set_base(lfd_handle* h, const float* frames, int n_base, const int32_t* rects, const int32_t* rect_offsets);
+/* Make the n frames of the last collected whole-frame batch (lfd_submit, or lfd_upload + lfd_run_resident) the handle's
+ * injection bases, without any host<->device copy: base b = batch slot b in native byte order (byte-swapped on the device
+ * when that batch was LFD_INPUT_BIGENDIAN), with the star rectangles that batch was submitted with.  Replaces the bases
+ * like lfd_set_base.  LFD_E_STATE, with nothing launched, while a batch is pending, before any whole-frame batch, and when
+ * the slots no longer hold that batch's input (after lfd_run_pass, lfd_blot, lfd_submit_injected[_shaped], and
+ * lfd_run_resident of injected frames).  Asynchronous: the copy, k_capture_bases, runs on the handle's stream ahead of the
+ * next lfd_submit_injected; its duration is lfd_get_kernel_times index 15 of the next collected batch.  A drop-in run
+ * can so measure completeness on every frame it reads, at the cost of one device copy per batch. */
+int lfd_capture_bases(lfd_handle* h);
 int lfd_submit_injected(lfd_handle* h, int n, const int32_t* base_index, const lfd_trail* trails,
                         const int32_t* trail_offsets, int flags);
 /* lfd_set_trail_tables uploads the pool of tabulated shapes (lfd_table) once, synchronously; a second call replaces it.
@@ -312,6 +321,7 @@ int lfd_get_timings(lfd_handle* h, float* ms, int max_entries, int* n_entries);
    the captured graph of the production path - so the durations are measured live, with the other streams running.
    index = 0 .. 13 (7 kernels x 2 passes); ms is summed over the batch parts, launches = number of parts.
    index 14 = k_inject of the last collected lfd_submit_injected batch (always bracketed; launches 0 otherwise).
+   index 15 = k_capture_bases of an lfd_capture_bases call made before the last collected batch (launches 0 otherwise).
    Returns LFD_E_ARG past the last index. */
 int lfd_get_kernel_times(lfd_handle* h, int index, const char** name, int* pass, float* ms, int* launches);
 const char* lfd_timing_name(int i);

@@ -142,7 +142,8 @@ def lib():
                                        ctypes.c_double, ctypes.c_double, ctypes.c_longlong, ctypes.c_double,
                                        ctypes.POINTER(ctypes.c_char_p), ctypes.c_int, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_int,
                                        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]
-        for sym in ("lfd_set_base", "lfd_submit_injected", "lfd_set_trail_tables", "lfd_submit_injected_shaped"):
+        for sym in ("lfd_set_base", "lfd_submit_injected", "lfd_set_trail_tables", "lfd_submit_injected_shaped",
+                    "lfd_capture_bases"):
             # added within ABI version 1: a stale build lacks them
             if not hasattr(L, sym):
                 raise ImportError("liblfd_b200.so predates %s: rebuild it (`python -c 'import __graft_entry__ as g; g.build()'`)" % sym)
@@ -152,6 +153,7 @@ def lib():
         L.lfd_set_trail_tables.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
         L.lfd_submit_injected_shaped.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
                                                  ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]
+        L.lfd_capture_bases.argtypes = [ctypes.c_void_p]
         if L.lfd_abi_version() != 1:
             raise ImportError("liblfd_b200.so ABI mismatch")
         _lib = L
@@ -398,6 +400,11 @@ class Handle:
             raise ValueError("frames must have shape (n, %d, %d)" % (self.H, self.W))
         _flat, _offs, rp, op = self._rects_arrays(rects_per_frame)
         self._ck(self._L.lfd_set_base(self.h, frames.ctypes.data_as(ctypes.c_void_p), frames.shape[0], rp, op))
+
+    def capture_bases(self):
+        """Make the frames of the last collected whole-frame batch the injection bases (base b = slot b, native order,
+        with the batch's star rectangles), without any host<->device copy (include/lfd_b200.h: lfd_capture_bases)."""
+        self._ck(self._L.lfd_capture_bases(self.h))
 
     def set_trail_tables(self, tables):
         """Upload the pool of tabulated trail shapes, a list of ``(lo, hi, samples)`` (``samples`` evenly spaced on

@@ -1,4 +1,5 @@
-// k_inject.cuh - on-device trail injection for completeness campaigns (lfd_set_base / lfd_submit_injected[_shaped]).
+// k_inject.cuh - on-device trail injection for completeness campaigns (lfd_set_base / lfd_submit_injected[_shaped]),
+// and k_capture_bases, which makes a collected batch the injection bases (lfd_capture_bases).
 //
 // in[f] = base[base_index[f]] + the line segments of slot f (the checkers are oracle/inject_ref.py::render_trails and,
 // for tabulated shapes, tests/inject_shapes_ref.py::render_trails).  Per pixel, in float32 and in
@@ -132,6 +133,32 @@ k_inject(const float* __restrict__ base, const int* __restrict__ base_index, con
                 }
             }
             dst[i] = v[j];
+        }
+    }
+}
+
+#define CAP_THREADS 256
+
+// lfd_capture_bases: the batch slots -> the injection bases, n16 16-byte words, each 4-byte word byte-swapped when the
+// slots hold a raw FITS payload (BE).  Grid-stride, four independent loads in flight per thread; the slots are
+// overwritten by k_inject next, so they are read with evict-first loads.
+template <bool BE>
+__global__ void __launch_bounds__(CAP_THREADS) k_capture_bases(const uint4* __restrict__ src, uint4* __restrict__ dst, size_t n16)
+{
+    const size_t step = (size_t)gridDim.x * CAP_THREADS;
+    for (size_t i0 = (size_t)blockIdx.x * CAP_THREADS + threadIdx.x; i0 < n16; i0 += 4 * step) {
+        uint4 v[4];
+#pragma unroll
+        for (int j = 0; j < 4; j++)
+            if (i0 + j * step < n16) v[j] = __ldcs(src + i0 + j * step);
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            if (i0 + j * step >= n16) break;
+            if (BE) {
+                v[j].x = __byte_perm(v[j].x, 0, 0x0123); v[j].y = __byte_perm(v[j].y, 0, 0x0123);
+                v[j].z = __byte_perm(v[j].z, 0, 0x0123); v[j].w = __byte_perm(v[j].w, 0, 0x0123);
+            }
+            dst[i0 + j * step] = v[j];
         }
     }
 }

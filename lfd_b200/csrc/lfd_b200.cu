@@ -97,8 +97,9 @@ struct lfd_handle {
     int64_t launches = 0;
     int last_n = 0, last_flags = 0;
     bool pending = false;
-    // what h->in holds: the un-flipped frames the last whole-frame run read (LFD_STAGE_INPUT), in FITS byte order if in_be
-    bool in_whole = false, in_be = false;
+    // what h->in holds: the un-flipped frames the last whole-frame run read (LFD_STAGE_INPUT), in FITS byte order if in_be;
+    // in_injected: they are base + trails written by lfd_submit_injected (until the next lfd_upload), not a submitted batch
+    bool in_whole = false, in_be = false, in_injected = false;
 
     // device
     float* in = nullptr;              // [B][N]
@@ -152,6 +153,10 @@ struct lfd_handle {
     cudaEvent_t ev_inj[2] = {nullptr, nullptr};   // around k_inject; inj_recorded: the last run was lfd_submit_injected
     bool inj_recorded = false;
     float inj_ms = 0.f;
+    cudaEvent_t ev_cap[2] = {nullptr, nullptr};   // around k_capture_bases; reported with the next collected batch
+    bool cap_recorded = false;
+    float cap_ms = 0.f;
+    int cap_launches = 0;
 
     // host
     float* frames_h = nullptr;        // pinned [B][N]
@@ -172,9 +177,10 @@ struct lfd_handle {
     // CUDA graph of the two passes + verdict + result copies (whole-frame path without taps): ~100 small launches
     // become one graph launch, which removes the per-launch gaps between the latency-bound kernels
     bool use_graphs = true;
-    cudaGraphExec_t graph_exec = nullptr;
-    int graph_n = 0, graph_flags = 0;
-    int64_t graph_launches = 0;
+    // one instantiated graph per (n, flags) in use, oldest first: a drop-in run with injections alternates its big-endian
+    // batches with native injected steps, which would otherwise re-capture the graph twice per batch
+    struct CachedGraph { cudaGraphExec_t exec; int n, flags; int64_t launches; };
+    std::vector<CachedGraph> graphs;
     bool stage_timings_valid = true;
     // arbitrary structuring elements (lfd_set_kernels): [pass][0 erode / 1 dilate] chord lists (chords.cuh) in device
     // buffers sized by the element; kh == 0: no erosion.  anyk_on[pass] false: the all-ones rectangles of lfd_pass_params
@@ -235,6 +241,14 @@ static int dev_alloc(lfd_handle* h, T** p, size_t count)
 }
 
 static int next_pow2(int v) { int p = 1; while (p < v) p <<= 1; return p; }
+
+#define GRAPH_CACHE 4                 // instantiated graphs kept per handle (lfd_handle::graphs)
+
+static void graphs_clear(lfd_handle* h)
+{
+    for (auto& g : h->graphs) cudaGraphExecDestroy(g.exec);
+    h->graphs.clear();
+}
 
 // prologue of the entry points that enqueue work: the handle's device, and no batch in flight
 static int enter(lfd_handle* h)
@@ -423,7 +437,10 @@ extern "C" int lfd_destroy(lfd_handle* h)
     for (void* p : {(void*)h->frames_h, (void*)h->res_h, (void*)h->rects_h, (void*)h->rect_off_h, (void*)h->ctl_h,
                     (void*)h->inj_trails_h, (void*)h->inj_off_h, (void*)h->inj_base_h, (void*)h->counters_h})
         cudaFreeHost(p);
-    for (int i = 0; i < 2; i++) if (h->ev_inj[i]) cudaEventDestroy(h->ev_inj[i]);
+    for (int i = 0; i < 2; i++) {
+        if (h->ev_inj[i]) cudaEventDestroy(h->ev_inj[i]);
+        if (h->ev_cap[i]) cudaEventDestroy(h->ev_cap[i]);
+    }
     for (int i = 0; i <= N_TIMINGS; i++) if (h->ev_valid[i]) cudaEventDestroy(h->ev[i]);
     for (int k = 0; k < LFD_BATCH_PARTS; k++)
         for (int p = 0; p < 2; p++)
@@ -431,7 +448,7 @@ extern "C" int lfd_destroy(lfd_handle* h)
                 for (int e = 0; e < 2; e++)
                     if (h->kb[k][p][b][e]) cudaEventDestroy(h->kb[k][p][b][e]);
     for (int i = 0; i < 4; i++) if (h->mark_valid[i]) cudaEventDestroy(h->mark[i]);
-    if (h->graph_exec) cudaGraphExecDestroy(h->graph_exec);
+    graphs_clear(h);
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     for (int k = 0; k < LFD_BATCH_PARTS; k++)
         for (int p = 0; p < 2; p++) {
@@ -672,7 +689,7 @@ extern "C" int lfd_set_params(lfd_handle* h, const lfd_params* p)
     h->params = *p;
     h->have_params = true;
     h->anyk_on[0] = h->anyk_on[1] = false;       // back to all-ones rectangles until lfd_set_kernels says otherwise
-    if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }   // kernel arguments changed
+    graphs_clear(h);                             // kernel arguments changed
     return LFD_OK;
 }
 
@@ -715,7 +732,7 @@ extern "C" int lfd_set_kernels(lfd_handle* h, int pass, const uint8_t* erode_mas
     TRY(fill_anykernel(h, &h->anyk[pass][1], dilate_mask, dh, dw, "dilateKernel"));
     if (h->anyk[pass][0].kh > 0 && !h->anyk_eroded) TRY(dev_alloc(h, &h->anyk_eroded, (size_t)h->B * h->d.N));
     h->anyk_on[pass] = true;
-    if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
+    graphs_clear(h);
     size_t need = 0;
     for (int k = 0; k < 2; k++) {
         const lfd_handle::AnyElem& e = h->anyk[pass][k];
@@ -964,7 +981,9 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
     h->inj_recorded = false;           // lfd_submit_injected sets it after this returns
     CK(cudaMemsetAsync(h->counters_d, 0, 16 * sizeof(int64_t), s));
     CK(cudaEventRecord(h->ev[0], s));
-    const bool replay = h->graph_exec && h->use_graphs && h->graph_n == n && h->graph_flags == flags && mode == 0 &&
+    lfd_handle::CachedGraph* cached = nullptr;
+    for (auto& g : h->graphs) if (g.n == n && g.flags == flags) cached = &g;
+    const bool replay = cached && h->use_graphs && mode == 0 &&
                         !(flags & (LFD_SERIAL_PASSES | LFD_KEEP_TAPS | LFD_FULL_LINES)) && !h->ktiming;
     if (!replay) memset(h->kb_used, 0, sizeof(h->kb_used));       // a replayed graph records the brackets of its capture again
     if (h->ktiming) { h->kn = 0; ktime_mark(h, 0); }
@@ -1048,8 +1067,8 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
         return LFD_OK;
     };
     if (graph) {
-        if (!h->graph_exec || h->graph_n != n || h->graph_flags != flags) {
-            if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
+        if (!cached) {
+            if ((int)h->graphs.size() >= GRAPH_CACHE) { cudaGraphExecDestroy(h->graphs.front().exec); h->graphs.erase(h->graphs.begin()); }
             const int64_t l0 = h->launches;
             CK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
             const int rc = passes(false);
@@ -1057,15 +1076,16 @@ static int run_pipeline(lfd_handle* h, int n, int flags, int mode, bool want_cli
             cudaError_t ce = cudaStreamEndCapture(s, &g);
             if (rc != LFD_OK) { if (g) cudaGraphDestroy(g); cudaGetLastError(); return rc; }
             if (ce != cudaSuccess) { h->err = std::string("cudaStreamEndCapture: ") + cudaGetErrorString(ce); return LFD_E_CUDA; }
-            ce = cudaGraphInstantiate(&h->graph_exec, g, 0);
+            cudaGraphExec_t exec = nullptr;
+            ce = cudaGraphInstantiate(&exec, g, 0);
             cudaGraphDestroy(g);
-            if (ce != cudaSuccess) { h->graph_exec = nullptr; h->err = std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ce); return LFD_E_CUDA; }
-            h->graph_launches = h->launches - l0;
+            if (ce != cudaSuccess) { h->err = std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ce); return LFD_E_CUDA; }
+            h->graphs.push_back({exec, n, flags, h->launches - l0});
             h->launches = l0;
-            h->graph_n = n; h->graph_flags = flags;
+            cached = &h->graphs.back();
         }
-        CK(cudaGraphLaunch(h->graph_exec, s));
-        h->launches += h->graph_launches;
+        CK(cudaGraphLaunch(cached->exec, s));
+        h->launches += cached->launches;
     } else {
         TRY(passes(true));
     }
@@ -1131,7 +1151,7 @@ extern "C" int lfd_upload(lfd_handle* h, const float* frames, int n, const int32
     }
     if (ce != cudaSuccess) { h->err = std::string("cudaMemcpyAsync(H2D): ") + cudaGetErrorString(ce); return LFD_E_CUDA; }
     h->last_flags = flags;
-    h->in_whole = false;
+    h->in_whole = h->in_injected = false;
     return LFD_OK;
 }
 
@@ -1164,17 +1184,15 @@ extern "C" int lfd_run_resident(lfd_handle* h, int n, int flags)
 // ------------------------------------------------------------------------------------------------
 // injection campaigns: resident bases + per-slot synthetic trails added on the device before k_prep
 // ------------------------------------------------------------------------------------------------
-extern "C" int lfd_set_base(lfd_handle* h, const float* frames, int n_base, const int32_t* rects, const int32_t* rect_offsets)
+// room for n_base bases and the per-slot trail buffers, allocated on first use by lfd_set_base / lfd_capture_bases;
+// the current bases are dropped (n_base = 0) until the caller has replaced them
+static int inj_reserve(lfd_handle* h, int n_base)
 {
-    if (!h) return LFD_E_ARG;
-    if (!frames || n_base < 1) { h->err = "lfd_set_base: frames must be non-NULL and n_base >= 1"; return LFD_E_ARG; }
-    TRY(enter(h));
-    if (rects && rect_offsets) TRY(check_rect_offsets(h, n_base, rect_offsets));
-    const size_t N = h->d.N;
+    h->n_base = 0;
     if (n_base > h->base_cap) {
         if (h->base_d) { cudaFree(h->base_d); h->base_d = nullptr; }
-        h->base_cap = 0; h->n_base = 0;
-        CK(cudaMalloc((void**)&h->base_d, (size_t)n_base * N * sizeof(float)));
+        h->base_cap = 0;
+        CK(cudaMalloc((void**)&h->base_d, (size_t)n_base * h->d.N * sizeof(float)));
         h->base_cap = n_base;
     }
     if (!h->inj_trails_d) {
@@ -1184,9 +1202,19 @@ extern "C" int lfd_set_base(lfd_handle* h, const float* frames, int n_base, cons
         CK(cudaMallocHost((void**)&h->inj_trails_h, (size_t)h->B * LFD_MAX_INJECT_TRAILS * sizeof(InjTrail)));
         CK(cudaMallocHost((void**)&h->inj_off_h, ((size_t)h->B + 1) * sizeof(int)));
         CK(cudaMallocHost((void**)&h->inj_base_h, (size_t)h->B * sizeof(int)));
-        for (int i = 0; i < 2; i++) CK(cudaEventCreate(&h->ev_inj[i]));
+        for (int i = 0; i < 2; i++) { CK(cudaEventCreate(&h->ev_inj[i])); CK(cudaEventCreate(&h->ev_cap[i])); }
     }
-    h->n_base = 0;
+    return LFD_OK;
+}
+
+extern "C" int lfd_set_base(lfd_handle* h, const float* frames, int n_base, const int32_t* rects, const int32_t* rect_offsets)
+{
+    if (!h) return LFD_E_ARG;
+    if (!frames || n_base < 1) { h->err = "lfd_set_base: frames must be non-NULL and n_base >= 1"; return LFD_E_ARG; }
+    TRY(enter(h));
+    if (rects && rect_offsets) TRY(check_rect_offsets(h, n_base, rect_offsets));
+    const size_t N = h->d.N;
+    TRY(inj_reserve(h, n_base));
     CK(cudaMemcpyAsync(h->base_d, frames, (size_t)n_base * N * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));          // the caller may free `frames` on return
     h->base_rect_off.assign((size_t)n_base + 1, 0);
@@ -1196,6 +1224,32 @@ extern "C" int lfd_set_base(lfd_handle* h, const float* frames, int n_base, cons
         h->base_rects.assign((const int4*)rects, (const int4*)rects + rect_offsets[n_base]);
     }
     h->n_base = n_base;
+    return LFD_OK;
+}
+
+extern "C" int lfd_capture_bases(lfd_handle* h)
+{
+    if (!h) return LFD_E_ARG;
+    TRY(enter(h));
+    if (!h->in_whole || h->in_injected) {
+        h->err = "lfd_capture_bases: the batch slots do not hold the input of a collected whole-frame batch"; return LFD_E_STATE;
+    }
+    const int n = h->last_n;
+    TRY(inj_reserve(h, n));
+    const size_t n16 = (size_t)n * h->d.N / 4;           // W % 4 == 0 (lfd_create)
+    const size_t want = (n16 + 4 * CAP_THREADS - 1) / (4 * CAP_THREADS);
+    const int grid = (int)(want < (size_t)h->sm_count * 8 ? want : (size_t)h->sm_count * 8);
+    CK(cudaEventRecord(h->ev_cap[0], h->stream));
+    if (h->in_be) k_capture_bases<true><<<grid, CAP_THREADS, 0, h->stream>>>((const uint4*)h->in, (uint4*)h->base_d, n16);
+    else k_capture_bases<false><<<grid, CAP_THREADS, 0, h->stream>>>((const uint4*)h->in, (uint4*)h->base_d, n16);
+    LAUNCH_CHECK();
+    CK(cudaEventRecord(h->ev_cap[1], h->stream));
+    h->cap_recorded = true;
+    // the batch's star rectangles are still in the submit staging: every other writer of rects_h (lfd_submit_injected,
+    // lfd_blot) also leaves the slots in a state this call refuses
+    h->base_rect_off.assign(h->rect_off_h, h->rect_off_h + n + 1);
+    h->base_rects.assign(h->rects_h, h->rects_h + h->rect_off_h[n]);
+    h->n_base = n;
     return LFD_OK;
 }
 
@@ -1315,6 +1369,7 @@ extern "C" int lfd_submit_injected_shaped(lfd_handle* h, int n, const int32_t* b
     CK(cudaMemcpyAsync(h->inj_off_d, h->inj_off_h, ((size_t)n + 1) * sizeof(int), cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(h->inj_base_d, h->inj_base_h, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, h->stream));
     CK(cudaEventRecord(h->ev_inj[0], h->stream));
+    h->in_injected = true;
     k_inject<<<dim3((h->d.H + INJ_ROWS - 1) / INJ_ROWS, n), INJ_THREADS, 0, h->stream>>>(h->base_d, h->inj_base_d, h->inj_trails_d,
                                                                                        h->inj_off_d, h->tab_samples_d, h->in, h->d); LAUNCH_CHECK();
     CK(cudaEventRecord(h->ev_inj[1], h->stream));
@@ -1350,6 +1405,12 @@ extern "C" int lfd_wait(lfd_handle* h, lfd_result* out)
             }
     h->inj_ms = 0.f;
     if (h->inj_recorded && cudaEventElapsedTime(&h->inj_ms, h->ev_inj[0], h->ev_inj[1]) != cudaSuccess) { h->inj_ms = 0.f; cudaGetLastError(); }
+    h->cap_ms = 0.f; h->cap_launches = 0;
+    if (h->cap_recorded) {
+        h->cap_recorded = false;
+        if (cudaEventElapsedTime(&h->cap_ms, h->ev_cap[0], h->ev_cap[1]) == cudaSuccess) h->cap_launches = 1;
+        else { h->cap_ms = 0.f; cudaGetLastError(); }
+    }
     if (out) memcpy(out, h->res_h, (size_t)h->last_n * sizeof(lfd_result));
     return LFD_OK;
 }
@@ -1357,12 +1418,20 @@ extern "C" int lfd_wait(lfd_handle* h, lfd_result* out)
 // Bracketed kernels of the last collected batch: name, pass, summed duration over the batch parts and number of launches.
 extern "C" int lfd_get_kernel_times(lfd_handle* h, int index, const char** name, int* pass, float* ms, int* launches)
 {
-    if (!h || index < 0 || index > 2 * KB_COUNT) return LFD_E_ARG;
+    if (!h || index < 0 || index > 2 * KB_COUNT + 1) return LFD_E_ARG;
     if (index == 2 * KB_COUNT) {       // k_inject, bracketed on every lfd_submit_injected (outside the graph)
         const bool on = h->inj_recorded && !h->pending;
         if (name) *name = "k_inject";
         if (pass) *pass = 0;
         if (ms) *ms = on ? h->inj_ms : 0.f;
+        if (launches) *launches = on ? 1 : 0;
+        return LFD_OK;
+    }
+    if (index == 2 * KB_COUNT + 1) {   // k_capture_bases, bracketed on every lfd_capture_bases before this batch
+        const bool on = h->cap_launches && !h->pending;
+        if (name) *name = "k_capture_bases";
+        if (pass) *pass = 0;
+        if (ms) *ms = on ? h->cap_ms : 0.f;
         if (launches) *launches = on ? 1 : 0;
         return LFD_OK;
     }

@@ -17,7 +17,7 @@ import traceback
 
 import numpy as _np
 
-from . import _lib, sdssfiles as files
+from . import _lib, inject as _inject, sdssfiles as files
 from .processfield import result_from_device, setup_debug
 from .removestars import read_photoObj_arrays, star_rects
 
@@ -261,7 +261,8 @@ def _decode_batch(h, shape, n):
     return out
 
 
-def compute_fields_iter(frames, params_bright, params_dim, params_removestars, batch=16, device=0, loaders=None):
+def compute_fields_iter(frames, params_bright, params_dim, params_removestars, batch=16, device=0, loaders=None,
+                        injections=None, injection_tables=None):
     """Run an ordered list of (run, camcol, filter, field) through the GPU in batches.  Generator: yields, batch by batch
     and in list order, ``(index of the batch's first frame, records)`` with one record per frame - ("line", results_line)
     for a detection, ("none", "") for no detection, ("err", errors_text) for a failure - exactly what the reference's
@@ -273,10 +274,18 @@ def compute_fields_iter(frames, params_bright, params_dim, params_removestars, b
     byte-swaps.  Frames the native reader declines (compressed, scaled, another BITPIX) go through the Python readers on
     loader threads (bz2 releases the GIL) and end up in the same staging slots; frames of another shape use a cached
     handle of their own.  A frame whose run / contour lists overflow the batch handles is re-run on a worst-case-capacity
-    handle instead of being reported as an error."""
+    handle instead of being reported as an error.
+
+    With ``injections`` (see DetectTrails) the record of every frame with a verdict carries a third item, the frame's
+    lines of the injection table: after a batch is collected, its handle makes the frames still in its slots the
+    injection bases (lfd_capture_bases, a device copy) and runs each injection on the slot of its frame, in steps of
+    the handle's slots.  ``injection_tables`` is the pool their ``profile`` / ``lightcurve`` keys index.  The
+    injections of a batch are checked when it is loaded, before it is submitted: a bad one raises ValueError."""
     from concurrent.futures import ThreadPoolExecutor
     frames = list(frames)
     debug = bool(params_bright["debug"] or params_dim["debug"])
+    if debug and injections is not None:
+        raise ValueError("injections are not supported with debug=True (the debug path runs frames one at a time on the host)")
     if debug:
         recs = _compute_fields_debug(frames, params_bright, params_dim, params_removestars)
         for i0 in range(0, len(frames), max(int(batch), 1)):
@@ -356,6 +365,46 @@ def compute_fields_iter(frames, params_bright, params_dim, params_removestars, b
         except Exception as e:   # noqa: BLE001
             return ("failed", gidx, e)
 
+    hough = (float(params_bright["houghMethod"]), float(params_dim["houghMethod"]))
+    injection_tables = list(injection_tables) if injection_tables else None
+    ntab = len(injection_tables) if injection_tables else 0
+    tables_set = set()          # id() of the handles that hold this call's table pool
+
+    def specs_of(ci, items):
+        """{global index: checked injections} of the frames of batch ci that were read (their shape is known)."""
+        specs = {}
+        if injections is not None:
+            for j, it in enumerate(items):
+                if it[0] != "err":
+                    shp = shape0 if it[0] == "staged" else tuple(int(v) for v in it[1].shape)
+                    specs[ci * batch + j] = _inject.check_injections(injections(chunks[ci][j], shp), ntab)
+        return specs
+
+    def inject(entry, outcome, specs):
+        """Run the injections of a collected batch from the frames still in its handle's slots (slot k holds gidx[k]);
+        each frame with a verdict gets its injection lines appended to its outcome.  An injected frame that overflows
+        is reported in its status, not retried."""
+        if entry[0] != "entry":
+            return
+        _tag, h, shape, gidx, _rects, _be = entry
+        jobs = [(slot, g, k, ts) for slot, g in enumerate(gidx) if outcome.get(g, ("err",))[0] == "ok"
+                for k, ts in enumerate(specs.get(g, ()))]
+        if not jobs:
+            return
+        if injection_tables and id(h) not in tables_set:
+            h.set_trail_tables(injection_tables)
+            tables_set.add(id(h))
+        h.capture_bases()
+        rows = {}
+        for i in range(0, len(jobs), h.B):
+            step = jobs[i:i + h.B]
+            h.submit_injected([j[0] for j in step], [j[3] for j in step])
+            for (_slot, g, k, ts), r in zip(step, h.wait_array()):
+                rows.setdefault(g, []).append(_inject.format_injection(frames[g], k, outcome[g][1], ts, r,
+                                                                      _inject._recovered(r, ts, shape, hough)))
+        for g, lines in rows.items():
+            outcome[g] = outcome[g] + ("".join(lines),)
+
     def records_of(ci, items, outcome):
         recs = []
         base = ci * batch
@@ -371,28 +420,45 @@ def compute_fields_iter(frames, params_bright, params_dim, params_removestars, b
                 recs.append(("line", str(item[4]) + f"{res['x1']} {res['y1']} {res['x2']} {res['y2']}\n"))
             else:
                 recs.append(("none", ""))
+            if exc is None and len(oc) > 3:
+                recs[-1] += (oc[3],)
         return recs
 
     with ThreadPoolExecutor(max_workers=2) as bpool, ThreadPoolExecutor(max_workers=nload) as fpool:
         futs = {0: bpool.submit(load_chunk, 0, fpool)} if chunks else {}
-        inflight = []            # [(ci, items, submitted entries, {outcomes known so far})] in submission order
+        inflight = []            # [(ci, items, submitted entries, {outcomes known so far}, injections)] in submission order
+        collected = []           # the same for collected batches whose injections and records are still to come
 
-        def drain(upto):
-            """Collect (and yield the records of) every submitted batch with index <= upto, oldest first."""
+        def collect(upto):
+            """Collect every submitted batch with index <= upto, oldest first: verdicts and the overflow retry, which
+            reads the handle's host staging before the next load overwrites it."""
             while inflight and inflight[0][0] <= upto:
-                cj, itj, ents, oc = inflight.pop(0)
+                b = inflight.pop(0)
+                for e in b[2]:
+                    b[3].update(finish(e))
+                collected.append(b)
+
+        def release():
+            """Run the injections of the collected batches and yield their records.  The injections use only the
+            device slots and the library's own staging, so they overlap the two loads in flight."""
+            while collected:
+                cj, itj, ents, oc, spj = collected.pop(0)
                 for e in ents:
-                    oc.update(finish(e))
+                    inject(e, oc, spj)
                 yield cj * batch, records_of(cj, itj, oc)
 
         try:
             for ci, chunk in enumerate(chunks):
                 # the handle batch ci+1 loads into is the one batch ci-2 used (ring of three): collect that one, then start
-                # the next load so that it runs while batch ci is submitted and batch ci-1 computes
-                yield from drain(ci - (len(ring) - 1 if ring else 1))
+                # the next load so that it runs while batch ci is submitted and batch ci-1 computes.  Batch ci-2's
+                # injections run while loads ci and ci+1 are in flight and before batch ci's frames are copied: the
+                # injected steps' small host->device copies would otherwise queue behind that batch copy
+                collect(ci - (len(ring) - 1 if ring else 1))
                 if ci + 1 < len(chunks):
                     futs[ci + 1] = bpool.submit(load_chunk, ci + 1, fpool)
+                yield from release()
                 items = futs.pop(ci).result()
+                specs = specs_of(ci, items)
                 base = ci * batch
                 h = ring[ci % len(ring)] if ring else None
                 outcome = {}
@@ -413,20 +479,24 @@ def compute_fields_iter(frames, params_bright, params_dim, params_removestars, b
                 for (shape, big_endian), idxs in others.items():
                     # another frame shape (or no ring): a cached handle of that shape, run to completion right away
                     gidx = [base + j for j in idxs]
+                    ent = ("failed",)
                     try:
                         hh = _batch_handles(shape, batch, device, count=1)[0]
                         stg = hh.host_frames.view(_np.uint32) if big_endian else hh.host_frames
                         for slot, j in enumerate(idxs):
                             stg[slot] = items[j][1]
-                        outcome.update(finish(submit(hh, shape, gidx, [items[j][3] for j in idxs], big_endian)))
+                        ent = submit(hh, shape, gidx, [items[j][3] for j in idxs], big_endian)
+                        outcome.update(finish(ent))
                     except Exception as e:   # noqa: BLE001
                         outcome.update({g: ("err", e) for g in gidx})
-                inflight.append((ci, items, entries, outcome))
-            yield from drain(len(chunks))
+                    inject(ent, outcome, specs)
+                inflight.append((ci, items, entries, outcome, specs))
+            collect(len(chunks))
+            yield from release()
         finally:
             # the consumer stopped early (or something raised): collect what is still on the GPU, so that the cached
             # handles are not left with a pending batch ("previous batch not collected" on their next use)
-            for _cj, _itj, ents, _oc in inflight:
+            for _cj, _itj, ents, _oc, _sp in inflight + collected:
                 for e in ents:
                     if e[0] == "entry":
                         try:
@@ -440,11 +510,12 @@ def compute_fields_iter(frames, params_bright, params_dim, params_removestars, b
                     pass
 
 
-def compute_fields(frames, params_bright, params_dim, params_removestars, batch=16, device=0, loaders=None):
+def compute_fields(frames, params_bright, params_dim, params_removestars, batch=16, device=0, loaders=None,
+                   injections=None, injection_tables=None):
     """All records of ``compute_fields_iter`` as one list in frame order."""
     out = []
     for _i0, recs in compute_fields_iter(frames, params_bright, params_dim, params_removestars, batch=batch, device=device,
-                                         loaders=loaders):
+                                         loaders=loaders, injections=injections, injection_tables=injection_tables):
         out.extend(recs)
     return out
 
@@ -474,7 +545,8 @@ def _compute_fields_debug(frames, params_bright, params_dim, params_removestars)
 
 
 def write_records(results, errors, records):
-    for kind, text in records:
+    for rec in records:
+        kind, text = rec[0], rec[1]
         if kind == "line":
             results.write(text)
         elif kind == "err":
@@ -499,10 +571,14 @@ def read_progress(path):
 
 
 def process_fields(results, errors, frames, params_bright, params_dim, params_removestars, batch=16, device=0,
-                   distributed=None, compute=None, progress=None):
+                   distributed=None, compute=None, progress=None, injections=None, injection_tables=None,
+                   injection_results=None):
     """Process an ordered list of (run, camcol, filter, field); results/errors are written in list order,
     exactly the lines the reference's per-frame loop would write, and flushed after every GPU batch (the reference
     appends frame by frame, detecttrails.py:127-139: a killed run keeps what it finished).
+
+    ``injections`` / ``injection_tables``: see DetectTrails; the injection lines a record carries as its third item go
+    to the open file ``injection_results``, in frame order, written and flushed with the batch's results and errors.
 
     With ``torch.distributed`` initialised (one process per GPU, e.g. under torchrun) the list is sharded by
     frame across the ranks - blocks of ``batch`` consecutive frames dealt round-robin, no data-path collective -
@@ -522,9 +598,12 @@ def process_fields(results, errors, frames, params_bright, params_dim, params_re
     def emit(part, recs):
         write_records(results, errors, recs)
         results.flush(); errors.flush()
+        if injection_results is not None:
+            injection_results.write("".join(rec[2] for rec in recs if len(rec) > 2))
+            injection_results.flush()
         if progress:
             with open(progress, "a") as pf:
-                pf.write("".join(_progress_key(fr) + " " + kind + "\n" for fr, (kind, _text) in zip(part, recs)))
+                pf.write("".join(_progress_key(fr) + " " + rec[0] + "\n" for fr, rec in zip(part, recs)))
 
     if not distributed:
         if compute is not None:                       # injected compute stage (tests): one call per `batch * 32` frames
@@ -532,10 +611,12 @@ def process_fields(results, errors, frames, params_bright, params_dim, params_re
             for i0 in range(0, len(frames), step):
                 emit(frames[i0:i0 + step], compute(frames[i0:i0 + step]))
             return
-        for i0, recs in compute_fields_iter(frames, params_bright, params_dim, params_removestars, batch=batch, device=device):
+        for i0, recs in compute_fields_iter(frames, params_bright, params_dim, params_removestars, batch=batch, device=device,
+                                            injections=injections, injection_tables=injection_tables):
             emit(frames[i0:i0 + len(recs)], recs)
         return
-    compute = compute or (lambda fr: compute_fields(fr, params_bright, params_dim, params_removestars, batch=batch, device=device))
+    compute = compute or (lambda fr: compute_fields(fr, params_bright, params_dim, params_removestars, batch=batch, device=device,
+                                                    injections=injections, injection_tables=injection_tables))
     # frames per gather: every rank runs `32` of its own batches between two gathers (the ring drains at a gather)
     chunk = max(batch, 1) * sharding.world_size() * 32
     for i0 in range(0, len(frames), chunk):
@@ -558,7 +639,20 @@ class DetectTrails:
     ``device`` (CUDA device index, default: LOCAL_RANK under torchrun, else 0) and ``resume`` (path of a progress
     file, or True for ``<savepath>/progress.txt``: frames listed there are skipped and finished frames are appended,
     so an interrupted run can be restarted without duplicating lines - the reference only appends, detecttrails.py:349).
-    Under torchrun (torch.distributed initialised) the frame list is sharded over the ranks and rank 0 writes."""
+    Under torchrun (torch.distributed initialised) the frame list is sharded over the ranks and rank 0 writes.
+
+    Completeness of the run itself: ``injections``, a callable ``injections(frame, shape) -> [[trail, ...], ...]``
+    called with ``frame`` = (run, camcol, filter, field) and the frame's (H, W) as read, returns the frame's injections,
+    each a list of at most 16 trails in ``inject.recovery``'s format (``p0``, ``p1``, ``sigma``, ``peak``, optional
+    ``profile`` / ``lightcurve`` indices into ``injection_tables``), end points in the un-flipped FITS orientation.
+    Every frame with a verdict gets them, injected on the device into the copy of the frame already there (no second
+    read or upload), and one line per injection goes to ``injection_results`` (default ``<savepath>/injections.txt``,
+    appended like results.txt; inject.read_injections reads it): the frame, the index k of the injection, the
+    frame's own verdict, the injected frame's verdict, line and ``recovered`` (inject.recovery's default tolerances),
+    and the trails.  The callable must return the same injections for the same frame on every call (e.g. seeded
+    from synth.frame_seed): sharded and resumed runs rely on it.  A bad injection (more than 16 trails, a value that
+    is not finite, sigma <= 0 for a Gaussian, a table index outside the pool) raises ValueError before its batch is
+    submitted; so does ``debug=True``.  results.txt, errors.txt and the progress file are the same as without."""
 
     def __init__(self, **kwargs):
         savepth = (kwargs["savepath"] if "savepath" in kwargs else ".")
@@ -572,6 +666,9 @@ class DetectTrails:
             self.device = spread_device(os.environ.get("LOCAL_RANK", 0)) if "LOCAL_RANK" in os.environ else 0
         resume = kwargs.get("resume", None)
         self.progress = (os.path.join(savepth, "progress.txt") if resume is True else resume) or None
+        self.injections = kwargs.get("injections", None)
+        self.injection_tables = kwargs.get("injection_tables", None)
+        self.injection_results = kwargs.get("injection_results", os.path.join(savepth, "injections.txt"))
 
         if "results" in kwargs:
             self.results = kwargs["results"]
@@ -681,7 +778,10 @@ class DetectTrails:
         return out
 
     def process(self):
-        """Run the selected frames; results/errors files are opened in append mode like the original."""
-        with open(self.results, "a") as results, open(self.errors, "a") as errors:
+        """Run the selected frames; results/errors (and injection) files are opened in append mode like the original."""
+        import contextlib
+        with open(self.results, "a") as results, open(self.errors, "a") as errors, \
+                (open(self.injection_results, "a") if self.injections is not None else contextlib.nullcontext()) as inj:
             process_fields(results, errors, self.frame_list(), self.params_bright, self.params_dim,
-                           self.params_removestars, batch=self.batch, device=self.device, progress=self.progress)
+                           self.params_removestars, batch=self.batch, device=self.device, progress=self.progress,
+                           injections=self.injections, injection_tables=self.injection_tables, injection_results=inj)

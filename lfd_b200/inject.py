@@ -13,7 +13,7 @@ import numpy as np
 
 from . import _lib
 
-__all__ = ["trail_line", "recovery", "defocus_profile", "RECOVERY_DTYPE"]
+__all__ = ["trail_line", "recovery", "defocus_profile", "read_injections", "RECOVERY_DTYPE", "INJECTION_DTYPE"]
 
 _T = _lib.MAX_INJECT_TRAILS
 RECOVERY_DTYPE = np.dtype([
@@ -22,6 +22,15 @@ RECOVERY_DTYPE = np.dtype([
     ("sigma", "<f4", (_T,)), ("peak", "<f4", (_T,)),
     ("detected", "?"), ("pass", "<i4"), ("status", "<i4"), ("rho", "<f4"), ("theta", "<f4"),
     ("base_detected", "?"), ("recovered", "<i4")])
+# one row of a drop-in run's injection table (DetectTrails(injections=...), read_injections): the frame and the index k
+# of the injection in the callable's list instead of a base index, and each trail's table indices (-1 past ntrails)
+INJECTION_DTYPE = np.dtype([
+    ("run", "<i4"), ("camcol", "<i4"), ("filter", "U1"), ("field", "<i4"), ("k", "<i4"), ("ntrails", "<i4"),
+    ("x0", "<f4", (_T,)), ("y0", "<f4", (_T,)), ("x1", "<f4", (_T,)), ("y1", "<f4", (_T,)),
+    ("sigma", "<f4", (_T,)), ("peak", "<f4", (_T,)), ("profile", "<i4", (_T,)), ("lightcurve", "<i4", (_T,)),
+    ("detected", "?"), ("pass", "<i4"), ("status", "<i4"), ("rho", "<f4"), ("theta", "<f4"),
+    ("base_detected", "?"), ("recovered", "<i4")])
+_TRAIL_F = ("x0", "y0", "x1", "y1", "sigma", "peak")
 
 
 def trail_line(trail, shape):
@@ -91,6 +100,92 @@ def _first_match(rho, theta, lines, theta_tol, rho_tol):
             if abs(theta - tt - k * math.pi) <= theta_tol and abs(rho - (-rt if k else rt)) <= rho_tol:
                 return i
     return -1
+
+
+def _recovered(r, trails, shape, hough, theta_tol=np.deg2rad(2), rho_tol=None):
+    """``recovered`` of a device result ``r`` (an lfd_result row) for the injected ``trails``: the index of the first
+    trail its line matches, -1 when undetected, overflowed or unmatched; ``hough`` = the two passes' houghMethod."""
+    if not r["detected"] or (r["status"] & _lib.FRAME_OVERFLOW):
+        return -1
+    rt = hough[r["pass_"]] if rho_tol is None else float(rho_tol)
+    return _first_match(float(r["rho"]), float(r["theta"]), [trail_line(t, shape) for t in trails], float(theta_tol), rt)
+
+
+def check_injections(specs, n_tables):
+    """A frame's injections as the ``injections`` callable of DetectTrails returns them, checked: a list of lists of
+    at most 16 trail dicts with finite end points and peak, ``sigma`` > 0 for a Gaussian profile, and ``profile`` /
+    ``lightcurve`` indices in -1 .. n_tables - 1.  Raises ValueError naming the first bad trail, also for a missing
+    key or a value that is not a number."""
+    try:
+        specs = [list(ts) for ts in specs]
+    except TypeError as e:
+        raise ValueError("injections must be a list of lists of trail dicts (%s)" % e) from None
+    for k, ts in enumerate(specs):
+        if len(ts) > _T:
+            raise ValueError("injection %d has %d trails, at most %d are allowed" % (k, len(ts), _T))
+        for i, t in enumerate(ts):
+            where = "injection %d, trail %d" % (k, i)
+            try:
+                for key in ("profile", "lightcurve"):
+                    v = t.get(key, -1)
+                    if not isinstance(v, (int, np.integer)) or isinstance(v, bool) or not -1 <= v < n_tables:
+                        raise ValueError("%s %r is not a table index in -1 .. %d" % (key, v, n_tables - 1))
+                gauss = t["profile"] < 0 if "profile" in t else True
+                vals = [t["p0"][0], t["p0"][1], t["p1"][0], t["p1"][1], t["peak"]] + ([t["sigma"]] if gauss else [])
+                with np.errstate(over="ignore"):
+                    vals = [float(np.float32(v)) for v in vals]
+            except (KeyError, IndexError, TypeError, AttributeError, ValueError) as e:
+                raise ValueError("%s: %s" % (where, "missing key %s" % e if isinstance(e, KeyError) else e)) from None
+            if not all(math.isfinite(v) for v in vals):
+                raise ValueError("%s: end points, sigma and peak must be finite in float32" % where)
+            if gauss and not vals[5] > 0:
+                raise ValueError("%s: a Gaussian trail needs sigma > 0" % where)
+    return specs
+
+
+def _f9(v):
+    return "%.9g" % float(np.float32(v))
+
+
+def format_injection(frame, k, base_detected, trails, r, recovered):
+    """One line of the injection table: ``run camcol filter field k base_detected detected pass status rho theta
+    recovered ntrails`` then ``x0 y0 x1 y1 sigma peak profile lightcurve`` per trail (end points un-flipped, as given).
+    Floats are the float32 values in %.9g, which reads back to the same bits; ``r`` is the injected frame's lfd_result."""
+    run, camcol, flt, field = frame
+    arr = _lib.Handle.trails_array(trails)
+    head = "%d %d %s %d %d %d %d %d %d %s %s %d %d" % (
+        run, camcol, flt, field, k, bool(base_detected), bool(r["detected"]), r["pass_"], r["status"], _f9(r["rho"]),
+        _f9(r["theta"]), recovered, len(trails))
+    body = "".join(" %s %s %s %s %s %s %d %d" % (tuple(_f9(a[f]) for f in _TRAIL_F) + (t.get("profile", -1), t.get("lightcurve", -1)))
+                   for a, t in zip(arr, trails))
+    return head + body + "\n"
+
+
+def read_injections(path):
+    """The injection table a drop-in run wrote (DetectTrails(injections=...), one line per injection) as an
+    INJECTION_DTYPE array; trail fields past ``ntrails`` are NaN (table indices -1)."""
+    with open(path) as f:
+        lines = [ln.split() for ln in f if ln.strip()]
+    out = np.zeros(len(lines), INJECTION_DTYPE)
+    for f in _TRAIL_F:
+        out[f] = np.nan
+    out["profile"] = out["lightcurve"] = -1
+    for r, t in enumerate(lines):
+        n = int(t[12])
+        if len(t) != 13 + 8 * n or n > _T:
+            raise ValueError("%s: malformed injection line %d" % (path, r + 1))
+        out["run"][r], out["camcol"][r], out["filter"][r], out["field"][r], out["k"][r] = int(t[0]), int(t[1]), t[2], int(t[3]), int(t[4])
+        out["base_detected"][r], out["detected"][r] = bool(int(t[5])), bool(int(t[6]))
+        out["pass"][r], out["status"][r] = int(t[7]), int(t[8])
+        out["rho"][r], out["theta"][r] = float(t[9]), float(t[10])
+        out["recovered"][r], out["ntrails"][r] = int(t[11]), n
+        if n:
+            v = np.array(t[13:], dtype=object).reshape(n, 8)
+            for j, fld in enumerate(_TRAIL_F):
+                out[fld][r, :n] = [float(s) for s in v[:, j]]
+            out["profile"][r, :n] = [int(s) for s in v[:, 6]]
+            out["lightcurve"][r, :n] = [int(s) for s in v[:, 7]]
+    return out
 
 
 def recovery(frames, rects, injections, params_bright=None, params_dim=None, device=0, batch=64,
@@ -170,9 +265,5 @@ def recovery(frames, rects, injections, params_bright=None, params_dim=None, dev
         row["detected"], row["pass"], row["status"] = bool(r["detected"]), r["pass_"], r["status"]
         row["rho"], row["theta"] = r["rho"], r["theta"]
         row["base_detected"] = bool(res[b]["detected"])
-        row["recovered"] = -1
-        if r["detected"] and not (r["status"] & _lib.FRAME_OVERFLOW):
-            rt = hough[r["pass_"]] if rho_tol is None else float(rho_tol)
-            row["recovered"] = _first_match(float(r["rho"]), float(r["theta"]), [trail_line(t, (H, W)) for t in ts],
-                                            float(theta_tol), rt)
+        row["recovered"] = _recovered(r, ts, (H, W), hough, theta_tol, rho_tol)
     return out
